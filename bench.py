@@ -3,7 +3,7 @@
 same JSON line, key "bi_encoder" -- BASELINE metric (ii): bi-encoder passages/s at the 1B6 shape (configs[2]),
 batch-sharded over the ranks with one NCCL all_gather of the [B_local, D] embeddings per step.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one forward + backward pass of the WKV6 operator over one batch of synthetic input
 (B=8, T=4096, H=32, N=64, bf16) per GPU, through the reference-shaped Python surface
@@ -18,6 +18,9 @@ kernels' arithmetic on host cores) on a bounded sample; `reference_cuda` = the r
 kernels (oracle/_ref) timed on the same GPU and inputs, when they were built.
 `--impl reference` times the reference's CPU implementation of the path (the oracle port, all host
 threads) on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/<name>.npy, float32: a fixed sample of
+y, gr, gk, gv, gw (the same elements in every run, see dump_index) and the whole gu.  The inputs depend on nothing but
+the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -37,6 +40,27 @@ C = H * N
 BYTES_FWD = 10     # r,k,v,w read + y written, bf16                      (SURVEY.md 8d)
 BYTES_BWD = 18     # r,k,v,w,gy read + gr,gk,gv,gw written, bf16
 CPU_SAMPLE = dict(B=1, T=4096, H=32)   # 1/8 of one step's batch
+DUMP_SAMPLE = 1 << 21                  # elements dumped of each [B, T, C] output: 8 MB of float32 each, 40 MB in all
+
+
+def dump_index(device="cpu"):
+    """Sorted, distinct flat indices into a [B, T, C] output: one element of every run of B*T*C / DUMP_SAMPLE
+    consecutive ones, its offset in the run drawn by a generator with a fixed seed."""
+    import torch
+    run = B * T * C // DUMP_SAMPLE
+    assert run * DUMP_SAMPLE == B * T * C
+    g = torch.Generator().manual_seed(0)
+    return (torch.arange(DUMP_SAMPLE) * run + torch.randint(0, run, (DUMP_SAMPLE,), generator=g)).to(device)
+
+
+def dump_outputs(out_dir, y, grads):
+    """Writes one step's results of RUN_CUDA_RWKV6 + backward: y and gr, gk, gv, gw sampled at dump_index(), gu whole."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    idx = dump_index(y.device)
+    for name, t in zip(("y", "gr", "gk", "gv", "gw"), [y] + list(grads[:4])):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().reshape(-1)[idx].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "gu.npy"), grads[4].detach().float().cpu().numpy())
 
 
 def peaks():
@@ -296,7 +320,12 @@ def main():
     ap.add_argument("--no-bi-encoder", action="store_true")
     ap.add_argument("--bi-graph", action="store_true", help="bi-encoder leg as a CUDA-graph replay of the whole forward")
     ap.add_argument("--no-sft", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -400,12 +429,16 @@ def main():
     if graph is not None:
         for i in range(args.steps):
             graph.replay()
+        last = (y_static, [t.grad for t in static])
     else:
         for i in range(args.steps):
-            step(r, k, v, w, u, gy)
+            last = step(r, k, v, w, u, gy)
     t_end.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
     launches = launches_per_step * args.steps if graph is not None else M.launch_count() - launches0
     ms = t_start.elapsed_time(t_end) / args.steps
     eager_ms = ms

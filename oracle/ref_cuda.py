@@ -1,5 +1,5 @@
-"""ctypes binding of the reference's OWN CUDA kernels, compiled by `make -C oracle ref` from
-/root/reference/cuda/*.cu into oracle/_ref/ (git-ignored; travels to the GPU box).
+"""ctypes binding of the reference's OWN CUDA kernels, compiled by `make -C oracle ref REF=<RWKV_LM_EXT checkout>`
+from its cuda/*.cu into oracle/_ref/ (git-ignored).
 TEST / BENCH INFRASTRUCTURE ONLY: used as a second checker on the GPU and as the
 "reference wkv6_cuda" timing beside ours (BASELINE.json configs[1]).  Entry points are the
 `cuda_forward` / `cuda_backward` launchers at cuda/wkv6_cuda.cu:229-242 etc. (C++-mangled names).

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -22,6 +24,22 @@ def test_reference_arm_prints_the_contract_line():
     # a step is a bounded sample, timed as it is: ms_per_step x tokens/s = the tokens of one sample
     assert abs(line["ms_per_step"] * 1e-3 * line["value"] - line["tokens_per_step"]) <= 1e-6 * line["tokens_per_step"]
     assert line["gpu_launches"] == 0
+
+
+def test_bad_arguments_are_refused(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", extra
+    assert os.listdir(tmp_path) == []
+
+
+def test_dump_index_is_a_fixed_sample_without_repeats():
+    import bench
+    idx = bench.dump_index()
+    assert idx.numel() == bench.DUMP_SAMPLE and (idx[1:] > idx[:-1]).all()
+    assert 0 <= idx[0] and idx[-1] < bench.B * bench.T * bench.C
+    assert torch.equal(idx, bench.dump_index())
 
 
 def test_ranks_other_than_zero_do_no_work_in_the_reference_arm():

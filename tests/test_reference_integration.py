@@ -1,5 +1,5 @@
 """Drop-in boundary against the REAL caller (SURVEY.md 7 step 2c): the reference's own, unmodified `src/model.py` is
-imported -- here in the build container, where /root/reference exists; skipped elsewhere -- with its working directory
+imported from the RWKV_LM_EXT checkout named by $RWKV_LM_EXT_SRC (skipped without one) -- with its working directory
 pointing at shim/ (whose cuda/*_op.cpp replace the reference's), so that ITS `load(name="wkv6", sources=["cuda/wkv6_op.cpp",
 "cuda/wkv6_cuda.cu"], ...)` call (src/model.py:188-189) builds and imports OUR module; then `rwkv_lm_ext_b200.install`
 repoints the module-level operator every `RWKV_Tmix_x060` layer calls.  No GPU needed: nothing is launched."""
@@ -11,7 +11,7 @@ import textwrap
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("RWKV_LM_EXT_SRC", "")        # an unmodified checkout of yynil/RWKV_LM_EXT
 
 _SCRIPT = textwrap.dedent(r"""
     import os, sys, types
@@ -51,7 +51,8 @@ _SCRIPT = textwrap.dedent(r"""
 """)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="the reference tree only exists in the build container")
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "src")),
+                    reason="needs an unmodified RWKV_LM_EXT checkout: set RWKV_LM_EXT_SRC to its directory")
 @pytest.mark.parametrize("train_type", ["", "infctx"])
 def test_unmodified_reference_model_loads_our_ops(tmp_path, train_type):
     script = tmp_path / "probe.py"

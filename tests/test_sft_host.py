@@ -89,6 +89,7 @@ def test_lora_linear_fused_backward_equals_the_eager_chain():
             assert torch.allclose(a, b, atol=1e-10)
         # frozen weight, gradients straight into the flat buffer: two backward passes accumulate, the hooks fire once each
         m.weight.requires_grad = False
+        sinks_before = dict(sft._GRAD_SINKS)   # SftTrainer never calls GradBuckets.remove(): earlier tests' trainers keep theirs
         gbk = sft.GradBuckets([m.lora_A, m.lora_B], n_buckets=1)
         try:
             for rep in (1, 2):
@@ -100,7 +101,7 @@ def test_lora_linear_fused_backward_equals_the_eager_chain():
             assert torch.allclose(x.grad, 2 * want[0], atol=1e-10) and m.weight.grad is None
         finally:
             gbk.remove()
-        assert not sft._GRAD_SINKS
+        assert sft._GRAD_SINKS == sinks_before
         m.train()
         m.lora_dropout.p = 0.5                                   # dropout: the eager chain (different mask per call)
         assert m(x).shape == ref.shape
