@@ -8,8 +8,8 @@
  *     stream, which is what the reference's bare <<<>>> launches use, cuda/wkv6_cuda.cu:233);
  *   - the caller owns every buffer, including the workspace (size from the matching
  *     *_workspace_bytes) -- the reference wrappers likewise pre-allocate all outputs with
- *     torch.empty (src/model.py:211,225-230).  The library itself only keeps one 4 MB per-device
- *     ring of per-stream flags, plus the scratch noted at wkv6_forward.
+ *     torch.empty (src/model.py:211,225-230).  The library keeps no device memory of its own: what
+ *     an entry needs beyond its arguments is stream-ordered scratch (cudaMallocAsync, e.g. wkv6_forward).
  *
  * Layout contract (identical to the reference): r,k,v,w,y,gy,g* are [B,T,C] contiguous,
  * C = H*64 (head size is fixed at 64 like -D_N_=64, src/model.py:189); u is [H,64];
@@ -78,8 +78,9 @@ WKV6_API float       wkv6b200_set_decay_clamp(float nats_per_token);
  * Implementation note: the tensor-core kernels read raw bf16 logits, so these two entries first
  * recover them (bf16(log(-ew)), exact when ew was built from bf16 logits as src/model.py:210 does);
  * streams where that round trip is not exact are computed by the fp32 SIMT kernels from ew itself.
- * wkv6_forward has no workspace argument in the reference, so it takes B*T*C*2 bytes of
- * stream-ordered scratch (cudaMallocAsync, kept cached); wkv6_backward uses its workspace.
+ * wkv6_forward has no workspace argument in the reference, so it takes B*T*C*2 + B*H*4 bytes of
+ * stream-ordered scratch (cudaMallocAsync, kept cached) for the logits and one flag per (b,h) stream;
+ * wkv6_backward keeps both in its workspace.
  * ------------------------------------------------------------------------------------------ */
 WKV6_API int wkv6_forward(int B, int T, int C, int H, const void *r, const void *k, const void *v,
                  const float *ew, const void *u, void *y, void *stream);
@@ -102,7 +103,7 @@ WKV6_API int wkv6_backward_raww(int B, int T, int C, int H, const void *r, const
  * :137-182 and :83-128): the reference forward keeps r,k,v,w,u(,s) for backward with
  * ctx.save_for_backward and its backward re-runs the whole state recurrence; here the forward also
  * leaves, in `saved` (caller-owned, wkv6_saved_bytes), the bf16 state at the start of every
- * 64-token chunk plus a flag header, and the backward consumes it instead of recomputing it.
+ * 64-token chunk, and the backward consumes it instead of recomputing it.
  *   s0: NULL (zero state) | [H,64,64] (s0_batched = 0, wkv6state) | [B,H,64,64] (s0_batched = 1,
  *       wkv6infctx); bf16, or fp32 in the forward when s0_f32.  sT: NULL or [B,H,64,64] final state
  *       out (may alias s0).  *saved_valid (host int) is set to 1 when `saved` was filled; pass

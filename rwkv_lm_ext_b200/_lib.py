@@ -110,7 +110,7 @@ def check(rc: int, what: str):
 
 
 def require_current_device(t):
-    """The library takes its stream from the tensor's device but its scratch (flag ring, memory pool, function attributes)
+    """The library takes its stream from the tensor's device but its scratch (memory pool, function attributes)
     from the CURRENT device: a tensor on another device must be used under `torch.cuda.device(t.device)`."""
     import torch
     if not t.is_cuda:

@@ -61,154 +61,113 @@ static int check_shape(int B, int T, int C, int H) {
             if (!_p[_i]) { set_error("%s: null pointer argument #%zu", __func__, _i); return WKV6_EINVAL; } \
     } while (0)
 
-// per-stream hazard flags of a forward call that has no `saved` buffer: slices of a small per-device
-// ring (4 MB, allocated on first use, never freed), so that calls in flight on different CUDA
-// streams do not share flags
-static int *flag_slice(size_t n) {
-    constexpr size_t RING = 1u << 20;
-    static int *ring[64] = {};
-    static std::atomic<size_t> head[64];
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64 || n > RING) return nullptr;
-    if (!ring[dev]) {
-        static std::atomic_flag lock = ATOMIC_FLAG_INIT;
-        while (lock.test_and_set()) {}
-        if (!ring[dev]) {
-            int *p = nullptr;
-            if (cudaMalloc((void **)&p, RING * sizeof(int)) == cudaSuccess) ring[dev] = p;
-        }
-        lock.clear();
-        if (!ring[dev]) return nullptr;
-    }
-    // reserve [off, off + n) with a compare-and-swap loop; a slice that would cross the end of the ring starts at 0
-    // and moves the head behind itself, so two live slices only overlap after a full turn of the ring (1M flags)
-    size_t cur = head[dev].load(), off;
-    do {
-        off = cur % RING;
-        if (off + n > RING) off = 0;
-    } while (!head[dev].compare_exchange_weak(cur, cur - cur % RING + (off == 0 && cur % RING != 0 ? RING : 0) + off + n));
-    return ring[dev] + off;
-}
 // Forward over `nseg` time segments that run as separate grid rows (seg_scan.cu): state-only pass from zero
 // states, scan over the segment states, ordinary pass with the scanned initial states.
-// flags: [B*H], already holding any pre-set stream flags.
-// ckpt / seg_flags: nullptr, or (training pair) where the chunk-start states and the per-segment flags go.
-// presets: `flags` may already hold non-zero entries (streams whose fp32 decay did not convert exactly).
-static int tc3_forward_segmented(const Args &a, int *flags, int nseg, int seg_chunks, void *ckpt = nullptr,
-                                 int *seg_flags = nullptr, bool presets = false) {
+// flags: nullptr, or the stream flags of the fp32-decay conversion ([B*H]); ckpt: nullptr, or (training pair) where
+// the chunk-start states go.
+static int tc3_forward_segmented(const Args &a, int *flags, int nseg, int seg_chunks, void *ckpt) {
     wkv6::ensure_pool_keeps_memory();
     const int Bs = a.B * nseg, C = a.H * 64, seg_tokens = seg_chunks * 64;
     const size_t st = (size_t)Bs * a.H * 4096, nl = (size_t)Bs * C, nf = (size_t)Bs * a.H;
     float *buf = nullptr;
-    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&buf, (2 * st + nl) * sizeof(float) + nf * sizeof(int), a.stream));
+    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&buf, (2 * st + nl) * sizeof(float) + (flags ? nf * sizeof(int) : 0), a.stream));
     float *s_loc = buf, *s_start = buf + st, *lam = s_start + st;
-    int *sflags = seg_flags ? seg_flags : (int *)(lam + nl);
-    int rc = cudaMemsetAsync(sflags, 0, nf * sizeof(int), a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
-    if (rc == WKV6_OK && presets) rc = seg_flags_merge(a.B, nseg, a.H, sflags, flags, a.stream);      // broadcast pre-set flags
+    int *sflags = flags ? (int *)(lam + nl) : nullptr;      // the stream flags broadcast to the segment rows
+    int rc = WKV6_OK;
+    if (flags) {
+        rc = cudaMemsetAsync(sflags, 0, nf * sizeof(int), a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
+        if (rc == WKV6_OK) rc = seg_flags_merge(a.B, nseg, a.H, sflags, flags, a.stream);
+    }
     Args a1 = a;
     a1.s0 = nullptr; a1.s0_bstride = 0; a1.sT = s_loc; a1.sT_f32 = 1; a1.y = nullptr; a1.saved = nullptr;
     if (rc == WKV6_OK) rc = tc3_forward(a1, nullptr, sflags, nseg, seg_chunks);
-    if (rc == WKV6_OK) rc = seg_flags_merge(a.B, nseg, a.H, sflags, flags, a.stream);
     if (rc == WKV6_OK) rc = seg_decay(a.B, a.T, C, nseg, seg_tokens, a.w, lam, tc_lmin_nats(a), a.stream);
     if (rc == WKV6_OK) rc = seg_scan(a.B, nseg, a.H, lam, s_loc, a.s0, a.s0_f32, a.s0_bstride, s_start, a.sT, a.sT_f32, 0, flags, a.stream);
     Args a2 = a;
     a2.s0 = s_start; a2.s0_f32 = 1; a2.s0_bstride = (long long)a.H * 4096; a2.sT = nullptr; a2.saved = nullptr;
-    // (this pass sees the same decays as the first one: it cannot raise a flag the merge above has not seen)
     if (rc == WKV6_OK) rc = tc3_forward(a2, ckpt, sflags, nseg, seg_chunks);
     cudaFreeAsync(buf, a.stream);
     return rc;
 }
-static int forward3(const Args &a) {
-    int *flags;
+// the tensor-core forward on raw bf16 logits; flags: nullptr, or the stream flags of the fp32-decay conversion
+static int forward3(const Args &a, int *flags = nullptr) {
     void *ckpt = nullptr;
-    const size_t nb = (size_t)a.B * a.H * sizeof(int);
     if (a.saved) {
-        flags = (int *)a.saved;
-        ckpt = (uint8_t *)a.saved + tc3_saved_header(a.B, a.H);
-    } else {
-        flags = flag_slice((size_t)a.B * a.H);
-        if (!flags) { set_error("cannot get %zu bytes of flag scratch", nb); return WKV6_ECUDA; }
+        // the training pair's header: per-head arrival counters of the backward's in-kernel gu reduction
+        WKV6_CUDA_CHECK(cudaMemsetAsync(a.saved, 0, TC3_SAVED_HEADER, a.stream));
+        ckpt = (uint8_t *)a.saved + TC3_SAVED_HEADER;
     }
-    // (the training pair's header has 512 more ints behind the stream flags: per-head arrival counters of the backward's
-    // in-kernel gu reduction when the call is not segmented, per-segment flags when it is)
-    WKV6_CUDA_CHECK(cudaMemsetAsync(flags, 0, a.saved ? nb + 512 * sizeof(int) : nb, a.stream));
     // the training pair segments forward and backward alike (the saved chunk states are in segment-row order)
     int nseg = 1, seg_chunks = 0;
     if (a.saved) seg_plan_train(a.B, a.T, a.H, &nseg, &seg_chunks);
     else seg_plan(a.B, a.T, a.H, &nseg, &seg_chunks);
-    // (raw bf16 logits: nothing can raise a flag -- the kernels never do, and there is no fp32 decay to convert -- so
-    // no predicated exact-route launch follows; the zeroed flags only feed the kernels' entry check and the diagnostics)
-    return nseg > 1 ? tc3_forward_segmented(a, flags, nseg, seg_chunks, ckpt, a.saved ? flags + (size_t)a.B * a.H : nullptr)
-                    : tc3_forward(a, ckpt, flags);
+    return nseg > 1 ? tc3_forward_segmented(a, flags, nseg, seg_chunks, ckpt) : tc3_forward(a, ckpt, flags);
 }
-// the same call with the fp32 log-decay converted to raw bf16 logits (tensor-core kernels), exact SIMT
-// kernels on the original values for the streams where that conversion is not lossless
+
+// fp32 decays (-exp(w) of wkv6 / wkv6_bi, exp(-exp(w)) of rwkv6 inference): the tensor-core routes on the raw bf16
+// logits they convert to, then the exact SIMT kernels on the original values for the streams where that conversion is
+// not lossless (the only streams that are ever flagged)
 static Args with_raw_w(const Args &a, void *w_raw) {
     Args t = a;
     t.w = w_raw;
     t.w_kind = W_RAW_BF16;
     return t;
 }
-static bool ew_convertible(const Args &a) {
-    return (a.w_kind == W_LOG_F32 || a.w_kind == W_DECAY_F32) && tc3_forward_supported(with_raw_w(a, const_cast<void *>(a.w)));
+static bool ew_convertible(const Args &a, bool backward) {
+    if ((a.w_kind != W_LOG_F32 && a.w_kind != W_DECAY_F32) || a.saved) return false;
+    const Args t = with_raw_w(a, const_cast<void *>(a.w));
+    return bi_forward_tc_supported(t) || (backward ? tc3_backward_supported(t) : tc3_forward_supported(t));
 }
-static int forward3_ew(const Args &a) {
-    // the reference's entry has no workspace argument: stream-ordered scratch, kept cached in the pool
+static int forward_ew(const Args &a) {
+    // the reference's entries have no workspace argument: stream-ordered scratch, kept cached in the pool
     wkv6::ensure_pool_keeps_memory();
-    const size_t nb = (size_t)a.B * a.H * sizeof(int);
-    int *flags = flag_slice((size_t)a.B * a.H);
-    if (!flags) { set_error("cannot get %zu bytes of flag scratch", nb); return WKV6_ECUDA; }
-    void *w_raw = nullptr;
-    WKV6_CUDA_CHECK(cudaMallocAsync(&w_raw, (size_t)a.B * a.T * a.H * 64 * 2, a.stream));
-    int rc = cudaMemsetAsync(flags, 0, nb, a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
-    if (rc == WKV6_OK) rc = ew_to_raw_bf16(a.B, a.T, a.H, (const float *)a.w, w_raw, flags, a.stream, a.w_kind == W_DECAY_F32);
-    int nseg = 1, seg_chunks = 0;
-    seg_plan(a.B, a.T, a.H, &nseg, &seg_chunks);
-    if (rc == WKV6_OK) rc = nseg > 1 ? tc3_forward_segmented(with_raw_w(a, w_raw), flags, nseg, seg_chunks, nullptr, nullptr, true) : tc3_forward(with_raw_w(a, w_raw), nullptr, flags);
+    const size_t nw = (size_t)a.B * a.T * a.H * N * 2;
+    uint8_t *buf = nullptr;
+    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&buf, nw + (size_t)a.B * a.H * sizeof(int), a.stream));
+    int *flags = (int *)(buf + nw);
+    int rc = cudaMemsetAsync(flags, 0, (size_t)a.B * a.H * sizeof(int), a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
+    if (rc == WKV6_OK) rc = ew_to_raw_bf16(a.B, a.T, a.H, (const float *)a.w, buf, flags, a.stream, a.w_kind == W_DECAY_F32);
+    if (rc == WKV6_OK) rc = a.mask ? bi_forward_tc(with_raw_w(a, buf), flags) : forward3(with_raw_w(a, buf), flags);
     if (rc == WKV6_OK) {
         Args s = a;
         s.stream_flags = flags;
         rc = simt_forward(s);
     }
-    cudaFreeAsync(w_raw, a.stream);
+    cudaFreeAsync(buf, a.stream);
     return rc;
 }
+static int backward_ew(const Args &a) {
+    // workspace: [tensor-core backward workspace][raw bf16 logits][stream flags]
+    const size_t base = tc3_backward_workspace_bytes(a.B, a.T, a.H, false), nw = (size_t)a.B * a.T * a.H * N * 2;
+    const size_t need = base + nw + (size_t)a.B * a.H * sizeof(int);
+    if (!a.workspace || a.workspace_bytes < need) { set_error("workspace too small: need %zu bytes", need); return WKV6_EWORKSPACE; }
+    void *w_raw = (uint8_t *)a.workspace + base;
+    int *flags = (int *)((uint8_t *)w_raw + nw);
+    if (cudaMemsetAsync(flags, 0, (size_t)a.B * a.H * sizeof(int), a.stream) != cudaSuccess) { set_error("cudaMemsetAsync failed"); return WKV6_ECUDA; }
+    if (int rc = ew_to_raw_bf16(a.B, a.T, a.H, (const float *)a.w, w_raw, flags, a.stream)) return rc;
+    Args t = with_raw_w(a, w_raw);
+    t.workspace_bytes = base;
+    if (int rc = a.mask ? bi_backward_tc(t, flags) : tc3_backward(t, flags)) return rc;
+    Args s = a;                   // (the exact route's scratch is the front of the workspace)
+    s.stream_flags = flags;
+    return simt_backward(s);
+}
+
 static int dispatch_forward(const Args &a0) {
     Args a = a0;
     if (a.hi_lo < 0) a.hi_lo = a.sT != nullptr;      // one precision class for every internal pass of this call
     const int impl = current_impl();
     if (impl != WKV6_IMPL_SIMT && tc3_forward_supported(a)) return forward3(a);
-    if (impl != WKV6_IMPL_SIMT && ew_convertible(a) && !a.saved) return forward3_ew(a);
-    if (impl != WKV6_IMPL_SIMT && bi_forward_tc_supported(a) && !a.saved) {
-        wkv6::ensure_pool_keeps_memory();
-        const size_t nb = (size_t)a.B * a.H * sizeof(int);
-        int *flags = flag_slice((size_t)a.B * a.H);
-        if (!flags) { set_error("cannot get %zu bytes of flag scratch", nb); return WKV6_ECUDA; }
-        WKV6_CUDA_CHECK(cudaMemsetAsync(flags, 0, nb, a.stream));
-        return bi_forward_tc(a, flags);
-    }
+    if (impl != WKV6_IMPL_SIMT && bi_forward_tc_supported(a)) return bi_forward_tc(a, nullptr);
+    if (impl != WKV6_IMPL_SIMT && ew_convertible(a, false)) return forward_ew(a);
     if (impl == WKV6_IMPL_TC) { set_error("tensor-core forward does not support this call"); return WKV6_EUNSUPPORTED; }
     return simt_forward(a);
 }
 static int dispatch_backward(const Args &a) {
     const int impl = current_impl();
     if (impl != WKV6_IMPL_SIMT && tc3_backward_supported(a)) return tc3_backward(a);
-    if (impl != WKV6_IMPL_SIMT && a.mask && !a.saved && !a.s0 && bi_forward_tc_supported(a)) {
-        wkv6::ensure_pool_keeps_memory();
-        return bi_backward_tc(a);
-    }
-    if (impl != WKV6_IMPL_SIMT && a.w_kind == W_LOG_F32 && !a.saved && tc3_backward_supported(with_raw_w(a, const_cast<void *>(a.w)))) {
-        // workspace: [tensor-core backward workspace][raw bf16 logits]
-        const size_t base = tc3_backward_workspace_bytes(a.B, a.T, a.H, false), need = base + (size_t)a.B * a.T * a.H * 64 * 2;
-        if (!a.workspace || a.workspace_bytes < need) { set_error("workspace too small: need %zu bytes", need); return WKV6_EWORKSPACE; }
-        void *w_raw = (uint8_t *)a.workspace + base;
-        int *flags = (int *)((uint8_t *)a.workspace + simt_backward_workspace_bytes(a.B, a.T, a.H));
-        if (cudaMemsetAsync(flags, 0, (size_t)a.B * a.H * sizeof(int), a.stream) != cudaSuccess) { set_error("cudaMemsetAsync failed"); return WKV6_ECUDA; }
-        if (int rc = ew_to_raw_bf16(a.B, a.T, a.H, (const float *)a.w, w_raw, flags, a.stream)) return rc;
-        Args t = with_raw_w(a, w_raw);
-        t.workspace_bytes = base;
-        return tc3_backward(t, &a, true);
-    }
+    if (impl != WKV6_IMPL_SIMT && bi_forward_tc_supported(a)) return bi_backward_tc(a, nullptr);
+    if (impl != WKV6_IMPL_SIMT && ew_convertible(a, true)) return backward_ew(a);
     if (impl == WKV6_IMPL_TC) { set_error("tensor-core backward does not support this call"); return WKV6_EUNSUPPORTED; }
     return simt_backward(a);
 }
@@ -283,8 +242,8 @@ int wkv6_forward_raww(int B, int T, int C, int H, const void *r, const void *k, 
 }
 size_t wkv6_backward_workspace_bytes(int B, int T, int C, int H) {
     (void)C;
-    // superset: SIMT scratch + per-stream flags + chunk-start states (+ raw bf16 logits for the fp32-ew entries)
-    return tc3_backward_workspace_bytes(B, T, H, false) + (size_t)B * T * H * N * 2;
+    // superset: SIMT scratch + chunk-start states (+ raw bf16 logits and per-stream flags for the fp32-ew entries)
+    return tc3_backward_workspace_bytes(B, T, H, false) + (size_t)B * T * H * N * 2 + (size_t)B * H * sizeof(int);
 }
 int wkv6_backward(int B, int T, int C, int H, const void *r, const void *k, const void *v,
                   const float *ew, const void *u, const void *gy, void *gr, void *gk, void *gv,

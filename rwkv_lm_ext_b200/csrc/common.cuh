@@ -55,7 +55,7 @@ struct Args {
     // SIMT kernels only: nullptr, or one device int per (b,h) stream: block `s` runs only when
     // stream_flags[s] != 0 (lets the exact fallback be enqueued without a host round trip)
     const int *stream_flags = nullptr;
-    // training pair: forward fills it (per-stream hazard flags + bf16 chunk-start states), backward reads it
+    // training pair: forward fills it (gu arrival counters + bf16 chunk-start states), backward reads it
     void *saved = nullptr;
     cudaStream_t stream = nullptr;
 };
@@ -70,7 +70,11 @@ int simt_forward(const Args &a);
 int simt_backward(const Args &a);
 size_t simt_backward_workspace_bytes(int B, int T, int H);
 
-// role-uniform tcgen05 forward (per-stream hazard flags).  nseg > 1: every sequence is cut into nseg segments of
+// The tensor-core routes below take raw bf16 logits.  hz_flags / flags: nullptr (no stream is flagged), or one device int
+// per (b,h) stream; the kernels skip the flagged streams, which the caller recomputes on the exact SIMT kernels.  Only the
+// conversion of fp32 decays (capi.cu) flags streams: the tensor-core kernels never raise a flag.
+//
+// role-uniform tcgen05 forward.  nseg > 1: every sequence is cut into nseg segments of
 // seg_chunks 64-token chunks (the last may be shorter) that run as separate grid rows; s0 / sT / flags / ckpt
 // are then indexed by row = b*nseg + seg (seg_scan.cu)
 // bi != 0: one direction of the bidirectional op (tc3_common.cuh BI_CAUSAL / BI_REV) with per-row lengths row_len[B]
@@ -78,18 +82,19 @@ size_t simt_backward_workspace_bytes(int B, int T, int H);
 int tc3_forward(const Args &a, void *ckpt, int *hz_flags, int nseg = 1, int seg_chunks = 0, int bi = 0,
                 const int *row_len = nullptr, const int *row_order = nullptr);
 bool tc3_forward_supported(const Args &a);
-// role-uniform tcgen05 backward (+ per-stream SIMT fallback, which runs on `exact` when given: the
-// call as the caller made it, e.g. with the fp32 log-decay instead of the converted bf16 logits)
-int tc3_backward(const Args &a, const Args *exact = nullptr, bool flags_preset = false, bool run_fallback = true);
+// role-uniform tcgen05 backward
+int tc3_backward(const Args &a, int *flags = nullptr);
 int tc3_backward_bi(const Args &a, void *ckpt, int *flags, int bi, const int *row_len, const int *row_order);
-// wkv6_bi forward as two launches of the chunked forward kernel around a reverse-gather / combine pair
+// wkv6_bi forward and backward, both directions on the chunked tensor-core kernels
 int bi_forward_tc(const Args &a, int *flags);
 bool bi_forward_tc_supported(const Args &a);
-int bi_backward_tc(const Args &a);
+int bi_backward_tc(const Args &a, int *flags);
 // fp32 ew = -exp(w) (or decay = exp(-exp(w)) with from_decay) -> raw bf16 logits; raises flags[b*H+h] where the round trip is not exact
 int ew_to_raw_bf16(int B, int T, int H, const float *ew, void *w_raw, int *flags, cudaStream_t stream, int from_decay = 0);
 bool tc3_backward_supported(const Args &a);
-size_t tc3_saved_header(int B, int H);
+// `saved` of the training pair and the backward's own copy of it: the per-head arrival counters of the in-kernel gu sum
+// (H <= 512), then the bf16 chunk-start states
+constexpr size_t TC3_SAVED_HEADER = 512 * sizeof(int);
 size_t tc3_saved_bytes(int B, int T, int H);
 size_t tc3_backward_workspace_bytes(int B, int T, int H, bool has_saved);
 

@@ -11,8 +11,8 @@
 // everything that goes through ldmatrix / stmatrix, an in-place row swap for the two tiles the tensor cores read as
 // they arrive -- and ADDING its output tiles to the causal pass's with TMA reduce stores (bf16 accumulation across
 // the two passes, like the reference).  Forward: 2 launches; backward: per direction a state-only forward for the
-// chunk-start states and the backward kernel.  Streams whose fp32 decay does not convert exactly to bf16 logits are
-// recomputed by the exact SIMT bidirectional kernels, predicated per stream.
+// chunk-start states and the backward kernel.  Both take raw bf16 logits; the flagged streams (common.cuh) are left to
+// the caller's exact route.
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -65,29 +65,20 @@ static int dbg_sync(cudaStream_t st, const char *what) {
 bool bi_forward_tc_supported(const Args &a) {
     Args t = a;
     t.mask = nullptr;
-    if (t.w_kind == W_LOG_F32) t.w_kind = W_RAW_BF16;
     return a.mask != nullptr && a.s0 == nullptr && a.sT == nullptr && tc3_forward_supported(t);
 }
 
-// flags: device int [B*H], zeroed by the caller
 int bi_forward_tc(const Args &a, int *flags) {
     if (a.B * a.H == 0 || a.T == 0) return WKV6_OK;
-    const int C = a.H * N;
-    const size_t n = (size_t)a.B * a.T * C * sizeof(bf16);
-    const bool convert = a.w_kind == W_LOG_F32;
-    // stream-ordered scratch: zero u, row lengths, (raw logits when the caller passed fp32 -exp(w))
-    const size_t usz = ((size_t)a.H * N * sizeof(bf16) + 255) / 256 * 256, lsz = ((size_t)2 * a.B * sizeof(int) + 255) / 256 * 256;
+    // stream-ordered scratch, kept cached in the pool: zero u, row lengths
+    wkv6::ensure_pool_keeps_memory();
+    const size_t usz = ((size_t)a.H * N * sizeof(bf16) + 255) / 256 * 256;
     uint8_t *sc = nullptr;
-    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&sc, usz + lsz + (convert ? n : 0), a.stream));
+    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&sc, usz + (size_t)2 * a.B * sizeof(int), a.stream));
     bf16 *u0 = (bf16 *)sc;
     int *row_len = (int *)(sc + usz), *row_order = row_len + a.B;
-    const void *w_raw = a.w;
     int rc = WKV6_OK;
-    if (convert) {
-        w_raw = sc + usz + lsz;
-        rc = ew_to_raw_bf16(a.B, a.T, a.H, (const float *)a.w, const_cast<void *>(w_raw), flags, a.stream);
-    }
-    if (rc == WKV6_OK && cudaMemsetAsync(u0, 0, (size_t)a.H * N * sizeof(bf16), a.stream) != cudaSuccess) rc = WKV6_ECUDA;
+    if (cudaMemsetAsync(u0, 0, (size_t)a.H * N * sizeof(bf16), a.stream) != cudaSuccess) rc = WKV6_ECUDA;
     if (rc == WKV6_OK) {
         bi_last_kernel<<<a.B, 256, 0, a.stream>>>(a.T, a.mask, row_len);
         bi_order_kernel<<<1, 256, 0, a.stream>>>(a.B, row_len, row_order);
@@ -96,7 +87,7 @@ int bi_forward_tc(const Args &a, int *flags) {
     }
     if (rc == WKV6_OK) {
         Args f = a;                       // causal direction: stores y (zeros behind p)
-        f.mask = nullptr; f.w = w_raw; f.w_kind = W_RAW_BF16;
+        f.mask = nullptr;
         rc = tc3_forward(f, nullptr, flags, 1, 0, tc3::BI_CAUSAL, row_len, row_order);
         if (rc == WKV6_OK) rc = dbg_sync(a.stream, "forward, causal direction");
         if (rc == WKV6_OK) {              // reverse direction: u = 0, adds to y
@@ -105,45 +96,30 @@ int bi_forward_tc(const Args &a, int *flags) {
         }
         if (rc == WKV6_OK) rc = dbg_sync(a.stream, "forward, reverse direction");
     }
-    if (rc == WKV6_OK) {                  // exact route for the flagged streams (both passes), from the caller's own tensors
-        Args s = a;
-        s.stream_flags = flags;
-        rc = simt_forward(s);
-    }
     cudaFreeAsync(sc, a.stream);
     return rc;
 }
 
 // wkv6_bi backward: per direction, the chunk-start states (state-only forward) and the backward kernel; the reverse
-// direction adds its four gradient tiles to the causal direction's.  a.workspace must hold wkv6_backward_workspace_bytes
-// (the chunk-state checkpoints live there, one direction after the other).
-int bi_backward_tc(const Args &a) {
+// direction adds its four gradient tiles to the causal direction's.  a.workspace must hold
+// tc3_backward_workspace_bytes(B, T, H, false) (the chunk-state checkpoints live there, one direction after the other).
+int bi_backward_tc(const Args &a, int *flags) {
     if (a.B * a.H == 0 || a.T == 0) return WKV6_OK;
     const int C = a.H * N;
-    const size_t n = (size_t)a.B * a.T * C * sizeof(bf16);
-    const bool convert = a.w_kind == W_LOG_F32;
     const size_t base = tc3_backward_workspace_bytes(a.B, a.T, a.H, false);
     if (!a.workspace || a.workspace_bytes < base) { set_error("workspace too small: need %zu bytes", base); return WKV6_EWORKSPACE; }
-    const size_t nflag = (size_t)a.B * a.H * sizeof(int);
+    wkv6::ensure_pool_keeps_memory();
     const size_t usz = ((size_t)a.H * N * sizeof(bf16) + 255) / 256 * 256, lsz = ((size_t)2 * a.B * sizeof(int) + 255) / 256 * 256;
-    const size_t gsz = ((size_t)a.B * C * sizeof(bf16) + 255) / 256 * 256, fsz = (nflag + 255) / 256 * 256;
     uint8_t *sc = nullptr;
-    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&sc, usz + lsz + gsz + fsz + (convert ? n : 0), a.stream));
+    WKV6_CUDA_CHECK(cudaMallocAsync((void **)&sc, usz + lsz + (size_t)a.B * C * sizeof(bf16), a.stream));
     bf16 *u0 = (bf16 *)sc;
     int *row_len = (int *)(sc + usz), *row_order = row_len + a.B;
     bf16 *gu2 = (bf16 *)(sc + usz + lsz);
-    int *allflags = (int *)(sc + usz + lsz + gsz);
-    const void *w_raw = a.w;
-    if (convert) w_raw = sc + usz + lsz + gsz + fsz;
-    // the workspace is laid out as tc3_backward has it: [exact-route scratch][flags + chunk-state checkpoints]
-    uint8_t *sv = (uint8_t *)a.workspace + simt_backward_workspace_bytes(a.B, a.T, a.H);
-    int *wsflags = (int *)sv;
-    void *ckpt = sv + tc3_saved_header(a.B, a.H);
+    // the checkpoints sit where tc3_backward keeps them: behind the part of the workspace the caller's exact route uses
+    void *ckpt = (uint8_t *)a.workspace + simt_backward_workspace_bytes(a.B, a.T, a.H) + TC3_SAVED_HEADER;
     int rc = WKV6_OK;
     auto ck = [&](cudaError_t e) { if (e != cudaSuccess && rc == WKV6_OK) { set_error("wkv6_bi backward: %s", cudaGetErrorString(e)); rc = WKV6_ECUDA; } };
     ck(cudaMemsetAsync(u0, 0, (size_t)a.H * N * sizeof(bf16), a.stream));
-    ck(cudaMemsetAsync(wsflags, 0, nflag, a.stream));
-    if (rc == WKV6_OK && convert) rc = ew_to_raw_bf16(a.B, a.T, a.H, (const float *)a.w, const_cast<void *>(w_raw), wsflags, a.stream);
     if (rc == WKV6_OK) {
         bi_last_kernel<<<a.B, 256, 0, a.stream>>>(a.T, a.mask, row_len);
         bi_order_kernel<<<1, 256, 0, a.stream>>>(a.B, row_len, row_order);
@@ -151,21 +127,14 @@ int bi_backward_tc(const Args &a) {
         ck(cudaGetLastError());
     }
     Args d = a;
-    d.mask = nullptr; d.w = w_raw; d.w_kind = W_RAW_BF16; d.stream_flags = nullptr;
-    if (rc == WKV6_OK) rc = tc3_backward_bi(d, ckpt, wsflags, tc3::BI_CAUSAL, row_len, row_order);
+    d.mask = nullptr;
+    if (rc == WKV6_OK) rc = tc3_backward_bi(d, ckpt, flags, tc3::BI_CAUSAL, row_len, row_order);
     if (rc == WKV6_OK) rc = dbg_sync(a.stream, "backward, causal direction");
     if (rc == WKV6_OK) {
         d.u = u0; d.gu = gu2;
-        rc = tc3_backward_bi(d, ckpt, wsflags, tc3::BI_REV, row_len, row_order);
+        rc = tc3_backward_bi(d, ckpt, flags, tc3::BI_REV, row_len, row_order);
     }
     if (rc == WKV6_OK) rc = dbg_sync(a.stream, "backward, reverse direction");
-    if (rc == WKV6_OK) ck(cudaMemcpyAsync(allflags, wsflags, nflag, cudaMemcpyDeviceToDevice, a.stream));
-    if (rc == WKV6_OK) {          // exact bidirectional backward for the flagged streams, from the caller's own tensors
-        Args s = a;
-        s.stream_flags = allflags;
-        s.workspace_bytes = simt_backward_workspace_bytes(a.B, a.T, a.H);
-        rc = simt_backward(s);
-    }
     cudaFreeAsync(sc, a.stream);
     return rc;
 }

@@ -94,7 +94,7 @@ struct Params {
     bf16 *gu, *gs;
     bf16 *gu_total;           // nullptr, or bf16 [C]: sum of gu over the grid's rows, added up by the last CTA of every head
     int *gu_count;            // its arrival counters, int [H], zero before the launch (left zero again)
-    const int *hz_flags;
+    const int *hz_flags;      // nullptr, or [rows*H]: 1 = this stream needs the exact route
     const int *row_len;       // BI modes: tokens of every batch row (p + 1 of wkv6_bi), device int [B]
     const int *row_order;     // BI modes: batch rows sorted by length, longest first, device int [B]
     long long *dbg;           // nullptr, or [gridDim][NC][8 (32 in the profiling build)] clock64 stamps of warp 0 at the stage boundaries (profiling aid)
@@ -116,7 +116,7 @@ wkv6_tc3_bwd_kernel(const __grid_constant__ CUtensorMap map_r, const __grid_cons
     const int h = blockIdx.x % p.H;
     const int row = BI ? p.row_order[blockIdx.x / p.H] : blockIdx.x / p.H;
     const int rid = BI ? row * p.H + h : blockIdx.x;     // row id: flags, checkpoints
-    if (p.hz_flags[rid] != 0) return;               // the exact (SIMT) route handles this stream
+    if (p.hz_flags && p.hz_flags[rid] != 0) return; // the exact (SIMT) route handles this stream
     extern __shared__ __align__(1024) uint8_t sm[];
     Extra &ex = *reinterpret_cast<Extra *>(sm + OFF_TILES_END);
     if ((smem_u32(sm) & 1023u) != 0) __trap();
@@ -925,14 +925,12 @@ wkv6_tc3_bwd_kernel(const __grid_constant__ CUtensorMap map_r, const __grid_cons
 void *g_tc3_bwd_stamps = nullptr;   // profiling build: set through wkv6b200_debug_stamps()
 #endif
 
-// per-stream hazard flags [B*H], then (time-axis segmentation, at most 296 segment rows) per-segment flags
-size_t tc3_saved_header(int B, int H) { return ((((size_t)B * H + 512) * sizeof(int)) + 1023) / 1024 * 1024; }
 size_t tc3_saved_bytes(int B, int T, int H) {
     size_t NC = (size_t)(T + L - 1) / L;
     int nseg = 1, seg_chunks = 0;
     seg_plan_train(B, T, H, &nseg, &seg_chunks);           // uneven segments leave a few checkpoint slots unused
     if (nseg > 1) NC = (size_t)nseg * seg_chunks;
-    return tc3_saved_header(B, H) + (size_t)B * H * NC * 8192;
+    return TC3_SAVED_HEADER + (size_t)B * H * NC * 8192;
 }
 // scratch of the time-segmented backward (seg_scan.cu): r, gy, w reversed inside the segments, the segments'
 // own and scanned state gradients, decay sums, per-row gs and gu
@@ -958,7 +956,7 @@ __global__ void __launch_bounds__(256) clamp_gw_kernel(size_t n8, const bf16 *__
     const size_t C = (size_t)H * 64;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n8; i += (size_t)gridDim.x * blockDim.x) {
         const size_t e0 = 8 * i, bt = e0 / C, b = bt / T, h = (e0 % C) / 64;
-        if (flags[(b * nseg) * H + h] != 0) continue;             // the exact route writes its own gw
+        if (flags && flags[(b * nseg) * H + h] != 0) continue;    // the exact route writes its own gw
         const uint4 wv = *reinterpret_cast<const uint4 *>(w + e0);
         uint4 gv = *reinterpret_cast<const uint4 *>(gw + e0);
         const __nv_bfloat16 *wp = reinterpret_cast<const __nv_bfloat16 *>(&wv);
@@ -989,9 +987,11 @@ static int launch_bwd_kernel(dim3 grid, cudaStream_t stream, const CUtensorMap *
 }
 
 // one launch of the backward kernel on `a` viewed as given (B rows of T tokens), chunk-start states in ckpt
+// gu_count: nullptr, or the zeroed per-head arrival counters that let an ordinary call add gu up into a.gu_total
 // bi / row_len: direction of the bidirectional op (tc3_common.cuh) and the device int [B] row lengths it needs
-static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, const float *g_init, int nseg, int seg_chunks,
-                      bool has_s0, int bi = BI_NONE, const int *row_len = nullptr, const int *row_order = nullptr) {
+static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu_count, const float *g_init, int nseg,
+                      int seg_chunks, bool has_s0, int bi = BI_NONE, const int *row_len = nullptr,
+                      const int *row_order = nullptr) {
     const int C = a.H * 64;
     if (nseg <= 1) { nseg = 1; seg_chunks = (a.T + L - 1) / L; }
     const size_t NC = (size_t)nseg * seg_chunks;
@@ -1016,10 +1016,10 @@ static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, const f
     p.lmin = tc_lmin_log2(a);
     p.gu = (bf16 *)a.gu; p.gs = (bf16 *)a.gs;
     p.hz_flags = flags;
-    // in-kernel sum of gu over the rows: ordinary call only; the counters sit behind the stream flags (zeroed with them)
-    const bool sum_gu = a.gu_total && nseg == 1 && bi == BI_NONE && a.H <= 512;
+    // in-kernel sum of gu over the rows: ordinary call only
+    const bool sum_gu = a.gu_total && gu_count && nseg == 1 && bi == BI_NONE && a.H <= 512;
     p.gu_total = sum_gu ? (bf16 *)a.gu_total : nullptr;
-    p.gu_count = const_cast<int *>(flags) + (size_t)a.B * a.H;
+    p.gu_count = gu_count;
     if (sum_gu) a.gu_total_done = true;
 #ifdef WKV6_FINE_STAMPS
     p.dbg = (long long *)g_tc3_bwd_stamps;
@@ -1052,11 +1052,10 @@ static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, const f
 // so: reverse the three tensors inside every segment, a state-only forward pass (k := r_rev, v := gy_rev) gives
 // each segment's own contribution, a reverse scan over the segments chains them, and the ordinary backward
 // kernel starts every segment from its scanned G.  The forward of the training pair was segmented the same
-// way, so `saved` holds the chunk-start states in segment-row order and the per-segment flags.
+// way, so `saved` holds the chunk-start states in segment-row order.
 static int tc3_backward_segmented(const Args &a, int nseg, int seg_chunks) {
     const int Bs = a.B * nseg, C = a.H * 64, seg_tokens = seg_chunks * L;
-    int *flags = (int *)a.saved, *sflags = flags + (size_t)a.B * a.H;
-    const bf16 *ckpt = (const bf16 *)((uint8_t *)a.saved + tc3_saved_header(a.B, a.H));
+    const bf16 *ckpt = (const bf16 *)((uint8_t *)a.saved + TC3_SAVED_HEADER);
     const size_t n_el = (size_t)a.B * a.T * C, st = (size_t)Bs * a.H * 4096;
     // scratch lives in the caller's workspace, behind the part the exact route uses
     const size_t simt_ws = (simt_backward_workspace_bytes(a.B, a.T, a.H) + 1023) / 1024 * 1024;
@@ -1068,17 +1067,17 @@ static int tc3_backward_segmented(const Args &a, int nseg, int seg_chunks) {
     Args f = a;                                   // state-only pass: the "state" it ends with is each segment's own dL/dS_start
     f.r = r_rev; f.k = r_rev; f.v = gy_rev; f.w = w_rev;
     f.s0 = nullptr; f.s0_bstride = 0; f.s0_f32 = 0; f.sT = g_loc; f.sT_f32 = 1; f.y = nullptr; f.saved = nullptr; f.gy = nullptr;
-    if (rc == WKV6_OK) rc = tc3_forward(f, nullptr, sflags, nseg, seg_chunks);
+    if (rc == WKV6_OK) rc = tc3_forward(f, nullptr, nullptr, nseg, seg_chunks);
     if (rc == WKV6_OK) rc = seg_decay(a.B, a.T, C, nseg, seg_tokens, a.w, lam, tc_lmin_nats(a), a.stream);
     if (rc == WKV6_OK) rc = seg_scan(a.B, nseg, a.H, lam, g_loc, nullptr, 0, 0, g_end, nullptr, 0, 1, nullptr, a.stream);
     Args v = a;
     v.gu = gu_tmp; v.gs = a.gs ? gs_tmp : nullptr;
-    if (rc == WKV6_OK) rc = launch_bwd(v, ckpt, sflags, g_end, nseg, seg_chunks, a.s0 != nullptr);
+    if (rc == WKV6_OK) rc = launch_bwd(v, ckpt, nullptr, nullptr, g_end, nseg, seg_chunks, a.s0 != nullptr);
     if (rc == WKV6_OK) rc = seg_sum_gu(a.B, nseg, C, gu_tmp, a.gu, a.stream);
     if (rc == WKV6_OK && a.gs)                    // dL/dS_0 is what segment 0 of every sequence produced
         rc = cudaMemcpy2DAsync(a.gs, (size_t)a.H * 4096 * 2, gs_tmp, (size_t)nseg * a.H * 4096 * 2, (size_t)a.H * 4096 * 2, a.B,
                                cudaMemcpyDeviceToDevice, a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
-    return rc;      // (training pair on raw bf16 logits: no stream is ever flagged, no exact-route launch follows)
+    return rc;
 }
 
 // One direction of the bidirectional backward (wkv6_bi_tc.cu): recompute the chunk-start states of that direction
@@ -1088,44 +1087,34 @@ int tc3_backward_bi(const Args &a, void *ckpt, int *flags, int bi, const int *ro
     Args f = a;
     f.y = nullptr; f.sT = nullptr; f.s0 = nullptr;
     if (int rc = tc3_forward(f, ckpt, flags, 1, 0, bi, row_len, row_order)) return rc;
-    return launch_bwd(a, (const bf16 *)ckpt, flags, nullptr, 1, 0, false, bi, row_len, row_order);
+    return launch_bwd(a, (const bf16 *)ckpt, flags, nullptr, nullptr, 1, 0, false, bi, row_len, row_order);
 }
 
-int tc3_backward(const Args &a, const Args *exact, bool flags_preset, bool run_fallback) {
+int tc3_backward(const Args &a, int *flags) {
     if (a.B * a.H == 0 || a.T == 0) return WKV6_OK;
-    const size_t simt_ws = simt_backward_workspace_bytes(a.B, a.T, a.H);
     const size_t need = tc3_backward_workspace_bytes(a.B, a.T, a.H, a.saved != nullptr);
     if (!a.workspace || a.workspace_bytes < need) {
         set_error("workspace too small: need %zu bytes", need);
         return WKV6_EWORKSPACE;
     }
-    if (a.saved && !exact && run_fallback) {
+    if (a.saved) {
         int nseg = 1, seg_chunks = 0;
         seg_plan_train(a.B, a.T, a.H, &nseg, &seg_chunks);
         if (nseg > 1) return tc3_backward_segmented(a, nseg, seg_chunks);
     }
-    uint8_t *sv = a.saved ? (uint8_t *)a.saved : (uint8_t *)a.workspace + simt_ws;
-    int *flags = (int *)sv;
-    bf16 *ckpt = (bf16 *)(sv + tc3_saved_header(a.B, a.H));
+    // `saved`, or without a training pair the same layout in the workspace, behind the part the caller's exact route uses
+    uint8_t *sv = a.saved ? (uint8_t *)a.saved : (uint8_t *)a.workspace + simt_backward_workspace_bytes(a.B, a.T, a.H);
+    int *gu_count = (int *)sv;
+    bf16 *ckpt = (bf16 *)(sv + TC3_SAVED_HEADER);
     if (!a.saved) {
-        // no training pair: recompute the chunk-start states (and the per-stream hazard flags) first
-        if (!flags_preset) WKV6_CUDA_CHECK(cudaMemsetAsync(flags, 0, ((size_t)a.B * a.H + 512) * sizeof(int), a.stream));
-        else WKV6_CUDA_CHECK(cudaMemsetAsync(flags + (size_t)a.B * a.H, 0, 512 * sizeof(int), a.stream));
+        // recompute the chunk-start states first
+        if (a.gu_total) WKV6_CUDA_CHECK(cudaMemsetAsync(gu_count, 0, TC3_SAVED_HEADER, a.stream));
         Args f = a;
         f.y = nullptr;
         f.sT = nullptr;
         if (int rc = tc3_forward(f, ckpt, flags)) return rc;
     }
-    if (int rc = launch_bwd(a, ckpt, flags, nullptr, 1, 0, a.s0 != nullptr)) return rc;
-    if (!run_fallback) return WKV6_OK;      // the caller runs its own exact route on the flags in the workspace
-    // Flags are only ever raised by the fp32-decay conversion (flags_preset); a call on raw bf16 logits has none
-    if (!flags_preset && !exact) return WKV6_OK;
-    // exact route for the flagged streams only
-    Args s = exact ? *exact : a;
-    s.workspace = a.workspace;
-    s.stream_flags = flags;
-    s.workspace_bytes = simt_ws;
-    return simt_backward(s);
+    return launch_bwd(a, ckpt, flags, gu_count, nullptr, 1, 0, a.s0 != nullptr);
 }
 
 }  // namespace wkv6

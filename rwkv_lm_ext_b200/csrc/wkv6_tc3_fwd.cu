@@ -60,7 +60,7 @@ struct Params {
     void *sT;
     int sT_f32;
     int has_y, has_ckpt;
-    int *hz_flags;            // [rows*H]: 1 = this stream needs the exact route
+    int *hz_flags;            // nullptr, or [rows*H]: 1 = this stream needs the exact route
     // time-axis segmentation (seg_scan.cu): the grid has B*nseg rows; row = b*nseg + seg covers tokens
     // [seg*seg_chunks*64, min(T, (seg+1)*seg_chunks*64)) of sequence b.  States (s0, sT), flags and the
     // checkpoints are indexed by row; nseg = 1 and seg_chunks = ceil(T/64) for an ordinary call.
@@ -88,7 +88,7 @@ wkv6_tc3_fwd_kernel(const __grid_constant__ CUtensorMap map_r, const __grid_cons
     const int h = blockIdx.x % p.H;
     const int row = BI ? p.row_order[blockIdx.x / p.H] : blockIdx.x / p.H;
     const int rid = BI ? row * p.H + h : blockIdx.x;     // row id: flags, checkpoints
-    if (p.hz_flags[rid] != 0) return;               // flagged before launch (inexact logit conversion): exact route
+    if (p.hz_flags && p.hz_flags[rid] != 0) return; // flagged before launch (inexact logit conversion): exact route
     extern __shared__ __align__(1024) uint8_t sm[];
     Extra &ex = *reinterpret_cast<Extra *>(sm + OFF_TILES_END);
     if ((smem_u32(sm) & 1023u) != 0) __trap();
@@ -602,7 +602,7 @@ bool tc3_forward_supported(const Args &a) {
 }
 
 // ckpt: nullptr or bf16 [B*H][ceil(T/64)][64 i][64 j] receiving the state at the start of every chunk;
-// hz_flags: device int [B*H], zeroed by the caller; a.y may be nullptr (state-only pass).
+// hz_flags: nullptr or device int [B*H] (see common.cuh); a.y may be nullptr (state-only pass).
 // bi / row_len: direction of the bidirectional op (tc3_common.cuh) and the device int [B] row lengths it needs.
 template <bool SEG, bool SO, int BI, bool KLO>
 static int launch_fwd(dim3 grid, cudaStream_t stream, const CUtensorMap &mr, const CUtensorMap &mk, const CUtensorMap &mv,

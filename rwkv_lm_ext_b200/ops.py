@@ -50,29 +50,29 @@ def _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, sT, y):
           "wkv6_train_forward")
     ctx.saved_state = saved if valid.value else None
     if _diag["collect"] and ctx.saved_state is not None:
-        _diag["flags"].append(saved[: B * H * 4].view(torch.int32).view(B, H))    # a view, no synchronisation
+        _diag["streams"] += B * H
 
 
-# Diagnostics: which (b,h) streams left the tensor-core kernels for the exact SIMT route (their decay is
-# stronger than the block references allow, DESIGN.md 4.0) -- e.g. to see what a real checkpoint does.
-_diag = {"collect": False, "flags": []}
+# Diagnostics: how many (b,h) streams of the training forwards left the tensor-core kernels for the exact SIMT route.
+# None does: the block references and the decay floor cover every decay (DESIGN.md 4.0), and only an fp32 decay that is
+# not a bf16 logit -- never the training pair's raw logits -- is handed to the exact kernels.
+_diag = {"collect": False, "streams": 0}
 
 
 class exact_route_report:
     """with exact_route_report() as rep: ...training forwards...;  rep.streams() -> (flagged, total)"""
 
     def __enter__(self):
-        _diag["collect"], _diag["flags"] = True, []
+        _diag["collect"], _diag["streams"] = True, 0
         return self
 
     def __exit__(self, *exc):
-        self._flags = _diag["flags"]
-        _diag["collect"], _diag["flags"] = False, []
+        self._streams = _diag["streams"]
+        _diag["collect"], _diag["streams"] = False, 0
         return False
 
     def streams(self):
-        flagged = sum(int((f != 0).sum().item()) for f in self._flags)
-        return flagged, sum(f.numel() for f in self._flags)
+        return 0, self._streams
 
 
 def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs):

@@ -1,4 +1,4 @@
-"""One process driving two devices in turn (per-device kernel attributes, flag rings, memory pools).  Needs two
+"""One process driving two devices in turn (per-device kernel attributes and memory pools).  Needs two
 GPUs: skipped on a single-GPU box.  `pytest -m gpu`."""
 import pytest
 import torch

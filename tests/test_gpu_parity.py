@@ -740,8 +740,8 @@ def test_segmented_training_pair(M, with_state):
 
 
 def test_concurrent_streams_do_not_share_scratch(M):
-    """Calls in flight on different CUDA streams (forward-only path: hazard flags come from the library's static
-    ring; one of the inputs has a hazardous stream so the flags matter) give the same results as serial calls."""
+    """Calls in flight on different CUDA streams (forward-only path on raw logits; one of the inputs has a stream with
+    decays far beyond the block references) give the same results as serial calls."""
     B, T, H = 2, 320, 3
     C = H * 64
     sets = []
@@ -762,6 +762,66 @@ def test_concurrent_streams_do_not_share_scratch(M):
         torch.cuda.synchronize()
     for a, b_ in zip(outs, serial):
         assert torch.equal(a, b_)
+
+
+def test_concurrent_fp32_decay_entries(M):
+    """wkv6_cuda.forward / .backward (fp32 -exp(w), one stream per input set not representable as bf16 logits) in flight
+    on four CUDA streams at once: every call keeps its stream flags in its own stream-ordered scratch (forward) or
+    workspace (backward), so the results equal serial calls bit for bit."""
+    B, T, H = 2, 320, 3
+    C = H * 64
+    sets = []
+    for i in range(4):
+        r, k, v, w, u, gy = make_inputs(B, T, H, seed=90 + i, decay="model", device=DEV)
+        ew = -torch.exp(w.float())
+        b, c0 = i % B, 64 * (i % H)
+        ew[b, :, c0:c0 + 64] = -torch.exp(w.float()[b, :, c0:c0 + 64] + 0.001)
+        sets.append((r, k, v, ew.contiguous(), u, gy))
+
+    def run(r, k, v, ew, u, gy):
+        y = torch.empty_like(r)
+        M.wkv6_cuda.forward(B, T, C, H, r, k, v, ew, u, y)
+        g = [torch.empty_like(r) for _ in range(4)]
+        gu = torch.empty(B, C, device=DEV, dtype=torch.bfloat16)
+        M.wkv6_cuda.backward(B, T, C, H, r, k, v, ew, u, gy, *g, gu)
+        return [y, *g, gu]
+
+    serial = [run(*s) for s in sets]
+    torch.cuda.synchronize()
+    streams = [torch.cuda.Stream() for _ in range(4)]
+    outs = [None] * 4
+    for rep in range(5):
+        for i, st in enumerate(streams):
+            with torch.cuda.stream(st):
+                outs[i] = run(*sets[i])
+    torch.cuda.synchronize()
+    for a, b_ in zip(outs, serial):
+        for x, x_serial, name in zip(a, b_, ("y", "gr", "gk", "gv", "gw", "gu")):
+            assert torch.equal(x, x_serial), name
+
+
+def test_launch_counts_on_raw_logits(M):
+    """Raw bf16 logits carry no stream flags: the calls launch their tensor-core kernels and nothing else (no exact-route
+    launch whose blocks would all exit at once)."""
+    B, T, H = 2, 192, 2
+    C = H * 64
+    r, k, v, w, u, gy = make_inputs(B, T, H, seed=95, decay="model", device=DEV)
+    mask = torch.ones(B, T, dtype=torch.int32, device=DEV)
+    mask[0, 150:] = 0
+
+    def launches(fn):
+        n0 = M.launch_count()
+        out = fn()
+        return M.launch_count() - n0, out
+
+    with torch.no_grad():
+        assert launches(lambda: M.RUN_CUDA_RWKV6(B, T, C, H, r, k, v, w, u))[0] == 1
+    leaves = [t.clone().requires_grad_(True) for t in (r, k, v, w, u)]
+    assert launches(lambda: M.RUN_CUDA_RWKV6(B, T, C, H, *leaves).backward(gy))[0] == 2     # forward + backward kernel
+    leaves = [t.clone().requires_grad_(True) for t in (r, k, v, w, u)]
+    n, y = launches(lambda: M.RUN_CUDA_RWKV6_BI(B, T, C, H, mask, *leaves))
+    assert n == 4                 # row lengths, row order, causal and reverse forward
+    assert launches(lambda: y.backward(gy))[0] == 6      # row lengths, row order, per direction: states + backward
 
 
 def test_decay_clamp_opt_in(M, O):
