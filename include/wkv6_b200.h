@@ -197,6 +197,12 @@ WKV6_API int rwkv6_forward_raww(int B, int T, int C, int H, float *state, const 
 
 /* ------------------------------------------------------------------------------------------
  * Memory-bound neighbours of the recurrence.
+ * Their kernels read and write tensors with 16-byte vector accesses: every tensor argument of these
+ * entries, and of their gradients and the channel-mix pieces below, must start at a 16-byte aligned
+ * address (a contiguous view at an element offset, x[1:], does not).  A misaligned pointer is rejected
+ * with WKV6_EINVAL, naming the argument, before anything is launched.  int64 index tensors, fp32
+ * pooling outputs, fp32 parameter gradients and workspaces are exempt, and so are gather_rows_bf16,
+ * gather_tokens_bf16 and pooling_bf16 when D % 8 != 0 (they then copy element by element).
  * ------------------------------------------------------------------------------------------ */
 /* (a9) pos[b] = first t with idx[b,t]==token_id, 0 if absent
  * (== torch.eq(idx,id).int().argmax(-1), src/model_ext.py:209,1765); idx int64 [B,T]; pos int64 [B]. */
@@ -231,7 +237,8 @@ WKV6_API int tmix_ddlerp_mix_bf16(int B, int T, int C, const void *x, const void
 /* The same with the rank-R LoRA product fused in (src/model.py:442-448): m_n = h_n @ W2_n is computed on
  * the tensor cores inside the kernel and never written to memory.  h bf16 [B*T, 5*R] = tanh(xxx @ W1)
  * (row-major, the five R-wide slices side by side), w2 bf16 [5,R,C], out bf16 [5,B,T,C].
- * R = 32 and C % 64 == 0 only (WKV6_EUNSUPPORTED otherwise: use a bmm + tmix_ddlerp_mix_bf16). */
+ * R = 32 and C % 64 == 0 only (WKV6_EUNSUPPORTED otherwise: use a bmm + tmix_ddlerp_mix_bf16).
+ * Misaligned tensors are WKV6_EINVAL, as for every entry of this section. */
 WKV6_API int tmix_ddlerp_lora_bf16(int B, int T, int C, int R, const void *x, const void *shift_state,
                           const void *maa, const void *h, const void *w2, void *out, void *stream);
 /* xxx = x + (shift(x)-x)*maa_x  (src/model.py:439-441), the LoRA input.  bf16. */

@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 from ._lib import check, ptr, stream_of
-from .heads import _bf16_param, _cuda, _needs_grad, _ws
+from .heads import _bf16_param, _cuda, _dense, _needs_grad, _ws
 
 
 class _ShiftLerp2(torch.autograd.Function):
@@ -29,8 +29,8 @@ class _ShiftLerp2(torch.autograd.Function):
         x, shift_state, maa_kr = ctx.saved_tensors
         lib = _lib.load()
         B, T, C = x.shape
-        gxk = torch.zeros_like(x) if gxk is None else gxk.contiguous()
-        gxr = torch.zeros_like(x) if gxr is None else gxr.contiguous()
+        gxk = torch.zeros_like(x) if gxk is None else _dense(gxk)
+        gxr = torch.zeros_like(x) if gxr is None else _dense(gxr)
         gx = torch.empty_like(x)
         gmaa = torch.empty(2, C, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[2] else None
         gshift = torch.empty_like(shift_state) if shift_state is not None else None
@@ -53,7 +53,7 @@ def cmix_shift_lerp2(x, maa_k, maa_r, shift_state=None):
     """(xk, xr) of src/model.py:637-639."""
     _cuda(x)
     assert x.dtype == torch.bfloat16
-    x = x.contiguous()
+    x = _dense(x)
     C = x.shape[-1]
     maa_kr = _bf16_param(torch.cat([maa_k.reshape(1, C), maa_r.reshape(1, C)], 0))      # (two [C] rows: a 3 us launch)
     shift_state = _bf16_param(shift_state)
@@ -73,7 +73,7 @@ class _ReluSq(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gy):
         (x,) = ctx.saved_tensors
-        gy = gy.contiguous()
+        gy = _dense(gy)
         gx = torch.empty_like(x)
         check(_lib.load().relu_sq_backward_bf16(x.numel(), ptr(x), ptr(gy), ptr(gx), stream_of(x)), "relu_sq_backward_bf16")
         return gx
@@ -83,7 +83,7 @@ def relu_sq(x):
     """torch.relu(x) ** 2  (src/model.py:642)."""
     _cuda(x)
     assert x.dtype == torch.bfloat16
-    x = x.contiguous()
+    x = _dense(x)
     if x.numel() % 8:
         return torch.relu(x) ** 2
     return _ReluSq.apply(x)
@@ -100,7 +100,7 @@ class _SigmoidMul(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gout):
         r, kv = ctx.saved_tensors
-        gout = gout.contiguous()
+        gout = _dense(gout)
         gr, gkv = torch.empty_like(r), torch.empty_like(kv)
         check(_lib.load().sigmoid_mul_backward_bf16(r.numel(), ptr(r), ptr(kv), ptr(gout), ptr(gr), ptr(gkv), stream_of(r)),
               "sigmoid_mul_backward_bf16")
@@ -111,7 +111,7 @@ def sigmoid_mul(r, kv):
     """torch.sigmoid(r) * kv  (src/model.py:644)."""
     _cuda(r)
     assert r.dtype == torch.bfloat16 and kv.dtype == torch.bfloat16 and r.shape == kv.shape
-    r, kv = r.contiguous(), kv.contiguous()
+    r, kv = _dense(r), _dense(kv)
     if r.numel() % 8:
         return torch.sigmoid(r) * kv
     return _SigmoidMul.apply(r, kv)

@@ -132,8 +132,6 @@ __global__ void __launch_bounds__(256) sigmoid_mul_bwd_kernel(size_t nvec, const
     }
 }
 
-inline bool ok16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
 }  // namespace
 }  // namespace wkv6
 
@@ -146,6 +144,7 @@ int cmix_shift_lerp2_bf16(int B, int T, int C, const void *x, const void *shift_
     if (B < 0 || T < 0 || C <= 0 || (C & 7)) { set_error("cmix_shift_lerp2_bf16: need C %% 8 == 0"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!x || !maa_kr || !out) { set_error("cmix_shift_lerp2_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("cmix_shift_lerp2_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa_kr", maa_kr}, {"out", out}})) return WKV6_EINVAL;
     shift_lerp_n_kernel<2><<<grid_for((size_t)B * T * C / 8, 256), 256, 0, (cudaStream_t)stream>>>(
         B, T, C, (const bf16 *)x, (const bf16 *)shift_state, (const bf16 *)maa_kr, (bf16 *)out);
     count_launch();
@@ -155,7 +154,8 @@ int cmix_shift_lerp2_bf16(int B, int T, int C, const void *x, const void *shift_
 
 int relu_sq_bf16(size_t n, const void *x, void *y, void *stream) {
     if (n == 0) return WKV6_OK;
-    if (!x || !y || (n & 7) || !ok16(x) || !ok16(y)) { set_error("relu_sq_bf16: need n %% 8 == 0 and 16-byte aligned pointers"); return WKV6_EINVAL; }
+    if (!x || !y || (n & 7)) { set_error("relu_sq_bf16: need n %% 8 == 0 and non-null pointers"); return WKV6_EINVAL; }
+    if (!check_aligned16("relu_sq_bf16", {{"x", x}, {"y", y}})) return WKV6_EINVAL;
     relu_sq_kernel<<<grid_for(n / 8, 256), 256, 0, (cudaStream_t)stream>>>(n / 8, (const bf16 *)x, (bf16 *)y);
     count_launch();
     WKV6_CUDA_CHECK(cudaGetLastError());
@@ -164,7 +164,8 @@ int relu_sq_bf16(size_t n, const void *x, void *y, void *stream) {
 
 int relu_sq_backward_bf16(size_t n, const void *x, const void *gy, void *gx, void *stream) {
     if (n == 0) return WKV6_OK;
-    if (!x || !gy || !gx || (n & 7) || !ok16(x) || !ok16(gy) || !ok16(gx)) { set_error("relu_sq_backward_bf16: need n %% 8 == 0 and 16-byte aligned pointers"); return WKV6_EINVAL; }
+    if (!x || !gy || !gx || (n & 7)) { set_error("relu_sq_backward_bf16: need n %% 8 == 0 and non-null pointers"); return WKV6_EINVAL; }
+    if (!check_aligned16("relu_sq_backward_bf16", {{"x", x}, {"gy", gy}, {"gx", gx}})) return WKV6_EINVAL;
     relu_sq_bwd_kernel<<<grid_for(n / 8, 256), 256, 0, (cudaStream_t)stream>>>(n / 8, (const bf16 *)x, (const bf16 *)gy, (bf16 *)gx);
     count_launch();
     WKV6_CUDA_CHECK(cudaGetLastError());
@@ -173,7 +174,8 @@ int relu_sq_backward_bf16(size_t n, const void *x, const void *gy, void *gx, voi
 
 int sigmoid_mul_bf16(size_t n, const void *r, const void *kv, void *out, void *stream) {
     if (n == 0) return WKV6_OK;
-    if (!r || !kv || !out || (n & 7) || !ok16(r) || !ok16(kv) || !ok16(out)) { set_error("sigmoid_mul_bf16: need n %% 8 == 0 and 16-byte aligned pointers"); return WKV6_EINVAL; }
+    if (!r || !kv || !out || (n & 7)) { set_error("sigmoid_mul_bf16: need n %% 8 == 0 and non-null pointers"); return WKV6_EINVAL; }
+    if (!check_aligned16("sigmoid_mul_bf16", {{"r", r}, {"kv", kv}, {"out", out}})) return WKV6_EINVAL;
     sigmoid_mul_kernel<<<grid_for(n / 8, 256), 256, 0, (cudaStream_t)stream>>>(n / 8, (const bf16 *)r, (const bf16 *)kv, (bf16 *)out);
     count_launch();
     WKV6_CUDA_CHECK(cudaGetLastError());
@@ -182,10 +184,8 @@ int sigmoid_mul_bf16(size_t n, const void *r, const void *kv, void *out, void *s
 
 int sigmoid_mul_backward_bf16(size_t n, const void *r, const void *kv, const void *gout, void *gr, void *gkv, void *stream) {
     if (n == 0) return WKV6_OK;
-    if (!r || !kv || !gout || !gr || !gkv || (n & 7) || !ok16(r) || !ok16(kv) || !ok16(gout) || !ok16(gr) || !ok16(gkv)) {
-        set_error("sigmoid_mul_backward_bf16: need n %% 8 == 0 and 16-byte aligned pointers");
-        return WKV6_EINVAL;
-    }
+    if (!r || !kv || !gout || !gr || !gkv || (n & 7)) { set_error("sigmoid_mul_backward_bf16: need n %% 8 == 0 and non-null pointers"); return WKV6_EINVAL; }
+    if (!check_aligned16("sigmoid_mul_backward_bf16", {{"r", r}, {"kv", kv}, {"gout", gout}, {"gr", gr}, {"gkv", gkv}})) return WKV6_EINVAL;
     sigmoid_mul_bwd_kernel<<<grid_for(n / 8, 256), 256, 0, (cudaStream_t)stream>>>(n / 8, (const bf16 *)r, (const bf16 *)kv,
                                                                                   (const bf16 *)gout, (bf16 *)gr, (bf16 *)gkv);
     count_launch();

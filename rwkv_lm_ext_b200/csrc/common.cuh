@@ -6,6 +6,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <initializer_list>
+
 #include "../../include/wkv6_b200.h"
 
 namespace wkv6 {
@@ -101,6 +103,20 @@ size_t tc3_backward_workspace_bytes(int B, int T, int H, bool has_saved);
 void set_error(const char *fmt, ...);
 void count_launch(int n = 1);
 
+// The memory-bound kernels read and write caller tensors with single 16-byte accesses, so their entry points reject a
+// pointer that is not 16-byte aligned (a contiguous view at an element offset is not) before anything is launched.
+// nullptr passes (optional arguments).  On failure the error names the entry and the first misaligned argument.
+struct NamedPtr { const char *name; const void *p; };
+inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+inline bool check_aligned16(const char *fn, std::initializer_list<NamedPtr> args) {
+    for (const NamedPtr &a : args)
+        if (!aligned16(a.p)) {
+            set_error("%s: %s is not 16-byte aligned", fn, a.name);
+            return false;
+        }
+    return true;
+}
+
 #define WKV6_CUDA_CHECK(expr)                                                            \
     do {                                                                                 \
         cudaError_t _e = (expr);                                                         \
@@ -133,8 +149,9 @@ template <int WK> __device__ __forceinline__ float load_logdecay(const void *w, 
     return fmaxf(l, lmin);
 }
 
-// ddlerp_tma.cu: TMA-fed token-shift ddlerp backward (nout = 5 with m, or 1 without).  Returns 1 when
-// the pointers are not 16-byte aligned (caller falls back to the register-fed kernel).
+// ddlerp_tma.cu: TMA-fed token-shift ddlerp backward (nout = 5 with m, or 1 / 2 without).  The caller has checked
+// C % 8 == 0 and the pointer alignment.  Returns 1 when the five m planes (5*B rows) do not fit the tensor map's int
+// dimension (caller falls back to the register-fed kernel); never for nout < 5.
 size_t ddlerp_tma_partial_slots(int nout, int B, int T, int C);
 int ddlerp_backward_tma(int nout, int B, int T, int C, const void *x, const void *shift, const void *maa, const void *m,
                         const void *const *gouts, void *gx, void *gm, void *gshift, float *partial, int *slots,
@@ -152,8 +169,7 @@ int seg_scan(int B, int nseg, int H, const float *lam, const float *s_loc, const
              cudaStream_t stream);
 int seg_flags_merge(int B, int nseg, int H, int *seg_flags, int *stream_flags, cudaStream_t stream);
 // ddlerp_lora.cu: ddlerp forward with the LoRA product on the tensor cores
-bool ddlerp_lora_supported(int B, int T, int C, int R, const void *x, const void *h, const void *w2, const void *out,
-                           const void *maa);
+bool ddlerp_lora_supported(int B, int T, int C, int R);
 int ddlerp_lora_forward(int B, int T, int C, const void *x, const void *shift, const void *maa, const void *h,
                         const void *w2, void *out, cudaStream_t stream);
 }  // namespace wkv6

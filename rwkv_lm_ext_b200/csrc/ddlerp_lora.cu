@@ -204,14 +204,10 @@ ddlerp_lora_kernel(const __grid_constant__ CUtensorMap map_h, const __grid_const
     if (warp == 8) tmem_dealloc(tmem, TM_COLS);
 }
 
-inline bool aligned16(const void *q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; }
-
 }  // namespace
 
-bool ddlerp_lora_supported(int B, int T, int C, int R, const void *x, const void *h, const void *w2, const void *out,
-                           const void *maa) {
-    return aligned16(maa) && R == RANK && C % NC == 0 && (long long)B * T > 0 && (long long)B * T < (1ll << 31) - TM && aligned16(x) &&
-           aligned16(h) && aligned16(w2) && aligned16(out);
+bool ddlerp_lora_supported(int B, int T, int C, int R) {
+    return R == RANK && C % NC == 0 && (long long)B * T > 0 && (long long)B * T < (1ll << 31) - TM;
 }
 
 int ddlerp_lora_forward(int B, int T, int C, const void *x, const void *shift, const void *maa, const void *h,
@@ -257,8 +253,10 @@ extern "C" int tmix_ddlerp_lora_bf16(int B, int T, int C, int R, const void *x, 
     if (B < 0 || T < 0 || C <= 0 || R <= 0) { set_error("tmix_ddlerp_lora_bf16: bad shape"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!x || !maa || !h || !w2 || !out) { set_error("tmix_ddlerp_lora_bf16: null pointer"); return WKV6_EINVAL; }
-    if (!ddlerp_lora_supported(B, T, C, R, x, h, w2, out, maa)) {
-        set_error("tmix_ddlerp_lora_bf16: needs R == 32, C %% 64 == 0 and 16-byte aligned tensors (use bmm + tmix_ddlerp_mix_bf16)");
+    if (!check_aligned16("tmix_ddlerp_lora_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa", maa}, {"h", h}, {"w2", w2}, {"out", out}}))
+        return WKV6_EINVAL;
+    if (!ddlerp_lora_supported(B, T, C, R)) {
+        set_error("tmix_ddlerp_lora_bf16: needs R == 32 and C %% 64 == 0 (use bmm + tmix_ddlerp_mix_bf16)");
         return WKV6_EUNSUPPORTED;
     }
     return ddlerp_lora_forward(B, T, C, x, shift_state, maa, h, w2, out, (cudaStream_t)stream);

@@ -354,6 +354,7 @@ int gather_rows_bf16(int B, int T, int D, const void *x, const int64_t *pos, voi
     if (B < 0 || T <= 0 || D <= 0) { set_error("gather_rows_bf16: bad shape"); return WKV6_EINVAL; }
     if (B == 0) return WKV6_OK;
     if (!x || !pos || !out) { set_error("gather_rows_bf16: null pointer"); return WKV6_EINVAL; }
+    if ((D & 7) == 0 && !check_aligned16("gather_rows_bf16", {{"x", x}, {"out", out}})) return WKV6_EINVAL;
     gather_rows_kernel<<<B, 256, 0, (cudaStream_t)stream>>>(T, D, (const bf16 *)x, pos, (bf16 *)out);
     count_launch();
     WKV6_CUDA_CHECK(cudaGetLastError());
@@ -365,6 +366,7 @@ int pooling_bf16(int kind, int variant, int B, int T, int D, const void *x, cons
     if (B < 0 || T <= 0 || D <= 0 || kind < 0 || kind > 2) { set_error("pooling_bf16: bad arguments"); return WKV6_EINVAL; }
     if (B == 0) return WKV6_OK;
     if (!x || !actual_len || !out_f32) { set_error("pooling_bf16: null pointer"); return WKV6_EINVAL; }
+    if ((D & 7) == 0 && !check_aligned16("pooling_bf16", {{"x", x}})) return WKV6_EINVAL;
     if (kind == 1) { set_error("pooling_bf16: lasttoken is gather_rows_bf16"); return WKV6_EINVAL; }
     dim3 grid((D + 63) / 64, B);
     pooling_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(kind, T, D, (const bf16 *)x, actual_len,
@@ -389,6 +391,7 @@ int gather_tokens_bf16(int B, int T, int D, const void *x, const int64_t *rev_id
     if (B < 0 || T < 0 || D <= 0) { set_error("gather_tokens_bf16: bad shape"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!x || !rev_idx || !out) { set_error("gather_tokens_bf16: null pointer"); return WKV6_EINVAL; }
+    if ((D & 7) == 0 && !check_aligned16("gather_tokens_bf16", {{"x", x}, {"out", out}})) return WKV6_EINVAL;
     const int BT = B * T;
     gather_tokens_kernel<<<grid_for((size_t)BT * 32, 256), 256, 0, (cudaStream_t)stream>>>(
         BT, T, D, (const bf16 *)x, rev_idx, (bf16 *)out);
@@ -401,6 +404,7 @@ int stack_reversed_bf16(int B, int T, int D, const void *x, const int64_t *rev_i
     if (B < 0 || T < 0 || D <= 0 || (D & 7)) { set_error("stack_reversed_bf16: need D %% 8 == 0"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!x || !rev_idx || !out) { set_error("stack_reversed_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("stack_reversed_bf16", {{"x", x}, {"out", out}})) return WKV6_EINVAL;
     const int BT = B * T;
     stack_reversed_kernel<<<grid_for((size_t)BT * 32, 256), 256, 0, (cudaStream_t)stream>>>(BT, T, D, (const bf16 *)x, rev_idx, (bf16 *)out);
     count_launch();
@@ -413,6 +417,8 @@ int tmix_ddlerp_mix_bf16(int B, int T, int C, const void *x, const void *shift_s
     if (B < 0 || T < 0 || C <= 0 || (C & 7)) { set_error("tmix_ddlerp_mix_bf16: need C %% 8 == 0"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!x || !maa || !m || !out) { set_error("tmix_ddlerp_mix_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("tmix_ddlerp_mix_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa", maa}, {"m", m}, {"out", out}}))
+        return WKV6_EINVAL;
     ddlerp_mix_kernel<<<grid_for((size_t)B * T * C / 8, 256), 256, 0, (cudaStream_t)stream>>>(
         B, T, C, (const bf16 *)x, (const bf16 *)shift_state, (const bf16 *)maa, (const bf16 *)m, (bf16 *)out);
     count_launch();
@@ -425,6 +431,7 @@ int tmix_shift_lerp_bf16(int B, int T, int C, const void *x, const void *shift_s
     if (B < 0 || T < 0 || C <= 0 || (C & 7)) { set_error("tmix_shift_lerp_bf16: need C %% 8 == 0"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!x || !maa_x || !out) { set_error("tmix_shift_lerp_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("tmix_shift_lerp_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa_x", maa_x}, {"out", out}})) return WKV6_EINVAL;
     shift_lerp_kernel<<<(unsigned)((size_t)B * ((T + SHIFT_ROWS - 1) / SHIFT_ROWS)), 256, 0, (cudaStream_t)stream>>>(
         B, T, C, (const bf16 *)x, (const bf16 *)shift_state, (const bf16 *)maa_x, (bf16 *)out);
     count_launch();
@@ -437,6 +444,7 @@ int groupnorm_gate_bf16(int BT, int C, int H, float eps, int gate_act, const voi
     if (BT < 0 || H <= 0 || C != H * 64) { set_error("groupnorm_gate_bf16: need C == H*64"); return WKV6_EINVAL; }
     if (BT == 0) return WKV6_OK;
     if (!y || !g || !ln_w || !ln_b || !out) { set_error("groupnorm_gate_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("groupnorm_gate_bf16", {{"y", y}, {"g", g}, {"ln_w", ln_w}, {"ln_b", ln_b}, {"out", out}})) return WKV6_EINVAL;
     const size_t ngroups = (size_t)BT * H;
     if (gate_act)
         gn_gate_kernel<true, false><<<grid_for(ngroups * 8, 256), 256, 0, (cudaStream_t)stream>>>(
@@ -455,6 +463,8 @@ int groupnorm_gate_pair_bf16(int B, int T, int C, int H, float eps, int gate_act
     if (B < 0 || T < 0 || H <= 0 || C != H * 64) { set_error("groupnorm_gate_pair_bf16: need C == H*64"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!y || !y_rev || !rev_idx || !g || !ln_w || !ln_b || !out) { set_error("groupnorm_gate_pair_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("groupnorm_gate_pair_bf16", {{"y", y}, {"y_rev", y_rev}, {"g", g}, {"ln_w", ln_w}, {"ln_b", ln_b}, {"out", out}}))
+        return WKV6_EINVAL;
     const size_t ngroups = (size_t)B * T * H;
     if (gate_act)
         gn_gate_kernel<true, true><<<grid_for(ngroups * 8, 256), 256, 0, (cudaStream_t)stream>>>(

@@ -45,7 +45,7 @@ __device__ __forceinline__ bf16x8 pack8(const float *f) {
 __device__ __forceinline__ float rb(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
 constexpr int TL = 8;  // token lanes (warps) per block
-// register-fed ddlerp gradient (the fallback of ddlerp_tma.cu for unaligned pointers): 8 channels per thread,
+// register-fed ddlerp gradient (the "simt" route of the one- and five-output forms; ddlerp_tma.cu otherwise): 8 channels per thread,
 // one 256-thread block per SM.  Measured alternatives: 4 channels per thread 1.07 ms, two blocks per SM 0.93 ms,
 // a block spanning 2048 channels 0.73 ms, against 0.59 ms for this layout (1B6 shape).
 constexpr int DD_V = 8;
@@ -361,12 +361,6 @@ __global__ void scatter_tokens_kernel(int BT, int T, int D, const bf16 *__restri
     }
 }
 
-// a += b (bf16, fp32 add): only on the unaligned-pointer fallback of the two-output shift-lerp gradient
-__global__ void add_bf16_kernel(size_t n, bf16 *__restrict__ a, const bf16 *__restrict__ b) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
-        a[i] = __float2bfloat16_rn(__bfloat162float(a[i]) + __bfloat162float(b[i]));
-}
-
 int grid_for(size_t items, int block) {
     size_t g = (items + block - 1) / block;
     const size_t cap = 148 * 16;
@@ -421,6 +415,10 @@ int tmix_ddlerp_mix_backward_bf16(int B, int T, int C, const void *x, const void
     gout.p[0] = (const bf16 *)gxw; gout.p[1] = (const bf16 *)gxk; gout.p[2] = (const bf16 *)gxv;
     gout.p[3] = (const bf16 *)gxr; gout.p[4] = (const bf16 *)gxg;
     if (ws_bytes < elementwise_backward_workspace_bytes(B, T, C, 5)) { set_error("tmix_ddlerp_mix_backward_bf16: workspace too small"); return WKV6_EINVAL; }
+    if (!check_aligned16("tmix_ddlerp_mix_backward_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa", maa}, {"m", m}, {"gxw", gxw},
+                                                            {"gxk", gxk}, {"gxv", gxv}, {"gxr", gxr}, {"gxg", gxg}, {"gx", gx}, {"gm", gm},
+                                                            {"gshift", shift_state ? gshift : nullptr}}))
+        return WKV6_EINVAL;
     if (wkv6b200_get_impl() != WKV6_IMPL_SIMT) {
         const void *gs[5] = {gxw, gxk, gxv, gxr, gxg};
         int slots = 0;
@@ -455,6 +453,9 @@ int tmix_shift_lerp_backward_bf16(int B, int T, int C, const void *x, const void
     Ptr5 g1;
     for (int i = 0; i < 5; i++) g1.p[i] = (const bf16 *)gout;
     if (ws_bytes < elementwise_backward_workspace_bytes(B, T, C, 1)) { set_error("tmix_shift_lerp_backward_bf16: workspace too small"); return WKV6_EINVAL; }
+    if (!check_aligned16("tmix_shift_lerp_backward_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa_x", maa_x}, {"gout", gout}, {"gx", gx},
+                                                            {"gshift", shift_state ? gshift : nullptr}}))
+        return WKV6_EINVAL;
     if (wkv6b200_get_impl() != WKV6_IMPL_SIMT) {
         const void *gs[1] = {gout};
         int slots = 0;
@@ -488,6 +489,8 @@ int groupnorm_gate_backward_bf16(int BT, int C, int H, float eps, int gate_act, 
         set_error("groupnorm_gate_backward_bf16: null pointer");
         return WKV6_EINVAL;
     }
+    if (!check_aligned16("groupnorm_gate_backward_bf16", {{"y", y}, {"g", g}, {"ln_w", ln_w}, {"ln_b", ln_b}, {"gout", gout}, {"gy", gy}, {"gg", gg}}))
+        return WKV6_EINVAL;
     const int S = splits_for(BT, C);
     if (ws_bytes < (size_t)S * 2 * C * sizeof(float)) {
         set_error("groupnorm_gate_backward_bf16: workspace too small");
@@ -515,6 +518,7 @@ int pooling_backward_bf16(int kind, int variant, int B, int T, int D, const int6
     if (B < 0 || T <= 0 || D <= 0 || (D & 7) || (kind != 0 && kind != 2)) { set_error("pooling_backward_bf16: bad arguments (D %% 8 == 0, kind 0 or 2)"); return WKV6_EINVAL; }
     if (B == 0) return WKV6_OK;
     if (!actual_len || !gout_f32 || !gx) { set_error("pooling_backward_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("pooling_backward_bf16", {{"gout_f32", gout_f32}, {"gx", gx}})) return WKV6_EINVAL;
     pooling_bwd_kernel<<<(unsigned)((size_t)B * ((T + POOL_ROWS - 1) / POOL_ROWS)), 256, 0, (cudaStream_t)stream>>>(
         kind, B, T, D, actual_len, (kind == 0 && variant == 1) ? 1 : 0, gout_f32, (bf16 *)gx);
     count_launch();
@@ -526,6 +530,7 @@ int scatter_rows_bf16(int B, int T, int D, const void *gout, const int64_t *pos,
     if (B < 0 || T <= 0 || D <= 0 || (D & 7)) { set_error("scatter_rows_bf16: need D %% 8 == 0"); return WKV6_EINVAL; }
     if (B == 0) return WKV6_OK;
     if (!gout || !pos || !gx) { set_error("scatter_rows_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("scatter_rows_bf16", {{"gout", gout}, {"gx", gx}})) return WKV6_EINVAL;
     scatter_rows_kernel<<<grid_for((size_t)B * T * D / 8, 256), 256, 0, (cudaStream_t)stream>>>(
         B, T, D, (const bf16 *)gout, pos, (bf16 *)gx);
     count_launch();
@@ -537,6 +542,7 @@ int scatter_tokens_bf16(int B, int T, int D, const void *gout, const int64_t *re
     if (B < 0 || T < 0 || D <= 0 || (D & 7)) { set_error("scatter_tokens_bf16: need D %% 8 == 0"); return WKV6_EINVAL; }
     if ((size_t)B * T == 0) return WKV6_OK;
     if (!gout || !rev_idx || !gx) { set_error("scatter_tokens_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("scatter_tokens_bf16", {{"gout", gout}, {"gx", gx}})) return WKV6_EINVAL;
     const int BT = B * T;
     scatter_tokens_kernel<<<grid_for((size_t)BT * 32, 256), 256, 0, (cudaStream_t)stream>>>(
         BT, T, D, (const bf16 *)gout, rev_idx, (bf16 *)gx);
@@ -554,34 +560,14 @@ int cmix_shift_lerp2_backward_bf16(int B, int T, int C, const void *x, const voi
     if (BT == 0) return WKV6_OK;
     if (!x || !maa_kr || !gxk || !gxr || !gx || !ws) { set_error("cmix_shift_lerp2_backward_bf16: null pointer"); return WKV6_EINVAL; }
     if (ws_bytes < elementwise_backward_workspace_bytes(B, T, C, 3)) { set_error("cmix_shift_lerp2_backward_bf16: workspace too small"); return WKV6_EINVAL; }
+    if (!check_aligned16("cmix_shift_lerp2_backward_bf16", {{"x", x}, {"shift_state", shift_state}, {"gxk", gxk}, {"gxr", gxr}, {"gx", gx},
+                                                             {"gshift", shift_state ? gshift : nullptr}}))
+        return WKV6_EINVAL;
     const void *gs[2] = {gxk, gxr};
     int slots = 0;
-    int rc = ddlerp_backward_tma(2, B, T, C, x, shift_state, maa_kr, nullptr, gs, gx, nullptr, shift_state ? gshift : nullptr,
-                                 (float *)ws, &slots, (cudaStream_t)stream);
-    if (rc < 0) return rc;
-    if (rc == 1) {          // unaligned pointers: two passes of the register-fed one-output kernel
-        const int S = splits_for(BT, C, DD_COLS, DD_LANES);
-        dim3 grid((C + DD_COLS - 1) / DD_COLS, S);
-        float *part = (float *)ws;
-        bf16 *tmp = nullptr;
-        WKV6_CUDA_CHECK(cudaMallocAsync((void **)&tmp, (size_t)BT * C * 2 + (shift_state ? (size_t)B * C * 2 : 0), (cudaStream_t)stream));
-        bf16 *tmp_shift = shift_state ? tmp + (size_t)BT * C : nullptr;
-        for (int n = 0; n < 2; n++) {
-            Ptr5 g1;
-            for (int i = 0; i < 5; i++) g1.p[i] = (const bf16 *)gs[n];
-            ddlerp_bwd_kernel<1, false, DD_V><<<grid, 256, 0, (cudaStream_t)stream>>>(
-                B, T, C, split_of(BT, S, DD_LANES), (const bf16 *)x, (const bf16 *)shift_state, (const bf16 *)maa_kr + (size_t)n * C,
-                nullptr, g1, n == 0 ? (bf16 *)gx : tmp, nullptr, shift_state ? (n == 0 ? (bf16 *)gshift : tmp_shift) : nullptr, part);
-            if (gmaa_kr) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, C, (size_t)C, part, gmaa_kr + (size_t)n * C);
-            count_launch(gmaa_kr ? 2 : 1);
-        }
-        add_bf16_kernel<<<1184, 256, 0, (cudaStream_t)stream>>>((size_t)BT * C, (bf16 *)gx, tmp);
-        if (shift_state) add_bf16_kernel<<<64, 256, 0, (cudaStream_t)stream>>>((size_t)B * C, (bf16 *)gshift, tmp_shift);
-        count_launch(shift_state ? 2 : 1);
-        WKV6_CUDA_CHECK(cudaGetLastError());
-        cudaFreeAsync(tmp, (cudaStream_t)stream);
-        return WKV6_OK;
-    }
+    const int rc = ddlerp_backward_tma(2, B, T, C, x, shift_state, maa_kr, nullptr, gs, gx, nullptr, shift_state ? gshift : nullptr,
+                                       (float *)ws, &slots, (cudaStream_t)stream);
+    if (rc != WKV6_OK) return rc;      // (the TMA kernel declines only the five-output form)
     if (gmaa_kr) sum_partials_kernel<<<(2 * C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(slots, 2 * C, (size_t)2 * C, (const float *)ws, gmaa_kr);
     if (gmaa_kr) count_launch();
     WKV6_CUDA_CHECK(cudaGetLastError());

@@ -13,12 +13,22 @@ def _cuda(t):
     _lib.require_current_device(t)
 
 
+def _dense(t):
+    """t as a contiguous tensor whose data starts 16-byte aligned.  The kernels use 16-byte vector accesses and the
+    library rejects a misaligned pointer, so a contiguous view at an element offset (`buf[1:].view(...)`) is copied
+    into fresh storage first."""
+    if t is None:
+        return None
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 def _bf16_param(t):
     """Parameters reach the kernels as bf16.  A model kept in fp32 ('bf16-mixed', ln_x in fp32, ...) is cast here --
     differentiably, so the gradient returns in the parameter's own dtype -- instead of being reinterpreted."""
     if t is None:
         return None
-    return (t if t.dtype == torch.bfloat16 else t.to(torch.bfloat16)).contiguous()
+    return _dense(t if t.dtype == torch.bfloat16 else t.to(torch.bfloat16))
 
 
 def eos_index(idx: torch.Tensor, token_id: int) -> torch.Tensor:
@@ -58,7 +68,7 @@ class _GatherRows(torch.autograd.Function):
     def backward(ctx, gout):
         (pos,) = ctx.saved_tensors
         B, T, D = ctx.shape
-        gout = gout.contiguous()
+        gout = _dense(gout)
         gx = torch.empty(B, T, D, dtype=torch.bfloat16, device=gout.device)
         check(_lib.load().scatter_rows_bf16(B, T, D, ptr(gout), ptr(pos), ptr(gx), stream_of(gout)), "scatter_rows_bf16")
         return gx, None
@@ -69,7 +79,7 @@ def gather_rows(x: torch.Tensor, pos: torch.Tensor) -> torch.Tensor:
     _cuda(x)
     assert x.dtype == torch.bfloat16 and x.dim() == 3 and pos.dtype == torch.int64
     assert pos.numel() == x.shape[0], "one position per batch row"
-    x, pos = x.contiguous(), pos.contiguous()
+    x, pos = _dense(x), pos.contiguous()
     if _needs_grad(x):
         assert x.shape[-1] % 8 == 0, "gather_rows under autograd needs D % 8 == 0 (scatter_rows_bf16)"
         return _GatherRows.apply(x, pos)
@@ -103,7 +113,7 @@ class _Pooling(torch.autograd.Function):
     def backward(ctx, gout):
         (alen,) = ctx.saved_tensors
         (B, T, D), kind, variant = ctx.meta
-        gout = gout.float().contiguous()
+        gout = _dense(gout.float())
         gx = torch.empty(B, T, D, dtype=torch.bfloat16, device=gout.device)
         check(_lib.load().pooling_backward_bf16(kind, variant, B, T, D, ptr(alen), ptr(gout), ptr(gx), stream_of(gout)),
               "pooling_backward_bf16")
@@ -120,7 +130,7 @@ def pooling(x: torch.Tensor, actual_len: torch.Tensor, pooling_type: str, varian
         return gather_rows(x, actual_len.to(torch.int64))
     if pooling_type not in _KIND or (variant == "infer" and pooling_type == "avg"):
         raise ValueError(pooling_type)
-    x = x.contiguous()
+    x = _dense(x)
     alen = actual_len.to(torch.int64).contiguous()
     kind, var = _KIND[pooling_type], 1 if variant == "infer" else 0
     out = _Pooling.apply(x, alen, kind, var) if _needs_grad(x) else _pooling_fwd(x, alen, kind, var)
@@ -157,7 +167,7 @@ class _ReverseX(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gout):
         (rev_idx,) = ctx.saved_tensors
-        gout = gout.contiguous()
+        gout = _dense(gout)
         B, T, D = gout.shape
         gx = torch.empty_like(gout)
         check(_lib.load().scatter_tokens_bf16(B, T, D, ptr(gout), ptr(rev_idx), ptr(gx), stream_of(gout)), "scatter_tokens_bf16")
@@ -171,7 +181,7 @@ def stack_reversed(x: torch.Tensor, rev_idx: torch.Tensor) -> torch.Tensor:
     if _needs_grad(x) or x.shape[-1] % 8 != 0:
         return torch.cat([x, reverse_x(x, rev_idx)], 0)
     assert x.dtype == torch.bfloat16 and x.dim() == 3 and rev_idx.dtype == torch.int64 and rev_idx.shape == x.shape[:2]
-    x, rev_idx = x.contiguous(), rev_idx.contiguous()
+    x, rev_idx = _dense(x), rev_idx.contiguous()
     B, T, D = x.shape
     out = torch.empty((2 * B, T, D), device=x.device, dtype=x.dtype)
     check(_lib.load().stack_reversed_bf16(B, T, D, ptr(x), ptr(rev_idx), ptr(out), stream_of(x)), "stack_reversed_bf16")
@@ -183,7 +193,7 @@ def reverse_x(x: torch.Tensor, rev_idx: torch.Tensor) -> torch.Tensor:
     Differentiable w.r.t. x when rev_idx is a per-row permutation (what reverse_x_idx builds)."""
     _cuda(x)
     assert x.dtype == torch.bfloat16 and x.dim() == 3 and rev_idx.dtype == torch.int64
-    x, rev_idx = x.contiguous(), rev_idx.contiguous()
+    x, rev_idx = _dense(x), rev_idx.contiguous()
     if _needs_grad(x):
         return _ReverseX.apply(x, rev_idx)
     return _reverse_fwd(x, rev_idx)
@@ -208,7 +218,7 @@ class _ShiftLerp(torch.autograd.Function):
         x, shift_state, maa_x = ctx.saved_tensors
         lib = _lib.load()
         B, T, C = x.shape
-        gout = gout.contiguous()
+        gout = _dense(gout)
         gx = torch.empty_like(x)
         gmaa = torch.empty(C, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[2] else None   # frozen: no reduction
         gshift = torch.empty_like(shift_state) if shift_state is not None else None
@@ -223,8 +233,7 @@ def tmix_shift_lerp(x, maa_x, shift_state=None):
     x, time_maa_x and the shift state."""
     _cuda(x)
     assert x.dtype == torch.bfloat16
-    x = x.contiguous()
-    shift_state = shift_state.contiguous() if shift_state is not None else None
+    x = _dense(x)
     flat = _bf16_param(maa_x).view(-1)
     assert flat.numel() == x.shape[-1]
     shift_state = _bf16_param(shift_state)
@@ -255,7 +264,7 @@ class _DdlerpMix(torch.autograd.Function):
         x, shift_state, maa, m = ctx.saved_tensors
         lib = _lib.load()
         B, T, C = x.shape
-        gouts = [torch.zeros_like(x) if g is None else g.contiguous() for g in gouts]
+        gouts = [torch.zeros_like(x) if g is None else _dense(g) for g in gouts]
         gx, gm = torch.empty_like(x), torch.empty_like(m)
         gmaa = torch.empty(5, C, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[2] else None
         gshift = torch.empty_like(shift_state) if shift_state is not None else None
@@ -273,7 +282,7 @@ def tmix_ddlerp_mix(x, maa_wkvrg, m, shift_state=None):
     it either way.  Differentiable w.r.t. x, maa_wkvrg, m and the shift state."""
     _cuda(x)
     assert x.dtype == torch.bfloat16 and m.dtype == torch.bfloat16
-    x, m, maa = x.contiguous(), m.contiguous(), _bf16_param(maa_wkvrg)
+    x, m, maa = _dense(x), _dense(m), _bf16_param(maa_wkvrg)
     assert tuple(maa.shape) == (5, x.shape[-1]) and tuple(m.shape) == (5,) + tuple(x.shape)
     shift_state = _bf16_param(shift_state)
     if _needs_grad(x, maa, m, shift_state):
@@ -298,7 +307,7 @@ class _DdlerpLora(torch.autograd.Function):
         R = w2.shape[1]
         h5 = h.view(B * T, 5, R).transpose(0, 1)                     # [5, BT, R]
         m = torch.bmm(h5, w2).view(5, B, T, C)
-        gouts = [torch.zeros_like(x) if g is None else g.contiguous() for g in gouts]
+        gouts = [torch.zeros_like(x) if g is None else _dense(g) for g in gouts]
         gx, gm = torch.empty_like(x), torch.empty_like(m)
         gmaa = torch.empty(5, C, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[2] else None
         gshift = torch.empty_like(shift_state) if shift_state is not None else None
@@ -330,9 +339,9 @@ def tmix_ddlerp_lora(x, maa_wkvrg, h, w2, shift_state=None):
     assert x.dtype == torch.bfloat16 and h.dtype == torch.bfloat16
     B, T, C = x.shape
     R = w2.shape[1]
-    x, maa, w2 = x.contiguous(), _bf16_param(maa_wkvrg), _bf16_param(w2)
+    x, maa, w2 = _dense(x), _bf16_param(maa_wkvrg), _bf16_param(w2)
     assert tuple(maa.shape) == (5, C) and tuple(w2.shape) == (5, R, C)
-    h = h.contiguous().view(B * T, 5 * R)
+    h = _dense(h).view(B * T, 5 * R)
     shift_state = _bf16_param(shift_state)
     if R != 32 or C % 64 != 0:
         m = torch.bmm(h.view(B * T, 5, R).transpose(0, 1), w2).view(5, B, T, C)
@@ -366,7 +375,7 @@ class _GroupNormGate(torch.autograd.Function):
         H, eps, act = ctx.meta
         lib = _lib.load()
         B, T, C = y.shape
-        gout = gout.contiguous()
+        gout = _dense(gout)
         gy, gg = torch.empty_like(y), torch.empty_like(g)
         need_p = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]                       # frozen affine: no reduction
         gw = torch.empty(C, dtype=torch.float32, device=y.device) if need_p else None
@@ -384,7 +393,7 @@ def groupnorm_gate(y, g, ln_w, ln_b, H, eps, gate_act=None):
     inside the kernel.  Differentiable w.r.t. y, g and the GroupNorm affine parameters."""
     _cuda(y)
     assert y.dtype == torch.bfloat16 and g.dtype == torch.bfloat16
-    y, g, ln_w, ln_b = y.contiguous(), g.contiguous(), _bf16_param(ln_w), _bf16_param(ln_b)
+    y, g, ln_w, ln_b = _dense(y), _dense(g), _bf16_param(ln_w), _bf16_param(ln_b)
     assert ln_w.numel() == y.shape[-1] and ln_b.numel() == y.shape[-1] and y.shape[-1] == H * 64
     act = _GATE_ACT[gate_act]
     if _needs_grad(y, g, ln_w, ln_b):
@@ -400,7 +409,7 @@ def groupnorm_gate_pair(y, y_rev, rev_idx, g, ln_w, ln_b, H, eps, gate_act=None)
     if _needs_grad(y, y_rev, g, ln_w, ln_b):
         return groupnorm_gate((y + reverse_x(y_rev, rev_idx)) / 2, g, ln_w, ln_b, H, eps, gate_act)
     assert y.dtype == torch.bfloat16 and y_rev.dtype == torch.bfloat16 and g.dtype == torch.bfloat16 and rev_idx.dtype == torch.int64
-    y, y_rev, g, rev_idx = y.contiguous(), y_rev.contiguous(), g.contiguous(), rev_idx.contiguous()
+    y, y_rev, g, rev_idx = _dense(y), _dense(y_rev), _dense(g), rev_idx.contiguous()
     B, T, C = y.shape
     out = torch.empty_like(y)
     check(_lib.load().groupnorm_gate_pair_bf16(B, T, C, H, float(eps), _GATE_ACT[gate_act], ptr(y), ptr(y_rev), ptr(rev_idx), ptr(g),
