@@ -46,7 +46,7 @@ extern "C" {
 #define WKV6_FP16 1
 #define WKV6_FP32 2
 
-/* implementation selector, see wkv6b200_set_impl */
+/* route of the WKV6 recurrence, see wkv6b200_set_impl; it selects nothing else (every other kernel has one route) */
 #define WKV6_IMPL_AUTO 0       /* tensor-core chunked kernels where the shape allows, else SIMT */
 #define WKV6_IMPL_SIMT 1       /* exact fp32 step recurrence on CUDA cores (all shapes)          */
 #define WKV6_IMPL_TC   2       /* tcgen05/TMA chunked kernels only; WKV6_EUNSUPPORTED otherwise  */
@@ -266,7 +266,8 @@ WKV6_API int groupnorm_gate_pair_bf16(int B, int T, int C, int H, float eps, int
  * ------------------------------------------------------------------------------------------ */
 WKV6_API size_t elementwise_backward_workspace_bytes(int B, int T, int C, int nparam);
 /* gx [B,T,C], gm [5,B,T,C], gmaa fp32 [5,C] from the gradients of xw,xk,xv,xr,xg (five separate
- * [B,T,C] tensors: they come out of five different Linear backward passes). */
+ * [B,T,C] tensors: they come out of five different Linear backward passes).  B > INT_MAX / 5 is
+ * rejected with WKV6_EINVAL: the kernel reads the m planes through one tensor map of 5*B rows. */
 WKV6_API int tmix_ddlerp_mix_backward_bf16(int B, int T, int C, const void *x, const void *shift_state,
                                   const void *maa, const void *m, const void *gxw, const void *gxk,
                                   const void *gxv, const void *gxr, const void *gxg, void *gx, void *gm,

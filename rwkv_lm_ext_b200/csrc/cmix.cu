@@ -6,6 +6,7 @@
 // All HBM-bound; 128-bit accesses; arithmetic in packed bf16 with the non-contracting intrinsics, i.e. with
 // exactly the op-by-op rounding of the eager bf16 chain (results are bit-identical to it).  The gradient of
 // the two-output shift-lerp is the TMA-fed kernel of ddlerp_tma.cu (nout = 2).
+#include "bf16x8.cuh"
 #include "common.cuh"
 
 namespace wkv6 {
@@ -13,29 +14,6 @@ namespace {
 
 typedef __nv_bfloat16 bf16;
 typedef __nv_bfloat162 bf162;
-struct alignas(16) bf16x8 { bf162 v[4]; };
-// ONE 128-bit access each way (copying the struct itself is compiled to four 32-bit accesses: __nv_bfloat162 has its own
-// copy operations)
-__device__ __forceinline__ bf16x8 ld8(const bf16 *p) {
-    const uint4 u = *reinterpret_cast<const uint4 *>(p);
-    bf16x8 r;
-    r.v[0] = *reinterpret_cast<const __nv_bfloat162 *>(&u.x);
-    r.v[1] = *reinterpret_cast<const __nv_bfloat162 *>(&u.y);
-    r.v[2] = *reinterpret_cast<const __nv_bfloat162 *>(&u.z);
-    r.v[3] = *reinterpret_cast<const __nv_bfloat162 *>(&u.w);
-    return r;
-}
-__device__ __forceinline__ void st8(bf16 *p, const bf16x8 &x) {
-    *reinterpret_cast<uint4 *>(p) = make_uint4(*reinterpret_cast<const uint32_t *>(&x.v[0]), *reinterpret_cast<const uint32_t *>(&x.v[1]),
-                                                *reinterpret_cast<const uint32_t *>(&x.v[2]), *reinterpret_cast<const uint32_t *>(&x.v[3]));
-}
-
-int grid_for(size_t items, int block) {
-    size_t g = (items + block - 1) / block;
-    const size_t cap = 148 * 16;
-    return (int)(g < 1 ? 1 : (g > cap ? cap : g));
-}
-
 // out_n = x + bf16(bf16(prev - x) * maa_n),  n = 0..NOUT-1
 template <int NOUT>
 __global__ void __launch_bounds__(256) shift_lerp_n_kernel(int B, int T, int C, const bf16 *__restrict__ x,

@@ -150,8 +150,8 @@ template <int WK> __device__ __forceinline__ float load_logdecay(const void *w, 
 }
 
 // ddlerp_tma.cu: TMA-fed token-shift ddlerp backward (nout = 5 with m, or 1 / 2 without).  The caller has checked
-// C % 8 == 0 and the pointer alignment.  Returns 1 when the five m planes (5*B rows) do not fit the tensor map's int
-// dimension (caller falls back to the register-fed kernel); never for nout < 5.
+// C % 8 == 0, the pointer alignment and, with m, 5*B <= INT_MAX (the five m planes are one tensor map of 5*B rows).
+// Returns WKV6_OK or an error.
 size_t ddlerp_tma_partial_slots(int nout, int B, int T, int C);
 int ddlerp_backward_tma(int nout, int B, int T, int C, const void *x, const void *shift, const void *maa, const void *m,
                         const void *const *gouts, void *gx, void *gm, void *gshift, float *partial, int *slots,

@@ -2,8 +2,8 @@
 //
 // The gradient of  out_n = x + xx * coef_n  reads 11 tensors of [B,T,C] (x, five incoming gradients,
 // five LoRA coefficients m_n) and writes 6 (gx, five gm_n): 34 B per element, nothing but HBM
-// traffic.  A register-fed kernel (elementwise_bwd.cu) keeps only ~45 KB per SM in flight and stalls
-// on every cold miss; here one elected thread streams [8 tokens x 256 channels] boxes of all 11
+// traffic.  A register-fed kernel keeps only ~45 KB per SM in flight and stalls on every cold miss
+// (DESIGN.md §4.4); here one elected thread streams [8 tokens x 256 channels] boxes of all 11
 // inputs into a 3-stage shared-memory ring with cp.async.bulk.tensor (~90 KB in flight per SM while
 // a tile is being consumed) and the 8 warps read the tile with conflict-free 16-byte loads.
 //
@@ -15,6 +15,7 @@
 // gxx[T] = 0 and the zero padding of nn.ZeroPad2d((0,0,1,-1)) (src/model.py:428).
 // Parameter gradients: per-thread accumulators, reduced over the 8 rows in shared memory, written as
 // fp32 partials [B*splits][n][C]; sum_partials (elementwise_bwd.cu) adds them in a fixed order.
+#include "bf16x8.cuh"
 #include "common.cuh"
 #include "tc_common.cuh"
 
@@ -25,33 +26,6 @@ using namespace tc;
 typedef __nv_bfloat16 bf16;
 
 constexpr int ROWS = 8, COLS = 256, NS = 3;
-
-struct alignas(16) bf16x8 { __nv_bfloat162 v[4]; };
-// ONE 128-bit access each way, global or shared (copying the struct itself is compiled to four 32-bit accesses)
-__device__ __forceinline__ bf16x8 ld8(const void *p) {
-    const uint4 u = *reinterpret_cast<const uint4 *>(p);
-    bf16x8 r;
-    r.v[0] = *reinterpret_cast<const __nv_bfloat162 *>(&u.x);
-    r.v[1] = *reinterpret_cast<const __nv_bfloat162 *>(&u.y);
-    r.v[2] = *reinterpret_cast<const __nv_bfloat162 *>(&u.z);
-    r.v[3] = *reinterpret_cast<const __nv_bfloat162 *>(&u.w);
-    return r;
-}
-__device__ __forceinline__ void st8(void *p, const bf16x8 &x) {
-    *reinterpret_cast<uint4 *>(p) = make_uint4(*reinterpret_cast<const uint32_t *>(&x.v[0]), *reinterpret_cast<const uint32_t *>(&x.v[1]),
-                                                *reinterpret_cast<const uint32_t *>(&x.v[2]), *reinterpret_cast<const uint32_t *>(&x.v[3]));
-}
-__device__ __forceinline__ void unpack8(const bf16x8 &x, float *f) {
-#pragma unroll
-    for (int i = 0; i < 4; i++) { float2 t = __bfloat1622float2(x.v[i]); f[2 * i] = t.x; f[2 * i + 1] = t.y; }
-}
-__device__ __forceinline__ bf16x8 pack8(const float *f) {
-    bf16x8 x;
-#pragma unroll
-    for (int i = 0; i < 4; i++) x.v[i] = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-    return x;
-}
-__device__ __forceinline__ float rb(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
 struct Maps5 { CUtensorMap m[5]; };
 struct Ptr5 { const bf16 *p[5]; };
@@ -235,11 +209,9 @@ size_t ddlerp_tma_partial_slots(int nout, int B, int T, int C) {
     return (size_t)B * splits;
 }
 
-// returns WKV6_OK, an error, or 1 = "not applicable, use the register-fed kernel" (common.cuh)
 int ddlerp_backward_tma(int nout, int B, int T, int C, const void *x, const void *shift, const void *maa, const void *m,
                         const void *const *gouts, void *gx, void *gm, void *gshift, float *partial, int *slots,
                         cudaStream_t stream) {
-    if (m && (size_t)5 * B > 0x7fffffffu) return 1;
     int splits, rps;
     geometry(nout, B, T, C, &splits, &rps);
     *slots = B * splits;

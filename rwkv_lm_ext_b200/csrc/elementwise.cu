@@ -1,41 +1,13 @@
 // Memory-bound neighbours of the WKV6 recurrence: eos gather, pooling, mask / reverse index,
 // token-shift ddlerp mixing, GroupNorm*gate.  All HBM-bound: 128-bit accesses, one pass over the
 // big tensor each, grids sized to oversubscribe the 148 SMs.
+#include "bf16x8.cuh"
 #include "common.cuh"
 
 namespace wkv6 {
 namespace {
 
 typedef __nv_bfloat16 bf16;
-
-struct alignas(16) bf16x8 { __nv_bfloat162 v[4]; };
-// ONE 128-bit access each way (copying the struct itself is compiled to four 32-bit accesses: __nv_bfloat162 has its own
-// copy operations)
-__device__ __forceinline__ bf16x8 ld8(const bf16 *p) {
-    const uint4 u = *reinterpret_cast<const uint4 *>(p);
-    bf16x8 r;
-    r.v[0] = *reinterpret_cast<const __nv_bfloat162 *>(&u.x);
-    r.v[1] = *reinterpret_cast<const __nv_bfloat162 *>(&u.y);
-    r.v[2] = *reinterpret_cast<const __nv_bfloat162 *>(&u.z);
-    r.v[3] = *reinterpret_cast<const __nv_bfloat162 *>(&u.w);
-    return r;
-}
-__device__ __forceinline__ void st8(bf16 *p, const bf16x8 &x) {
-    *reinterpret_cast<uint4 *>(p) = make_uint4(*reinterpret_cast<const uint32_t *>(&x.v[0]), *reinterpret_cast<const uint32_t *>(&x.v[1]),
-                                                *reinterpret_cast<const uint32_t *>(&x.v[2]), *reinterpret_cast<const uint32_t *>(&x.v[3]));
-}
-__device__ __forceinline__ void unpack8(const bf16x8 &x, float *f) {
-#pragma unroll
-    for (int i = 0; i < 4; i++) { float2 t = __bfloat1622float2(x.v[i]); f[2 * i] = t.x; f[2 * i + 1] = t.y; }
-}
-__device__ __forceinline__ bf16x8 pack8(const float *f) {
-    bf16x8 x;
-#pragma unroll
-    for (int i = 0; i < 4; i++) x.v[i] = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-    return x;
-}
-// round-trip through bf16: what a bf16 eager op in the reference does to its fp32 result
-__device__ __forceinline__ float rb(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
 // ------------------------------------------------------------------------------------------------
 // eos index: first t with idx[b,t] == id, 0 if absent.  One block per row.
@@ -313,12 +285,6 @@ __global__ void __launch_bounds__(256) ew_to_raw_kernel(size_t n8, int T, int H,
             flags[(bt / T) * H + c / 64] = 1;
         }
     }
-}
-
-int grid_for(size_t items, int block) {
-    size_t g = (items + block - 1) / block;
-    const size_t cap = 148 * 16;
-    return (int)(g < 1 ? 1 : (g > cap ? cap : g));
 }
 
 }  // namespace

@@ -1,187 +1,27 @@
 // Gradients of the memory-bound neighbours (token-shift ddlerp, GroupNorm*gate, pooling, the two
 // gathers), so the fused forwards of elementwise.cu can sit inside a training graph in place of the
-// reference's eager chains (src/model.py:434-468, src/model_ext.py:1708-1738).
+// reference's eager chains (src/model.py:434-468, src/model_ext.py:1708-1738).  The token-shift
+// gradients are the TMA-fed kernel of ddlerp_tma.cu; this file sums its partials.
 //
-// Layout of the two "column reduce" kernels: grid (ceil(C/256), S), block 256 = 32 column lanes
-// (8 channels each, so a warp reads 512 contiguous bytes of a token row) x 8 token lanes (one warp
-// each).  A block owns rows [split*R, split*R+R) of the flattened [B*T, C] tensor, a warp a contiguous
-// run of them walked backwards (the token-shift gradient needs the value of row t+1 when it is at
-// row t).  Parameter gradients (sums over all rows) are accumulated per thread, reduced over the 8
-// token lanes in shared memory and written as fp32 partials [S][n][C]; a second, tiny kernel sums
-// the S partials in a fixed order -> deterministic, no atomics.
+// Layout of the GroupNorm*gate "column reduce" kernel: grid (ceil(C/256), S), block 256 = 32 column
+// lanes (8 channels each, so a warp reads 512 contiguous bytes of a token row) x 8 token lanes (one
+// warp each).  A block owns rows [split*R, split*R+R) of the flattened [B*T, C] tensor, a warp a
+// contiguous run of them.  The parameter gradients (sums over all rows) are accumulated per thread,
+// reduced over the 8 token lanes in shared memory and written as fp32 partials [S][2][C]; a second,
+// tiny kernel sums the S partials in a fixed order -> deterministic, no atomics.
+#include "bf16x8.cuh"
 #include "common.cuh"
-#include <algorithm>
+
+#include <climits>
 
 namespace wkv6 {
 namespace {
 
 typedef __nv_bfloat16 bf16;
-struct alignas(16) bf16x8 { __nv_bfloat162 v[4]; };
-// ONE 128-bit access each way (copying the struct itself is compiled to four 32-bit accesses: __nv_bfloat162 has its own
-// copy operations)
-__device__ __forceinline__ bf16x8 ld8(const bf16 *p) {
-    const uint4 u = *reinterpret_cast<const uint4 *>(p);
-    bf16x8 r;
-    r.v[0] = *reinterpret_cast<const __nv_bfloat162 *>(&u.x);
-    r.v[1] = *reinterpret_cast<const __nv_bfloat162 *>(&u.y);
-    r.v[2] = *reinterpret_cast<const __nv_bfloat162 *>(&u.z);
-    r.v[3] = *reinterpret_cast<const __nv_bfloat162 *>(&u.w);
-    return r;
-}
-__device__ __forceinline__ void st8(bf16 *p, const bf16x8 &x) {
-    *reinterpret_cast<uint4 *>(p) = make_uint4(*reinterpret_cast<const uint32_t *>(&x.v[0]), *reinterpret_cast<const uint32_t *>(&x.v[1]),
-                                                *reinterpret_cast<const uint32_t *>(&x.v[2]), *reinterpret_cast<const uint32_t *>(&x.v[3]));
-}
-__device__ __forceinline__ void unpack8(const bf16x8 &x, float *f) {
-#pragma unroll
-    for (int i = 0; i < 4; i++) { float2 t = __bfloat1622float2(x.v[i]); f[2 * i] = t.x; f[2 * i + 1] = t.y; }
-}
-__device__ __forceinline__ bf16x8 pack8(const float *f) {
-    bf16x8 x;
-#pragma unroll
-    for (int i = 0; i < 4; i++) x.v[i] = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-    return x;
-}
-__device__ __forceinline__ float rb(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
 constexpr int TL = 8;  // token lanes (warps) per block
-// register-fed ddlerp gradient (the "simt" route of the one- and five-output forms; ddlerp_tma.cu otherwise): 8 channels per thread,
-// one 256-thread block per SM.  Measured alternatives: 4 channels per thread 1.07 ms, two blocks per SM 0.93 ms,
-// a block spanning 2048 channels 0.73 ms, against 0.59 ms for this layout (1B6 shape).
-constexpr int DD_V = 8;
 
 struct Split { int rows_per_split, rows_per_lane; };
-struct Ptr5 { const bf16 *p[5]; };   // the five incoming gradients (xw,xk,xv,xr,xg) are separate tensors
-
-// ------------------------------------------------------------------------------------------------
-// out_n = x + xx * coef_n,  xx = bf16(prev - x),  coef_n = bf16(maa_n + m_n)   (HAS_M)  or  maa_n
-//   gm_n   = gout_n * xx                                   (HAS_M only)
-//   gmaa_n = sum_rows gout_n * xx
-//   gxx    = sum_n gout_n * coef_n
-//   gx[t]  = sum_n gout_n[t] - gxx[t] + gxx[t+1]           (gxx[T] = 0)
-//   gshift[b] = gxx[b, 0]                                  (when a shift state was given)
-// ------------------------------------------------------------------------------------------------
-// V channels per thread
-template <int V> struct VecIO;
-template <> struct VecIO<8> {
-    static __device__ __forceinline__ void ld(const bf16 *p, float *f) { unpack8(ld8(p), f); }
-    static __device__ __forceinline__ void st(bf16 *p, const float *f) { st8(p, pack8(f)); }
-};
-
-template <int NOUT, bool HAS_M, int V>
-__global__ void __launch_bounds__(256) ddlerp_bwd_kernel(int B, int T, int C, Split sp, const bf16 *__restrict__ x,
-                                                         const bf16 *__restrict__ shift, const bf16 *__restrict__ maa,
-                                                         const bf16 *__restrict__ m, const Ptr5 gout,
-                                                         bf16 *__restrict__ gx, bf16 *__restrict__ gm,
-                                                         bf16 *__restrict__ gshift, float *__restrict__ partial) {
-    typedef VecIO<V> IO;
-    constexpr int COLS = 32 * V;                       // channels per block
-    const int lane = threadIdx.x & 31, tl = threadIdx.x >> 5;
-    const int c = (blockIdx.x * 32 + lane) * V;
-    const bool live = c < C;
-    const long long BT = (long long)B * T;
-    const size_t plane = (size_t)BT * C;
-    const long long s0 = (long long)blockIdx.y * sp.rows_per_split;
-    long long r0 = s0 + (long long)tl * sp.rows_per_lane;
-    long long r1 = r0 + sp.rows_per_lane;
-    const long long send = s0 + sp.rows_per_split < BT ? s0 + sp.rows_per_split : BT;
-    if (r1 > send) r1 = send;
-
-    float acc[NOUT][V];
-#pragma unroll
-    for (int n = 0; n < NOUT; n++)
-#pragma unroll
-        for (int e = 0; e < V; e++) acc[n][e] = 0.f;
-
-    if (live && r0 < r1) {
-        float af[NOUT][V];
-#pragma unroll
-        for (int n = 0; n < NOUT; n++) IO::ld(maa + (size_t)n * C + c, af[n]);
-
-        // gxx of one row (needed for the row after this run, if it belongs to the same sequence)
-        auto row_gxx = [&](long long row, const float *xx, float *gxx, float *gsum, bool write) {
-#pragma unroll
-            for (int e = 0; e < V; e++) { gxx[e] = 0.f; gsum[e] = 0.f; }
-#pragma unroll
-            for (int n = 0; n < NOUT; n++) {
-                float gf[V], cf[V];
-                IO::ld(gout.p[n] + (size_t)row * C + c, gf);
-                if (HAS_M) {
-                    IO::ld(m + n * plane + (size_t)row * C + c, cf);
-#pragma unroll
-                    for (int e = 0; e < V; e++) cf[e] = rb(af[n][e] + cf[e]);
-                } else {
-#pragma unroll
-                    for (int e = 0; e < V; e++) cf[e] = af[n][e];
-                }
-                float gmv[V];
-#pragma unroll
-                for (int e = 0; e < V; e++) {
-                    gxx[e] = fmaf(gf[e], cf[e], gxx[e]);
-                    gsum[e] += gf[e];
-                    gmv[e] = gf[e] * xx[e];
-                    if (write) acc[n][e] += gmv[e];
-                }
-                if (HAS_M && write) IO::st(gm + n * plane + (size_t)row * C + c, gmv);
-            }
-        };
-
-        float carry[V], xf[V], pf[V], xx[V], gxx[V], gsum[V];
-        // carry = gxx[r1] when row r1 continues the sequence of row r1-1
-        if (r1 < BT && (r1 % T) != 0) {
-#pragma unroll
-            for (int e = 0; e < V; e++) xf[e] = 0.f;
-            row_gxx(r1, xf, carry, gsum, false);
-        } else {
-#pragma unroll
-            for (int e = 0; e < V; e++) carry[e] = 0.f;
-        }
-        IO::ld(x + (size_t)(r1 - 1) * C + c, xf);
-        for (long long row = r1 - 1; row >= r0; row--) {
-            const int t = (int)(row % T);
-            if (t > 0) IO::ld(x + (size_t)(row - 1) * C + c, pf);
-            else if (shift) IO::ld(shift + (size_t)(row / T) * C + c, pf);
-            else {
-#pragma unroll
-                for (int e = 0; e < V; e++) pf[e] = 0.f;
-            }
-#pragma unroll
-            for (int e = 0; e < V; e++) xx[e] = rb(pf[e] - xf[e]);
-            row_gxx(row, xx, gxx, gsum, true);
-            float o[V];
-#pragma unroll
-            for (int e = 0; e < V; e++) o[e] = gsum[e] - gxx[e] + carry[e];
-            IO::st(gx + (size_t)row * C + c, o);
-            if (t == 0) {
-                if (gshift) IO::st(gshift + (size_t)(row / T) * C + c, gxx);
-#pragma unroll
-                for (int e = 0; e < V; e++) carry[e] = 0.f;   // previous row ends another sequence
-            } else {
-#pragma unroll
-                for (int e = 0; e < V; e++) carry[e] = gxx[e];
-            }
-#pragma unroll
-            for (int e = 0; e < V; e++) xf[e] = pf[e];         // x[row-1] (only used when t > 0)
-            if (t == 0 && row > r0) IO::ld(x + (size_t)(row - 1) * C + c, xf);
-        }
-    }
-
-    // reduce the parameter gradient over the 8 token lanes
-    __shared__ float red[TL][NOUT][COLS + V];
-#pragma unroll
-    for (int n = 0; n < NOUT; n++)
-#pragma unroll
-        for (int e = 0; e < V; e++) red[tl][n][lane * V + e] = acc[n][e];
-    __syncthreads();
-    for (int i = threadIdx.x; i < NOUT * COLS; i += 256) {
-        const int n = i / COLS, cc = i % COLS;
-        float s = 0.f;
-#pragma unroll
-        for (int l = 0; l < TL; l++) s += red[l][n][cc];
-        const int col = blockIdx.x * COLS + cc;
-        if (col < C) partial[((size_t)blockIdx.y * NOUT + n) * C + col] = s;
-    }
-}
 
 // out[i] = sum_s partial[s][i]
 __global__ void sum_partials_kernel(int S, int n, size_t stride, const float *__restrict__ partial,
@@ -361,28 +201,38 @@ __global__ void scatter_tokens_kernel(int BT, int T, int D, const bf16 *__restri
     }
 }
 
-int grid_for(size_t items, int block) {
-    size_t g = (items + block - 1) / block;
-    const size_t cap = 148 * 16;
-    return (int)(g < 1 ? 1 : (g > cap ? cap : g));
-}
-
 // number of row splits: enough blocks to fill 148 SMs a few times over, at least 8 rows per lane
-int splits_for(long long BT, int C, int cols = 256, int lanes = TL) {
-    const int colblocks = (C + cols - 1) / cols;
+int splits_for(long long BT, int C) {
+    const int colblocks = (C + 255) / 256;
     long long S = (148 * 6 + colblocks - 1) / colblocks;
-    const long long maxS = (BT + lanes * 8 - 1) / (lanes * 8);
+    const long long maxS = (BT + TL * 8 - 1) / (TL * 8);
     if (S > maxS) S = maxS;
     if (S < 1) S = 1;
     return (int)S;
 }
-Split split_of(long long BT, int S, int lanes = TL) {
+Split split_of(long long BT, int S) {
     Split sp;
     sp.rows_per_split = (int)((BT + S - 1) / S);
-    sp.rows_per_lane = (sp.rows_per_split + lanes - 1) / lanes;
+    sp.rows_per_lane = (sp.rows_per_split + TL - 1) / TL;
     return sp;
 }
-constexpr int DD_COLS = 32 * DD_V, DD_LANES = TL;
+
+// the shift-lerp backward entries (nout = 5 with m, 1 and 2 without): the TMA-fed kernel, then the fixed-order sum of
+// its partials when the parameter gradient is wanted.  The caller has checked the arguments.
+int shift_lerp_backward(int nout, int B, int T, int C, const void *x, const void *shift_state, const void *maa, const void *m,
+                        const void *const *gouts, void *gx, void *gm, float *gmaa, void *gshift, void *ws, void *stream) {
+    int slots = 0;
+    const int rc = ddlerp_backward_tma(nout, B, T, C, x, shift_state, maa, m, gouts, gx, gm, shift_state ? gshift : nullptr,
+                                       (float *)ws, &slots, (cudaStream_t)stream);
+    if (rc != WKV6_OK) return rc;
+    if (gmaa) {
+        sum_partials_kernel<<<(nout * C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(slots, nout * C, (size_t)nout * C,
+                                                                                      (const float *)ws, gmaa);
+        count_launch();
+    }
+    WKV6_CUDA_CHECK(cudaGetLastError());
+    return WKV6_OK;
+}
 
 }  // namespace
 }  // namespace wkv6
@@ -393,11 +243,10 @@ extern "C" {
 
 size_t elementwise_backward_workspace_bytes(int B, int T, int C, int nparam) {
     if (B <= 0 || T <= 0 || C <= 0 || nparam <= 0) return 0;
-    const long long BT = (long long)B * T;
     // nparam: 5 ddlerp, 1 shift-lerp, 2 GroupNorm*gate, 3 = the two-output channel-mix shift-lerp (2 rows)
-    size_t slots = nparam == 2 ? splits_for(BT, C) : splits_for(BT, C, DD_COLS, DD_LANES);
-    if (nparam != 2) slots = std::max(slots, ddlerp_tma_partial_slots(nparam == 3 ? 2 : nparam, B, T, C));
-    return slots * (nparam == 3 ? 2 : nparam) * C * sizeof(float);
+    if (nparam == 2) return (size_t)splits_for((long long)B * T, C) * 2 * C * sizeof(float);
+    const int nout = nparam == 3 ? 2 : nparam;
+    return ddlerp_tma_partial_slots(nout, B, T, C) * nout * C * sizeof(float);
 }
 
 int tmix_ddlerp_mix_backward_bf16(int B, int T, int C, const void *x, const void *shift_state, const void *maa,
@@ -405,79 +254,32 @@ int tmix_ddlerp_mix_backward_bf16(int B, int T, int C, const void *x, const void
                                   const void *gxr, const void *gxg, void *gx, void *gm, float *gmaa,
                                   void *gshift, void *ws, size_t ws_bytes, void *stream) {
     if (B < 0 || T < 0 || C <= 0 || (C & 7)) { set_error("tmix_ddlerp_mix_backward_bf16: need C %% 8 == 0"); return WKV6_EINVAL; }
-    const long long BT = (long long)B * T;
-    if (BT == 0) return WKV6_OK;
+    if (B > INT_MAX / 5) { set_error("tmix_ddlerp_mix_backward_bf16: need 5*B <= INT_MAX"); return WKV6_EINVAL; }
+    if ((long long)B * T == 0) return WKV6_OK;
     if (!x || !maa || !m || !gxw || !gxk || !gxv || !gxr || !gxg || !gx || !gm || !ws) {
         set_error("tmix_ddlerp_mix_backward_bf16: null pointer");
         return WKV6_EINVAL;
     }
-    Ptr5 gout;
-    gout.p[0] = (const bf16 *)gxw; gout.p[1] = (const bf16 *)gxk; gout.p[2] = (const bf16 *)gxv;
-    gout.p[3] = (const bf16 *)gxr; gout.p[4] = (const bf16 *)gxg;
     if (ws_bytes < elementwise_backward_workspace_bytes(B, T, C, 5)) { set_error("tmix_ddlerp_mix_backward_bf16: workspace too small"); return WKV6_EINVAL; }
     if (!check_aligned16("tmix_ddlerp_mix_backward_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa", maa}, {"m", m}, {"gxw", gxw},
                                                             {"gxk", gxk}, {"gxv", gxv}, {"gxr", gxr}, {"gxg", gxg}, {"gx", gx}, {"gm", gm},
                                                             {"gshift", shift_state ? gshift : nullptr}}))
         return WKV6_EINVAL;
-    if (wkv6b200_get_impl() != WKV6_IMPL_SIMT) {
-        const void *gs[5] = {gxw, gxk, gxv, gxr, gxg};
-        int slots = 0;
-        const int rc = ddlerp_backward_tma(5, B, T, C, x, shift_state, maa, m, gs, gx, gm, shift_state ? gshift : nullptr,
-                                           (float *)ws, &slots, (cudaStream_t)stream);
-        if (rc <= 0) {
-            if (rc < 0) return rc;
-            if (gmaa) sum_partials_kernel<<<(5 * C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(slots, 5 * C, (size_t)5 * C, (const float *)ws, gmaa);
-            if (gmaa) count_launch();
-            WKV6_CUDA_CHECK(cudaGetLastError());
-            return WKV6_OK;
-        }
-    }
-    const int S = splits_for(BT, C, DD_COLS, DD_LANES);
-    dim3 grid((C + DD_COLS - 1) / DD_COLS, S);
-    ddlerp_bwd_kernel<5, true, DD_V><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        B, T, C, split_of(BT, S, DD_LANES), (const bf16 *)x, (const bf16 *)shift_state, (const bf16 *)maa, (const bf16 *)m,
-        gout, (bf16 *)gx, (bf16 *)gm, shift_state ? (bf16 *)gshift : nullptr, (float *)ws);
-    if (gmaa) sum_partials_kernel<<<(5 * C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, 5 * C, (size_t)5 * C, (const float *)ws, gmaa);
-    count_launch(gmaa ? 2 : 1);
-    WKV6_CUDA_CHECK(cudaGetLastError());
-    return WKV6_OK;
+    const void *gouts[5] = {gxw, gxk, gxv, gxr, gxg};
+    return shift_lerp_backward(5, B, T, C, x, shift_state, maa, m, gouts, gx, gm, gmaa, gshift, ws, stream);
 }
 
 int tmix_shift_lerp_backward_bf16(int B, int T, int C, const void *x, const void *shift_state, const void *maa_x,
                                   const void *gout, void *gx, float *gmaa_x, void *gshift, void *ws,
                                   size_t ws_bytes, void *stream) {
     if (B < 0 || T < 0 || C <= 0 || (C & 7)) { set_error("tmix_shift_lerp_backward_bf16: need C %% 8 == 0"); return WKV6_EINVAL; }
-    const long long BT = (long long)B * T;
-    if (BT == 0) return WKV6_OK;
+    if ((long long)B * T == 0) return WKV6_OK;
     if (!x || !maa_x || !gout || !gx || !ws) { set_error("tmix_shift_lerp_backward_bf16: null pointer"); return WKV6_EINVAL; }
-    Ptr5 g1;
-    for (int i = 0; i < 5; i++) g1.p[i] = (const bf16 *)gout;
     if (ws_bytes < elementwise_backward_workspace_bytes(B, T, C, 1)) { set_error("tmix_shift_lerp_backward_bf16: workspace too small"); return WKV6_EINVAL; }
     if (!check_aligned16("tmix_shift_lerp_backward_bf16", {{"x", x}, {"shift_state", shift_state}, {"maa_x", maa_x}, {"gout", gout}, {"gx", gx},
                                                             {"gshift", shift_state ? gshift : nullptr}}))
         return WKV6_EINVAL;
-    if (wkv6b200_get_impl() != WKV6_IMPL_SIMT) {
-        const void *gs[1] = {gout};
-        int slots = 0;
-        const int rc = ddlerp_backward_tma(1, B, T, C, x, shift_state, maa_x, nullptr, gs, gx, nullptr,
-                                           shift_state ? gshift : nullptr, (float *)ws, &slots, (cudaStream_t)stream);
-        if (rc <= 0) {
-            if (rc < 0) return rc;
-            if (gmaa_x) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(slots, C, (size_t)C, (const float *)ws, gmaa_x);
-            if (gmaa_x) count_launch();
-            WKV6_CUDA_CHECK(cudaGetLastError());
-            return WKV6_OK;
-        }
-    }
-    const int S = splits_for(BT, C, DD_COLS, DD_LANES);
-    dim3 grid((C + DD_COLS - 1) / DD_COLS, S);
-    ddlerp_bwd_kernel<1, false, DD_V><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        B, T, C, split_of(BT, S, DD_LANES), (const bf16 *)x, (const bf16 *)shift_state, (const bf16 *)maa_x, nullptr,
-        g1, (bf16 *)gx, nullptr, shift_state ? (bf16 *)gshift : nullptr, (float *)ws);
-    if (gmaa_x) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, C, (size_t)C, (const float *)ws, gmaa_x);
-    count_launch(gmaa_x ? 2 : 1);
-    WKV6_CUDA_CHECK(cudaGetLastError());
-    return WKV6_OK;
+    return shift_lerp_backward(1, B, T, C, x, shift_state, maa_x, nullptr, &gout, gx, nullptr, gmaa_x, gshift, ws, stream);
 }
 
 int groupnorm_gate_backward_bf16(int BT, int C, int H, float eps, int gate_act, const void *y, const void *g,
@@ -563,15 +365,8 @@ int cmix_shift_lerp2_backward_bf16(int B, int T, int C, const void *x, const voi
     if (!check_aligned16("cmix_shift_lerp2_backward_bf16", {{"x", x}, {"shift_state", shift_state}, {"gxk", gxk}, {"gxr", gxr}, {"gx", gx},
                                                              {"gshift", shift_state ? gshift : nullptr}}))
         return WKV6_EINVAL;
-    const void *gs[2] = {gxk, gxr};
-    int slots = 0;
-    const int rc = ddlerp_backward_tma(2, B, T, C, x, shift_state, maa_kr, nullptr, gs, gx, nullptr, shift_state ? gshift : nullptr,
-                                       (float *)ws, &slots, (cudaStream_t)stream);
-    if (rc != WKV6_OK) return rc;      // (the TMA kernel declines only the five-output form)
-    if (gmaa_kr) sum_partials_kernel<<<(2 * C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(slots, 2 * C, (size_t)2 * C, (const float *)ws, gmaa_kr);
-    if (gmaa_kr) count_launch();
-    WKV6_CUDA_CHECK(cudaGetLastError());
-    return WKV6_OK;
+    const void *gouts[2] = {gxk, gxr};
+    return shift_lerp_backward(2, B, T, C, x, shift_state, maa_kr, nullptr, gouts, gx, nullptr, gmaa_kr, gshift, ws, stream);
 }
 
 }  // extern "C"

@@ -250,6 +250,21 @@ def _ddlerp_fwd(x, shift_state, maa, m):
     return out
 
 
+def _ddlerp_bwd(x, shift_state, maa, m, gouts, need_gmaa):
+    """(gx, gshift, gmaa, gm) of x + xx * (maa_n + m_n) for the five incoming gradients (None = zero)"""
+    lib = _lib.load()
+    B, T, C = x.shape
+    gouts = [torch.zeros_like(x) if g is None else _dense(g) for g in gouts]
+    gx, gm = torch.empty_like(x), torch.empty_like(m)
+    gmaa = torch.empty(5, C, dtype=torch.float32, device=x.device) if need_gmaa else None
+    gshift = torch.empty_like(shift_state) if shift_state is not None else None
+    ws = _ws(lib, B, T, C, 5, x.device)
+    check(lib.tmix_ddlerp_mix_backward_bf16(B, T, C, ptr(x), ptr(shift_state), ptr(maa), ptr(m), *[ptr(g) for g in gouts],
+                                            ptr(gx), ptr(gm), ptr(gmaa), ptr(gshift), ptr(ws), ws.numel(), stream_of(x)),
+          "tmix_ddlerp_mix_backward_bf16")
+    return gx, gshift, (gmaa.to(maa.dtype) if gmaa is not None else None), gm
+
+
 class _DdlerpMix(torch.autograd.Function):
     """Five outputs (views of one [5,B,T,C] buffer), five incoming gradients: the consumers are five
     different Linears, so autograd never has to stack their gradients into one tensor."""
@@ -262,17 +277,7 @@ class _DdlerpMix(torch.autograd.Function):
     @staticmethod
     def backward(ctx, *gouts):
         x, shift_state, maa, m = ctx.saved_tensors
-        lib = _lib.load()
-        B, T, C = x.shape
-        gouts = [torch.zeros_like(x) if g is None else _dense(g) for g in gouts]
-        gx, gm = torch.empty_like(x), torch.empty_like(m)
-        gmaa = torch.empty(5, C, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[2] else None
-        gshift = torch.empty_like(shift_state) if shift_state is not None else None
-        ws = _ws(lib, B, T, C, 5, x.device)
-        check(lib.tmix_ddlerp_mix_backward_bf16(B, T, C, ptr(x), ptr(shift_state), ptr(maa), ptr(m), *[ptr(g) for g in gouts],
-                                                ptr(gx), ptr(gm), ptr(gmaa), ptr(gshift), ptr(ws), ws.numel(), stream_of(x)),
-              "tmix_ddlerp_mix_backward_bf16")
-        return gx, gshift, (gmaa.to(maa.dtype) if gmaa is not None else None), gm
+        return _ddlerp_bwd(x, shift_state, maa, m, gouts, ctx.needs_input_grad[2])
 
 
 def tmix_ddlerp_mix(x, maa_wkvrg, m, shift_state=None):
@@ -302,24 +307,16 @@ class _DdlerpLora(torch.autograd.Function):
     @staticmethod
     def backward(ctx, *gouts):
         x, shift_state, maa, h, w2 = ctx.saved_tensors
-        lib = _lib.load()
         B, T, C = x.shape
         R = w2.shape[1]
         h5 = h.view(B * T, 5, R).transpose(0, 1)                     # [5, BT, R]
         m = torch.bmm(h5, w2).view(5, B, T, C)
-        gouts = [torch.zeros_like(x) if g is None else _dense(g) for g in gouts]
-        gx, gm = torch.empty_like(x), torch.empty_like(m)
-        gmaa = torch.empty(5, C, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[2] else None
-        gshift = torch.empty_like(shift_state) if shift_state is not None else None
-        ws = _ws(lib, B, T, C, 5, x.device)
-        check(lib.tmix_ddlerp_mix_backward_bf16(B, T, C, ptr(x), ptr(shift_state), ptr(maa), ptr(m), *[ptr(g) for g in gouts],
-                                                ptr(gx), ptr(gm), ptr(gmaa), ptr(gshift), ptr(ws), ws.numel(), stream_of(x)),
-              "tmix_ddlerp_mix_backward_bf16")
-        gm5 = gm.view(5, B * T, C)
         need = ctx.needs_input_grad                                  # frozen parameters (LoRA SFT): no cast, no bmm
+        gx, gshift, gmaa, gm = _ddlerp_bwd(x, shift_state, maa, m, gouts, need[2])
+        gm5 = gm.view(5, B * T, C)
         gh = torch.bmm(gm5, w2.transpose(1, 2)).transpose(0, 1).reshape(B * T, 5 * R).view_as(h) if need[3] else None
         gw2 = torch.bmm(h5.transpose(1, 2), gm5) if need[4] else None
-        return gx, gshift, (gmaa.to(maa.dtype) if gmaa is not None else None), gh, gw2
+        return gx, gshift, gmaa, gh, gw2
 
 
 def _ddlerp_lora_fwd(x, shift_state, maa, h, w2):

@@ -109,6 +109,20 @@ def test_misaligned_pointers_are_rejected_before_any_launch(entry):
         assert msg == f"{entry}: {bad} is not 16-byte aligned", (entry, bad, msg)
 
 
+@pytest.mark.skipif(torch.cuda.is_available(),
+                    reason="a library without the check would launch its kernels on the fake addresses")
+def test_ddlerp_backward_rejects_more_than_int_max_m_rows():
+    """The five m planes are read through one tensor map of 5*B rows, an int dimension: B > INT_MAX / 5 is rejected
+    before anything is launched, whatever the workspace."""
+    from rwkv_lm_ext_b200 import _lib
+    lib = _lib.load()
+    names = _ALIGNED_ENTRIES["tmix_ddlerp_mix_backward_bf16"][0]
+    fake = {name: 0x7f0000000000 + 0x100000 * i for i, name in enumerate(names)}
+    shape = {"B": (2**31 - 1) // 5 + 1, "T": 1, "C": 8, "ws_bytes": 1 << 62, "stream": None}
+    rc = lib.tmix_ddlerp_mix_backward_bf16(*[shape[n] if n in shape else fake[n] for n in names])
+    assert rc == -1 and lib.wkv6b200_last_error().decode() == "tmix_ddlerp_mix_backward_bf16: need 5*B <= INT_MAX"
+
+
 def test_product_never_imports_oracle():
     pkg = os.path.join(ROOT, "rwkv_lm_ext_b200")
     for dirpath, _, files in os.walk(pkg):

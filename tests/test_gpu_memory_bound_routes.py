@@ -1,7 +1,7 @@
 """The memory-bound kernels around the recurrence on the routes and at the sizes the per-op tests do not reach:
 
-A. both routes of the token-shift backward (the TMA-fed kernel of "auto" and the register-fed kernel of "simt") at
-   shapes whose row splits and 8-row lanes start in the middle of a sequence, against fp64 autograd;
+A. the token-shift backward at shapes whose splits start in the middle of a sequence, against fp64 autograd, and the
+   same kernel under every setting of the WKV6 route selector;
 B. the later passes of every grid-stride loop (the grid is capped at 148*16 blocks of 256 threads), with a shift
    state so that the t == 0 rows of later passes must find their own row of it;
 C. tensors that are contiguous views at an element offset, which the wrappers must copy to 16-byte aligned storage.
@@ -49,54 +49,17 @@ def _eager_shift(x, st):
 
 
 # --------------------------------------------------------------------------------------------------
-# A. token-shift backward: TMA-fed ("auto") and register-fed ("simt") routes
+# A. token-shift backward
 # --------------------------------------------------------------------------------------------------
-def splits_for(BT, C, cols=256, lanes=8):
-    """csrc/elementwise_bwd.cu splits_for: row splits of the register-fed kernel"""
-    colblocks = (C + cols - 1) // cols
-    S = (148 * 6 + colblocks - 1) // colblocks
-    return max(1, min(S, (BT + lanes * 8 - 1) // (lanes * 8)))
-
-
-def split_of(BT, S, lanes=8):
-    """csrc/elementwise_bwd.cu split_of: (rows per split, rows per 8-row lane) of the flattened B*T rows"""
-    rps = (BT + S - 1) // S
-    return rps, (rps + lanes - 1) // lanes
-
-
-def register_fed_layout(B, T, C):
-    """Which of the places where the register-fed backward can go wrong a shape reaches."""
-    BT = B * T
-    rps, rpl = split_of(BT, splits_for(BT, C))
-    splits = list(range(0, BT, rps))
-    lanes = [(r, min(r + rpl, s + rps, BT)) for s in splits for r in range(s, min(s + rps, BT), rpl)]
-    found = set()
-    if any(r % T and r // T > 0 for r in splits):
-        found.add("split starts mid-sequence in b > 0")
-    if any(r0 % T and (r1 - 1) // T != r0 // T for r0, r1 in lanes):
-        found.add("lane starts mid-sequence and runs into the next one")
-    if T == 1:
-        found.add("every row is t = 0")
-    if BT - splits[-1] < rps:
-        found.add("last split short")
-    return found
-
-
 SHIFT_SHAPES = [
-    # S = 7 splits of 56 rows, lanes of 7 rows: split 3 starts at b=1, t=38
-    (3, 130, 768, True, "split starts mid-sequence in b > 0"),
-    # S = 37 splits of 63 rows, lanes of 8 rows: six lanes run from one sequence into the next
-    (7, 333, 256, True, "lane starts mid-sequence and runs into the next one"),
-    # one split, lanes of 2 rows: every row reads its row of the shift state
-    (16, 1, 2048, True, "every row is t = 0"),
-    # 65 splits of 64 rows, the last one a single row; C = 64 leaves 3/4 of the column lanes idle
-    (1, 4097, 64, False, "last split short"),
-    # 19 splits of 62 rows, the last one 45; seven lanes cross a sequence end
-    (9, 129, 512, True, "last split short"),
-    # 7 splits of 55 rows, lanes of 7 rows; C = 320: the second column block is 1/4 live
-    (5, 77, 320, False, "lane starts mid-sequence and runs into the next one"),
+    (3, 130, 768, True),
+    (7, 333, 256, True),
+    (16, 1, 2048, True),      # every row reads its row of the shift state
+    (1, 4097, 64, False),     # C = 64 leaves 3/4 of the column lanes idle
+    (9, 129, 512, True),
+    (5, 77, 320, False),      # C = 320: the second column block is 1/4 live
 ]
-SHAPE_IDS = [f"{B}x{T}x{C}{'_state' if s else ''}" for B, T, C, s, _ in SHIFT_SHAPES]
+SHAPE_IDS = [f"{B}x{T}x{C}{'_state' if s else ''}" for B, T, C, s in SHIFT_SHAPES]
 
 
 def _shift_inputs(B, T, C, with_state, seed):
@@ -111,7 +74,7 @@ def _shift_inputs(B, T, C, with_state, seed):
 
 
 def _run_shift_backward(M, impl, x, maa_x, maa, m, st, go1, go5):
-    """gradients of tmix_shift_lerp (x, maa_x, st) and tmix_ddlerp_mix (x, maa, m, st) on one route"""
+    """gradients of tmix_shift_lerp (x, maa_x, st) and tmix_ddlerp_mix (x, maa, m, st) under one route setting"""
     M.set_impl(impl)
     try:
         leaves = [t.clone().requires_grad_(True) if t is not None else None for t in (x, maa_x, maa, m, st)]
@@ -126,12 +89,10 @@ def _run_shift_backward(M, impl, x, maa_x, maa, m, st, go1, go5):
     return g1, g5
 
 
-@pytest.mark.parametrize("impl", ["auto", "simt"])
-@pytest.mark.parametrize("B,T,C,with_state,layout", SHIFT_SHAPES, ids=SHAPE_IDS)
-def test_shift_lerp_backward_against_fp64(M, impl, B, T, C, with_state, layout):
-    assert layout in register_fed_layout(B, T, C)
+@pytest.mark.parametrize("B,T,C,with_state", SHIFT_SHAPES, ids=SHAPE_IDS)
+def test_shift_lerp_backward_against_fp64(M, B, T, C, with_state):
     x, maa_x, maa, m, st, go1, go5 = _shift_inputs(B, T, C, with_state, seed=B * 1000 + T)
-    g1, g5 = _run_shift_backward(M, impl, x, maa_x, maa, m, st, go1, go5)
+    g1, g5 = _run_shift_backward(M, "auto", x, maa_x, maa, m, st, go1, go5)
 
     l64 = [t.double().requires_grad_(True) if t is not None else None for t in (x, maa_x, maa, m, st)]
     x64, maa_x64, maa64, m64, st64 = l64
@@ -140,33 +101,32 @@ def test_shift_lerp_backward_against_fp64(M, impl, B, T, C, with_state, layout):
     out5 = torch.stack([x64 + xx * (maa64[n] + m64[n]) for n in range(5)])
     want5 = torch.autograd.grad(out5, [t for t in (x64, maa64, m64, st64) if t is not None], go5.double())
     for name, got, want in zip(("gx", "gmaa_x", "gshift"), g1, want1):
-        assert_bf16_close(got, want, f"{impl} shift_lerp {name}")
+        assert_bf16_close(got, want, f"shift_lerp {name}")
     for name, got, want in zip(("gx", "gmaa", "gm", "gshift"), g5, want5):
-        assert_bf16_close(got, want, f"{impl} ddlerp {name}")
+        assert_bf16_close(got, want, f"ddlerp {name}")
 
 
-@pytest.mark.parametrize("B,T,C,with_state,layout", SHIFT_SHAPES, ids=SHAPE_IDS)
-def test_shift_lerp_backward_routes_agree(M, B, T, C, with_state, layout):
-    """gm = bf16(gout * xx) is one rounding per element on both routes: bit-equal.  gx, gmaa, gshift are the same sums
-    in another order.  The profiler shows that each route runs its own kernel."""
+@pytest.mark.parametrize("B,T,C,with_state", SHIFT_SHAPES, ids=SHAPE_IDS)
+def test_shift_lerp_backward_is_the_same_kernel_under_simt(M, B, T, C, with_state):
+    """set_impl chooses the route of the WKV6 recurrence only: under "simt" the profiler shows the TMA-fed kernel of
+    "auto" and nothing else, and every gradient is bit-equal (the kernel and the partial sums have no atomics)."""
     args = _shift_inputs(B, T, C, with_state, seed=B * 1000 + T + 7)
     got = {}
-    for impl, kernel, other in (("auto", "ddlerp_bwd_tma_kernel", "ddlerp_bwd_kernel"),
-                                ("simt", "ddlerp_bwd_kernel", "ddlerp_bwd_tma_kernel")):
+    for impl in ("auto", "simt"):
         with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
             got[impl] = _run_shift_backward(M, impl, *args)
         names = {e.name for e in prof.events()}
-        assert any(kernel in n for n in names) and not any(other in n for n in names), (impl, sorted(n for n in names if "ddlerp" in n))
+        assert any("ddlerp_bwd_tma_kernel" in n for n in names) and not any("ddlerp_bwd_kernel" in n for n in names), \
+            (impl, sorted(n for n in names if "ddlerp" in n))
     (a1, a5), (s1, s5) = got["auto"], got["simt"]
-    assert torch.equal(a5[2], s5[2]), "gm differs between the routes"
     for name, a, s in zip(("shift_lerp gx", "shift_lerp gmaa_x", "shift_lerp gshift"), a1, s1):
-        assert_bf16_close(s, a, name)
+        assert torch.equal(a, s), name
     for name, a, s in zip(("ddlerp gx", "ddlerp gmaa", "ddlerp gm", "ddlerp gshift"), a5, s5):
-        assert_bf16_close(s, a, name)
+        assert torch.equal(a, s), name
 
 
-@pytest.mark.parametrize("B,T,C,with_state,layout", SHIFT_SHAPES, ids=SHAPE_IDS)
-def test_cmix_shift_lerp2_backward_against_fp64(M, B, T, C, with_state, layout):
+@pytest.mark.parametrize("B,T,C,with_state", SHIFT_SHAPES, ids=SHAPE_IDS)
+def test_cmix_shift_lerp2_backward_against_fp64(M, B, T, C, with_state):
     x, maa_k, maa_r = _randn(B, T, C, seed=T), _rand(C, seed=T + 1), _rand(C, seed=T + 2)
     st = _randn(B, C, seed=T + 3) if with_state else None
     gk, gr = _randn(B, T, C, seed=T + 4), _randn(B, T, C, seed=T + 5)
