@@ -125,6 +125,17 @@ WKV6_API int wkv6_train_backward(int B, int T, int C, int H, const void *r, cons
                         const void *w, const void *u, const void *s0, int s0_batched, const void *gy,
                         void *gr, void *gk, void *gv, void *gw, void *gu, void *gu_total, void *gs,
                         const void *saved, void *workspace, size_t workspace_bytes, void *stream);
+/* The same backward when the loss also depends on the final state S_T (chunked long-context training that
+ * carries the state from one chunk to the next and lets its gradient flow back): gT = dL/dS_T, bf16
+ * (gT_f32 = 0) or fp32 (gT_f32 = 1) [B,H,64(value),64(key)] like sT, 16-byte aligned, non-NULL (wkv6_train_backward
+ * is this call with gT = NULL).  The reverse sweep starts from gT instead of 0, so gw[:,T-1] is no longer forced
+ * to 0 (the last decay feeds the final state); it is an exact 0 again where gT is 0.  Same `saved` and workspace as wkv6_train_backward;
+ * the exact SIMT route (wkv6b200_set_impl) takes B*H*64*4 bytes of stream-ordered scratch on top. */
+WKV6_API int wkv6_train_backward_state_grad(int B, int T, int C, int H, const void *r, const void *k, const void *v,
+                                   const void *w, const void *u, const void *s0, int s0_batched, const void *gy,
+                                   void *gr, void *gk, void *gv, void *gw, void *gu, void *gu_total, void *gs,
+                                   const void *gT, int gT_f32, const void *saved, void *workspace,
+                                   size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * (a3) wkv6state -- cuda/wkv6state_cuda.cu:298-311 bound by cuda/wkv6state_op.cpp:8-21.

@@ -4,7 +4,8 @@ Importing the package does not touch the GPU or the shared library; the first op
 ``libwkv6_b200.so`` and raises if it is missing (there is no CPU / eager fallback)."""
 from ._lib import LIB_PATH, Wkv6B200Error, launch_count, load, set_decay_clamp, set_impl  # noqa: F401
 from .ops import (HEAD_SIZE, RUN_CUDA_RWKV6, RUN_CUDA_RWKV6_BI, RUN_CUDA_RWKV6_STATE, RUN_RWKV_6, RWKV_6,  # noqa: F401
-                  WKV_6, WKV_6_BI, WKV_6STATE, WKV_6STATE_INFCTX, exact_route_report, install, rwkv6, wkv6_bi_cuda, wkv6_cuda,
+                  RUN_CUDA_RWKV6_STATE_BPTT, WKV_6, WKV_6_BI, WKV_6STATE, WKV_6STATE_BPTT, WKV_6STATE_INFCTX,
+                  exact_route_report, install, rwkv6, wkv6_bi_cuda, wkv6_cuda,
                   wkv6infctx_cuda, wkv6state_cuda)
 from .heads import (add_layernorm, create_mask_and_rev_idx, eos_gather, eos_index, gather_rows, groupnorm_gate, groupnorm_gate_pair, pooling,  # noqa: F401
                     reverse_x, tmix_ddlerp_lora, tmix_ddlerp_mix, tmix_shift_lerp)

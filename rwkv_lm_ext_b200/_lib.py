@@ -31,6 +31,7 @@ SIGNATURES = {
     "wkv6_train_backward_workspace_bytes": (c_sz, _BTCH + [c_i]),
     "wkv6_train_forward": (c_i, _BTCH + [c_p] * 6 + [c_i, c_i, c_p, c_i, c_p, c_p, ctypes.POINTER(c_i), c_p]),
     "wkv6_train_backward": (c_i, _BTCH + [c_p] * 6 + [c_i] + [c_p] * 10 + [c_sz, c_p]),
+    "wkv6_train_backward_state_grad": (c_i, _BTCH + [c_p] * 6 + [c_i] + [c_p] * 9 + [c_i] + [c_p] * 2 + [c_sz, c_p]),
     "wkv6state_forward": (c_i, _BTCH + [c_p] * 8),
     "wkv6state_backward": (c_i, _BTCH + [c_p] * 14 + [c_sz, c_p]),
     "wkv6infctx_forward": (c_i, _BTCH + [c_p] * 8),

@@ -51,6 +51,9 @@ struct Args {
     const void *gy = nullptr;
     void *gr = nullptr, *gk = nullptr, *gv = nullptr, *gw = nullptr, *gu = nullptr, *gs = nullptr;
     void *gu_total = nullptr;         // training pair only: bf16 [C], sum of gu over the batch rows
+    // training pair only: nullptr (the final state feeds nothing) | dL/dS_T, bf16/fp32 [B,H,64(value),64(key)]
+    const void *gT = nullptr;
+    int gT_f32 = 0;
     mutable bool gu_total_done = false;   // set by the route whose kernel added the rows itself
     void *workspace = nullptr;
     size_t workspace_bytes = 0;

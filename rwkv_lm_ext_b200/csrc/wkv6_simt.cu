@@ -141,11 +141,12 @@ __global__ void __launch_bounds__(NT) fwd_kernel(Args a, int mode) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// backward, forward-time sweep: gr, gu partials, A_t[i] = r_t[i] * sum_j S_t[i][j] gy_t[j]
+// backward, forward-time sweep: gr, gu partials, A_t[i] = r_t[i] * sum_j S_t[i][j] gy_t[j];
+// with a final-state gradient also Q0[b,h,i] = sum_j S_T[i][j] gT[i][j], where the reverse sweep's Q starts
 // thread (x = i, g): S[i = x][j in 16g..16g+15]
 // ---------------------------------------------------------------------------------------------
 template <typename IO, int WK>
-__global__ void __launch_bounds__(NT) bwd_f_kernel(Args a, int mode, float *Abuf) {
+__global__ void __launch_bounds__(NT) bwd_f_kernel(Args a, int mode, float *Abuf, float *Q0) {
     if (a.stream_flags && a.stream_flags[blockIdx.x] == 0) return;
     const int b = blockIdx.x / a.H, h = blockIdx.x % a.H;
     const int x = threadIdx.x & (N - 1), g = threadIdx.x >> 6;
@@ -242,17 +243,27 @@ __global__ void __launch_bounds__(NT) bwd_f_kernel(Args a, int mode, float *Abuf
         __syncthreads();
         if (g == 0)
             ((IO *)a.gu)[(size_t)b * C + h * N + x] = from_f32<IO>(sgu[0][x] + sgu[1][x] + sgu[2][x] + sgu[3][x]);
+        if (a.gT) {
+            float q = 0.f;
+#pragma unroll
+            for (int jj = 0; jj < SL; jj++)
+                q = fmaf(S[jj], load_state<IO>(a.gT, a.gT_f32, ((size_t)blockIdx.x * N + g * SL + jj) * N + x), q);
+            __syncthreads();
+            sgu[g][x] = q;
+            __syncthreads();
+            if (g == 0) Q0[(size_t)blockIdx.x * N + x] = sgu[0][x] + sgu[1][x] + sgu[2][x] + sgu[3][x];
+        }
     }
 }
 
 // ---------------------------------------------------------------------------------------------
-// backward, reverse-time sweep: gk, gv, gw, gs.  G = dL/dS_{t+1}.
+// backward, reverse-time sweep: gk, gv, gw, gs.  G = dL/dS_{t+1}, starting from gT (or 0).
 //   G1: thread (x = i, g) holds G[i][j in slice]  -> gk_t[i], B_t[i] = k_t[i] sum_j G[i][j] v_t[j]
 //   G2: thread (x = j, g) holds G[i in slice][j]  -> gv_t[j]
-//   gl_t = Q - B_t ;  Q += A_t - B_t   (Q = sum_{s>t}(A_s - B_s));  gw_t = l_t * gl_t
+//   gl_t = Q - B_t ;  Q += A_t - B_t   (Q = Q0 + sum_{s>t}(A_s - B_s));  gw_t = l_t * gl_t
 // ---------------------------------------------------------------------------------------------
 template <typename IO, int WK>
-__global__ void __launch_bounds__(NT, 2) bwd_r_kernel(Args a, int mode, const float *Abuf) {   // 2 blocks per SM: at most 128 registers
+__global__ void __launch_bounds__(NT, 2) bwd_r_kernel(Args a, int mode, const float *Abuf, const float *Q0) {   // 2 blocks per SM: at most 128 registers
     if (a.stream_flags && a.stream_flags[blockIdx.x] == 0) return;
     const int b = blockIdx.x / a.H, h = blockIdx.x % a.H;
     const int x = threadIdx.x & (N - 1), g = threadIdx.x >> 6;
@@ -270,6 +281,10 @@ __global__ void __launch_bounds__(NT, 2) bwd_r_kernel(Args a, int mode, const fl
 #pragma unroll
     for (int q = 0; q < SL; q++) {
         G1[q] = 0.f; G2[q] = 0.f;
+        if (a.gT && !rev) {
+            G1[q] = load_state<IO>(a.gT, a.gT_f32, ((size_t)blockIdx.x * N + g * SL + q) * N + x);
+            G2[q] = load_state<IO>(a.gT, a.gT_f32, ((size_t)blockIdx.x * N + x) * N + g * SL + q);
+        }
         uu[q] = rev ? 0.f : to_f32(((const IO *)a.u)[h * N + g * SL + q]);
     }
     const float ui = rev ? 0.f : to_f32(((const IO *)a.u)[h * N + x]);
@@ -277,7 +292,8 @@ __global__ void __launch_bounds__(NT, 2) bwd_r_kernel(Args a, int mode, const fl
     IO *GK = (IO *)a.gk, *GV = (IO *)a.gv, *GW = (IO *)a.gw;
     const size_t base = (size_t)b * T * C + (size_t)h * N;
     const bool zero_gw0 = (a.s0 == nullptr) || rev;
-    float Q = 0.f;  // meaningful in threads with g == 0 (x = i)
+    float Q = a.gT && !rev ? Q0[(size_t)blockIdx.x * N + x] : 0.f;  // meaningful in threads with g == 0 (x = i)
+    const bool zero_gw_last = a.gT == nullptr || rev;   // the last decay feeds nothing but the final state
 
     const int ntiles = (Teff + TR - 1) / TR;
     float pr[PER], pk[PER], pl[PER], pv[PER], pg[PER], pa[PER];
@@ -353,7 +369,7 @@ __global__ void __launch_bounds__(NT, 2) bwd_r_kernel(Args a, int mode, const fl
                 float gkv = fmaf(ui * sr[tt][x], vg, gvd);
                 const float Bt = sk[tt][x] * gvd;
                 float gwv = sl[tt][x] > a.lmin ? sl[tt][x] * (Q - Bt) : 0.f;   // a clamped decay no longer depends on w
-                if (tau == Teff - 1 || (tau == 0 && zero_gw0)) gwv = 0.f;
+                if ((tau == Teff - 1 && zero_gw_last) || (tau == 0 && zero_gw0)) gwv = 0.f;
                 Q += sA[tt][x] - Bt;
                 if (rev) { gkv += to_f32(GK[o]); gwv += to_f32(GW[o]); }
                 GK[o] = from_f32<IO>(gkv);
@@ -390,16 +406,17 @@ int launch_fwd(const Args &a, int mode) {
     return WKV6_OK;
 }
 
-int launch_bwd(const Args &a, int mode) {
+// Q0: nullptr, or fp32 [B*H][64] that carries <S_T, gT>_i from the forward-time sweep to the reverse one
+int launch_bwd(const Args &a, int mode, float *Q0) {
     using IO = __nv_bfloat16;
     const dim3 grid(a.B * a.H), block(NT);
     float *A = (float *)a.workspace;
     if (a.w_kind == W_RAW_BF16) {
-        bwd_f_kernel<IO, W_RAW_BF16><<<grid, block, 0, a.stream>>>(a, mode, A);
-        bwd_r_kernel<IO, W_RAW_BF16><<<grid, block, 0, a.stream>>>(a, mode, A);
+        bwd_f_kernel<IO, W_RAW_BF16><<<grid, block, 0, a.stream>>>(a, mode, A, Q0);
+        bwd_r_kernel<IO, W_RAW_BF16><<<grid, block, 0, a.stream>>>(a, mode, A, Q0);
     } else {
-        bwd_f_kernel<IO, W_LOG_F32><<<grid, block, 0, a.stream>>>(a, mode, A);
-        bwd_r_kernel<IO, W_LOG_F32><<<grid, block, 0, a.stream>>>(a, mode, A);
+        bwd_f_kernel<IO, W_LOG_F32><<<grid, block, 0, a.stream>>>(a, mode, A, Q0);
+        bwd_r_kernel<IO, W_LOG_F32><<<grid, block, 0, a.stream>>>(a, mode, A, Q0);
     }
     count_launch(2);
     WKV6_CUDA_CHECK(cudaGetLastError());
@@ -429,9 +446,19 @@ int simt_backward(const Args &a) {
         set_error("workspace too small: need %zu bytes", simt_backward_workspace_bytes(a.B, a.T, a.H));
         return WKV6_EWORKSPACE;
     }
-    int rc = launch_bwd(a, 0);
+    if (a.gT) {
+        // the final-state gradient (training pair only, never with a mask): <S_T, gT> in stream-ordered scratch, so the
+        // workspace of a call without one stays what it was
+        ensure_pool_keeps_memory();
+        float *Q0 = nullptr;
+        WKV6_CUDA_CHECK(cudaMallocAsync((void **)&Q0, (size_t)a.B * a.H * N * sizeof(float), a.stream));
+        const int rc = launch_bwd(a, 0, Q0);
+        cudaFreeAsync(Q0, a.stream);
+        return rc;
+    }
+    int rc = launch_bwd(a, 0, nullptr);
     if (rc != WKV6_OK || !a.mask) return rc;
-    return launch_bwd(a, 1);
+    return launch_bwd(a, 1, nullptr);
 }
 
 }  // namespace wkv6

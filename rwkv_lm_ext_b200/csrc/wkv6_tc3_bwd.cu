@@ -86,9 +86,10 @@ struct Params {
     int has_s0;
     // time-axis segmentation (seg_scan.cu): the grid has B*nseg rows; row = b*nseg + seg covers tokens
     // [seg*seg_chunks*64, min(T, (seg+1)*seg_chunks*64)) of sequence b; g_init = dL/dS behind the last token of
-    // each row, fp32 [rows,H,64(value),64(key)]; gu, gs, flags and checkpoints are indexed by row.
-    // nseg = 1, seg_chunks = ceil(T/64), g_init = nullptr for an ordinary call.
-    const float *g_init;
+    // each row, [rows,H,64(value),64(key)], fp32 or (g_init_f32 = 0) bf16; gu, gs, flags and checkpoints are indexed
+    // by row.  nseg = 1, seg_chunks = ceil(T/64), g_init = nullptr for an ordinary call; the SEG instantiation with
+    // nseg = 1 and g_init = the caller's final-state gradient for an ordinary call that has one.
+    const void *g_init;
     int nseg, seg_chunks;
     float lmin;               // floor of the per-token log2-decay (>= -LCLAMP2)
     bf16 *gu, *gs;
@@ -98,7 +99,16 @@ struct Params {
     const int *row_len;       // BI modes: tokens of every batch row (p + 1 of wkv6_bi), device int [B]
     const int *row_order;     // BI modes: batch rows sorted by length, longest first, device int [B]
     long long *dbg;           // nullptr, or [gridDim][NC][8 (32 in the profiling build)] clock64 stamps of warp 0 at the stage boundaries (profiling aid)
+    int g_init_f32;           // (last: the fields above keep their offsets, and SEG = false reads none of the new ones)
 };
+
+// true when `x` holds in any of the 256 compute threads (named barrier B_SCAN, which they all reach)
+__device__ __forceinline__ bool compute_any(bool x) {
+    uint32_t r;
+    asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.u32 p, %1, 0;\n\tbar.red.or.pred q, %2, %3, p;\n\tselp.u32 %0, 1, 0, q;\n\t}"
+                 : "=r"(r) : "r"((uint32_t)x), "n"(B_SCAN_ID), "n"(CTHREADS) : "memory");
+    return r != 0;
+}
 
 __device__ __forceinline__ uint32_t pack_frag(const uint32_t *v, int g, int hh) {
     return pack2(__uint_as_float(v[4 * g + 2 * hh]), __uint_as_float(v[4 * g + 2 * hh + 1]));
@@ -372,20 +382,29 @@ wkv6_tc3_bwd_kernel(const __grid_constant__ CUtensorMap map_r, const __grid_cons
         int sig[2] = {0, 0};              // G in TMEM = G_true 2^(-sig) per key row: rho_0 of the chunk processed last
         uint32_t v[16];
 
-        // G = dL/dS behind the last token (0, or handed in when this row is a segment)
+        // G = dL/dS behind the last token (0, or handed in: a segment's scanned G, or the caller's final-state gradient)
         const int seg = SEG ? row % p.nseg : 0;
         const bool first_has_s0 = p.has_s0 || seg > 0;          // a later segment starts from a non-zero state
-        const bool g_is_zero = !SEG || p.g_init == nullptr || seg == p.nseg - 1;
+        bool g_is_zero = !SEG || p.g_init == nullptr;
 #pragma unroll
         for (int x = 0; x < 16; x++) v[x] = 0u;
         if (!g_is_zero) {
+            bool nz = false;
 #pragma unroll
             for (int g = 0; g < 4; g++)
 #pragma unroll
                 for (int hh = 0; hh < 2; hh++)
 #pragma unroll
-                    for (int e = 0; e < 2; e++)
-                        v[4 * g + 2 * hh + e] = __float_as_uint(p.g_init[(((size_t)row * p.H + h) * 64 + F.col(g, e)) * 64 + F.row(hh)]);
+                    for (int e = 0; e < 2; e++) {
+                        const size_t gi = (((size_t)row * p.H + h) * 64 + F.col(g, e)) * 64 + F.row(hh);
+                        const float gv = p.g_init_f32 ? static_cast<const float *>(p.g_init)[gi]
+                                                      : __bfloat162float(static_cast<const bf16 *>(p.g_init)[gi]);
+                        v[4 * g + 2 * hh + e] = __float_as_uint(gv);
+                        nz |= gv != 0.f;
+                    }
+            // the stream's last segment: its G is the final-state gradient, and where that is 0 the last decay feeds
+            // nothing, so its gw stays an exact 0 (what the call without a final-state gradient computes)
+            if (seg == p.nseg - 1) g_is_zero = !compute_any(nz);
         }
         tmem_st_frag(tG, v);
         tmem_wait_st();
@@ -988,9 +1007,11 @@ static int launch_bwd_kernel(dim3 grid, cudaStream_t stream, const CUtensorMap *
 
 // one launch of the backward kernel on `a` viewed as given (B rows of T tokens), chunk-start states in ckpt
 // gu_count: nullptr, or the zeroed per-head arrival counters that let an ordinary call add gu up into a.gu_total
+// g_init: nullptr, or dL/dS behind every row's last token (g_init_f32: fp32, else bf16); an unsegmented call with one
+// runs the SEG instantiation with nseg = 1 (which leaves gu_total to the caller)
 // bi / row_len: direction of the bidirectional op (tc3_common.cuh) and the device int [B] row lengths it needs
-static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu_count, const float *g_init, int nseg,
-                      int seg_chunks, bool has_s0, int bi = BI_NONE, const int *row_len = nullptr,
+static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu_count, const void *g_init, int g_init_f32,
+                      int nseg, int seg_chunks, bool has_s0, int bi = BI_NONE, const int *row_len = nullptr,
                       const int *row_order = nullptr) {
     const int C = a.H * 64;
     if (nseg <= 1) { nseg = 1; seg_chunks = (a.T + L - 1) / L; }
@@ -1011,13 +1032,13 @@ static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu
     p.B = a.B; p.T = a.T; p.H = a.H;
     p.u = (const bf16 *)a.u;
     p.has_s0 = has_s0;
-    p.g_init = g_init;
+    p.g_init = g_init; p.g_init_f32 = g_init_f32;
     p.nseg = nseg; p.seg_chunks = seg_chunks;
     p.lmin = tc_lmin_log2(a);
     p.gu = (bf16 *)a.gu; p.gs = (bf16 *)a.gs;
     p.hz_flags = flags;
     // in-kernel sum of gu over the rows: ordinary call only
-    const bool sum_gu = a.gu_total && gu_count && nseg == 1 && bi == BI_NONE && a.H <= 512;
+    const bool sum_gu = a.gu_total && gu_count && nseg == 1 && !g_init && bi == BI_NONE && a.H <= 512;
     p.gu_total = sum_gu ? (bf16 *)a.gu_total : nullptr;
     p.gu_count = gu_count;
     if (sum_gu) a.gu_total_done = true;
@@ -1032,7 +1053,7 @@ static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu
     int rc;
     if (bi == BI_CAUSAL) rc = launch_bwd_kernel<false, BI_CAUSAL>(grid, a.stream, maps, p);
     else if (bi == BI_REV) rc = launch_bwd_kernel<false, BI_REV>(grid, a.stream, maps, p);
-    else if (nseg > 1) rc = launch_bwd_kernel<true, BI_NONE>(grid, a.stream, maps, p);
+    else if (nseg > 1 || g_init) rc = launch_bwd_kernel<true, BI_NONE>(grid, a.stream, maps, p);
     else rc = launch_bwd_kernel<false, BI_NONE>(grid, a.stream, maps, p);
     if (rc != WKV6_OK) return rc;
     if (clamp) {                       // opt-in decay clamp: a clamped decay no longer depends on w (kept out of the hot kernel)
@@ -1069,10 +1090,11 @@ static int tc3_backward_segmented(const Args &a, int nseg, int seg_chunks) {
     f.s0 = nullptr; f.s0_bstride = 0; f.s0_f32 = 0; f.sT = g_loc; f.sT_f32 = 1; f.y = nullptr; f.saved = nullptr; f.gy = nullptr;
     if (rc == WKV6_OK) rc = tc3_forward(f, nullptr, nullptr, nseg, seg_chunks);
     if (rc == WKV6_OK) rc = seg_decay(a.B, a.T, C, nseg, seg_tokens, a.w, lam, tc_lmin_nats(a), a.stream);
-    if (rc == WKV6_OK) rc = seg_scan(a.B, nseg, a.H, lam, g_loc, nullptr, 0, 0, g_end, nullptr, 0, 1, nullptr, a.stream);
+    // the chain starts from the caller's final-state gradient (or 0), which the last segment then reads like the others
+    if (rc == WKV6_OK) rc = seg_scan(a.B, nseg, a.H, lam, g_loc, a.gT, a.gT_f32, (long long)a.H * 4096, g_end, nullptr, 0, 1, nullptr, a.stream);
     Args v = a;
     v.gu = gu_tmp; v.gs = a.gs ? gs_tmp : nullptr;
-    if (rc == WKV6_OK) rc = launch_bwd(v, ckpt, nullptr, nullptr, g_end, nseg, seg_chunks, a.s0 != nullptr);
+    if (rc == WKV6_OK) rc = launch_bwd(v, ckpt, nullptr, nullptr, g_end, 1, nseg, seg_chunks, a.s0 != nullptr);
     if (rc == WKV6_OK) rc = seg_sum_gu(a.B, nseg, C, gu_tmp, a.gu, a.stream);
     if (rc == WKV6_OK && a.gs)                    // dL/dS_0 is what segment 0 of every sequence produced
         rc = cudaMemcpy2DAsync(a.gs, (size_t)a.H * 4096 * 2, gs_tmp, (size_t)nseg * a.H * 4096 * 2, (size_t)a.H * 4096 * 2, a.B,
@@ -1087,7 +1109,7 @@ int tc3_backward_bi(const Args &a, void *ckpt, int *flags, int bi, const int *ro
     Args f = a;
     f.y = nullptr; f.sT = nullptr; f.s0 = nullptr;
     if (int rc = tc3_forward(f, ckpt, flags, 1, 0, bi, row_len, row_order)) return rc;
-    return launch_bwd(a, (const bf16 *)ckpt, flags, nullptr, nullptr, 1, 0, false, bi, row_len, row_order);
+    return launch_bwd(a, (const bf16 *)ckpt, flags, nullptr, nullptr, 0, 1, 0, false, bi, row_len, row_order);
 }
 
 int tc3_backward(const Args &a, int *flags) {
@@ -1114,7 +1136,7 @@ int tc3_backward(const Args &a, int *flags) {
         f.sT = nullptr;
         if (int rc = tc3_forward(f, ckpt, flags)) return rc;
     }
-    return launch_bwd(a, ckpt, flags, gu_count, nullptr, 1, 0, a.s0 != nullptr);
+    return launch_bwd(a, ckpt, flags, gu_count, a.gT, a.gT_f32, 1, 0, a.s0 != nullptr);
 }
 
 }  // namespace wkv6

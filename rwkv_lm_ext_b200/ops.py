@@ -75,15 +75,21 @@ class exact_route_report:
         return 0, self._streams
 
 
-def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs):
-    """Returns gu summed over the batch rows (src/model.py:232 `torch.sum(gu, 0)`), computed by the library."""
+def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs, gT=None):
+    """Returns gu summed over the batch rows (src/model.py:232 `torch.sum(gu, 0)`), computed by the library.
+    gT: None, or the gradient of the final state (bf16/fp32 [B,H,64,64], contiguous, 16-byte aligned)."""
     saved = ctx.saved_state
     n = lib.wkv6_train_backward_workspace_bytes(B, T, C, H, int(saved is not None))
     ws = torch.empty(max(n, 1), dtype=torch.uint8, device=gy.device)
     gu_total = torch.empty((C,), device=gy.device, dtype=torch.bfloat16)
-    check(lib.wkv6_train_backward(B, T, C, H, ptr(r), ptr(k), ptr(v), ptr(w), ptr(u), ptr(s0), int(s0_batched),
-                                  ptr(gy), ptr(gr), ptr(gk), ptr(gv), ptr(gw), ptr(gu), ptr(gu_total), ptr(gs), ptr(saved),
-                                  ptr(ws), n, stream_of(gy)), "wkv6_train_backward")
+    head = (B, T, C, H, ptr(r), ptr(k), ptr(v), ptr(w), ptr(u), ptr(s0), int(s0_batched),
+            ptr(gy), ptr(gr), ptr(gk), ptr(gv), ptr(gw), ptr(gu), ptr(gu_total), ptr(gs))
+    tail = (ptr(saved), ptr(ws), n, stream_of(gy))
+    if gT is None:
+        check(lib.wkv6_train_backward(*head, *tail), "wkv6_train_backward")
+    else:
+        check(lib.wkv6_train_backward_state_grad(*head, ptr(gT), int(gT.dtype == torch.float32), *tail),
+              "wkv6_train_backward_state_grad")
     return gu_total
 
 
@@ -204,6 +210,60 @@ class WKV_6STATE_INFCTX(torch.autograd.Function):
             # batch into [H,64,64] even here, src/model.py:128 -- a shape that cannot flow back
             # into a [B,H,64,64] leaf; truncated BPTT: the final state gets no gradient.)
             return (None, None, None, None, gr, gk, gv, gw, gu, gs.to(ctx.s_dtype))
+
+
+class WKV_6STATE_BPTT(torch.autograd.Function):
+    """The infctx operator with gradients through the carried state: out of place (``s`` is read, never written;
+    ``s_final`` is a new tensor with the dtype of ``s``, bf16 or the fp32 carry), and the gradient of ``s_final``
+    flows back into r, k, v, w, u and ``s``.  Chunked long-context training then computes the gradients of one
+    pass over the whole sequence.  A ``s_final`` that feeds nothing (gradient None) runs the backward of
+    WKV_6STATE_INFCTX."""
+
+    @staticmethod
+    def forward(ctx, B, T, C, H, r, k, v, w, u, s):
+        with torch.no_grad():
+            _assert_bf16_contig(r, k, v, w, u)
+            assert s.dtype in (torch.bfloat16, torch.float32)
+            assert s.is_contiguous()
+            assert HEAD_SIZE == C // H
+            _require_cuda(r)
+            assert tuple(s.shape) == (B, H, HEAD_SIZE, HEAD_SIZE)
+            ctx.B, ctx.T, ctx.C, ctx.H = B, T, C, H
+            ctx.save_for_backward(r, k, v, w, u, s.to(torch.bfloat16))
+            y = torch.empty((B, T, C), device=r.device, dtype=torch.bfloat16, memory_format=torch.contiguous_format)
+            s_final = torch.empty_like(s, memory_format=torch.contiguous_format)
+            lib = _lib.load()
+            _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, s_final, y)
+            ctx.s_dtype = s.dtype
+            return y, s_final
+
+    @staticmethod
+    def backward(ctx, gy, gs_final):
+        with torch.no_grad():
+            B, T, C, H = ctx.B, ctx.T, ctx.C, ctx.H
+            r, k, v, w, u, s = ctx.saved_tensors
+            if gy is None:                                         # only the final state feeds the loss
+                gy = torch.zeros((B, T, C), device=r.device, dtype=torch.bfloat16)
+            assert gy.dtype == torch.bfloat16
+            gy = gy.contiguous()
+            gr, gk, gv, gw = (torch.empty((B, T, C), device=gy.device, dtype=torch.bfloat16) for _ in range(4))
+            gu = torch.empty((B, C), device=gy.device, dtype=torch.bfloat16)
+            gs = torch.empty((B, H, C // H, C // H), device=gy.device, dtype=torch.bfloat16)
+            gT = None
+            if gs_final is not None:
+                gT = gs_final.contiguous()
+                assert gT.dtype in (torch.bfloat16, torch.float32) and tuple(gT.shape) == (B, H, HEAD_SIZE, HEAD_SIZE)
+                if gT.data_ptr() % 16:                             # the library reads it with 16-byte accesses
+                    gT = gT.clone()
+            lib = _lib.load()
+            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs, gT)
+            gu = gu.view(H, C // H)
+            return (None, None, None, None, gr, gk, gv, gw, gu, gs.to(ctx.s_dtype))
+
+
+def RUN_CUDA_RWKV6_STATE_BPTT(B, T, C, H, r, k, v, w, u, s):
+    """(y, s_final) of the infctx operator, differentiable through s_final (WKV_6STATE_BPTT); ``s`` is not modified."""
+    return WKV_6STATE_BPTT.apply(B, T, C, H, r, k, v, w, u, s)
 
 
 def RUN_CUDA_RWKV6_STATE(B, T, C, H, r, k, v, w, u, s):

@@ -20,6 +20,9 @@ serves SFT.  Variants: `time_state` attribute present -> state tuning (src/model
 `last_state` given -> infctx (src/model.py:738-781): a `TimeMixState` (the reference's or
 rwkv_lm_ext_b200.infctx's) returns `(out, TimeMixState(last_token, wkv_state))`, a plain
 `(shift_state, wkv_state)` tuple returns `(out, (last_token, wkv_state))`.
+With `exact_state_grad=True` the returned wkv_state is differentiable (ops.WKV_6STATE_BPTT): a model run chunk by
+chunk over a long sequence, carrying both states, gets the gradients of one pass over the whole sequence.  The
+default keeps the reference's truncated gradient, where the final wkv_state is a constant.
 """
 import torch
 
@@ -70,15 +73,19 @@ def tmix_x060_finish(layer, y, g):
     return layer.output(heads.groupnorm_gate(y, g, layer.ln_x.weight, layer.ln_x.bias, H, layer.ln_x.eps, gate_act="silu"))
 
 
-def tmix_x060_forward(layer, x, last_state=None):
-    """Drop-in for RWKV_Tmix_x060.forward (plain, state-tuning and infctx flavours)."""
+def tmix_x060_forward(layer, x, last_state=None, *, exact_state_grad=False):
+    """Drop-in for RWKV_Tmix_x060.forward (plain, state-tuning and infctx flavours).
+    exact_state_grad (infctx only): let the gradient of the returned wkv_state flow back into this chunk."""
     B, T, C = x.shape
     H = layer.time_faaaa.shape[0]
     if last_state is not None:                                  # infctx: (shift_state [B,C], wkv_state [B,H,64,64])
         shift_state, wkv_state = (last_state.shift_state, last_state.wkv_state) if hasattr(last_state, "shift_state") else last_state
         r, k, v, g, w = tmix_x060_project(layer, x, shift_state)
-        y, new_state = ops.WKV_6STATE_INFCTX.apply(B, T, C, H, r, k, v, w, heads._bf16_param(layer.time_faaaa),
-                                                   wkv_state.clone().contiguous())
+        u = heads._bf16_param(layer.time_faaaa)
+        if exact_state_grad:
+            y, new_state = ops.WKV_6STATE_BPTT.apply(B, T, C, H, r, k, v, w, u, wkv_state.contiguous())
+        else:
+            y, new_state = ops.WKV_6STATE_INFCTX.apply(B, T, C, H, r, k, v, w, u, wkv_state.clone().contiguous())
         out = tmix_x060_finish(layer, y, g)
         if hasattr(last_state, "shift_state"):                  # reference calling convention (src/model.py:781)
             return out, type(last_state)(x[:, -1], new_state)
@@ -116,5 +123,5 @@ class Tmix_x060(torch.nn.Module):
         self.gate = torch.nn.Linear(C, C, bias=False)
         self.ln_x = torch.nn.GroupNorm(n_head, C, eps=1e-5 * head_size_divisor ** 2)
 
-    def forward(self, x, last_state=None):
-        return tmix_x060_forward(self, x, last_state)
+    def forward(self, x, last_state=None, *, exact_state_grad=False):
+        return tmix_x060_forward(self, x, last_state, exact_state_grad=exact_state_grad)
