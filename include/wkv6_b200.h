@@ -136,6 +136,16 @@ WKV6_API int wkv6_train_backward_state_grad(int B, int T, int C, int H, const vo
                                    void *gr, void *gk, void *gv, void *gw, void *gu, void *gu_total, void *gs,
                                    const void *gT, int gT_f32, const void *saved, void *workspace,
                                    size_t workspace_bytes, void *stream);
+/* The same backward with the precision of dL/dS_0 chosen by the caller: gs is bf16 (gs_f32 = 0) or fp32
+ * (gs_f32 = 1) [B,H,64(value),64(key)], non-NULL and 16-byte aligned.  A reverse sweep over many chunks hands each
+ * chunk's dL/dS_0 to the previous chunk as its gT; with gs_f32 = 1 that carry is never rounded to bf16, like the
+ * fp32 state carry of the forward (sT_f32).  gT may be NULL here (the last chunk: no final-state gradient); gT_f32
+ * and gs_f32 must be 0 or 1.  Same `saved` and workspace as wkv6_train_backward. */
+WKV6_API int wkv6_train_backward_state_grad_ex(int B, int T, int C, int H, const void *r, const void *k, const void *v,
+                                      const void *w, const void *u, const void *s0, int s0_batched, const void *gy,
+                                      void *gr, void *gk, void *gv, void *gw, void *gu, void *gu_total,
+                                      const void *gT, int gT_f32, void *gs, int gs_f32, const void *saved,
+                                      void *workspace, size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * (a3) wkv6state -- cuda/wkv6state_cuda.cu:298-311 bound by cuda/wkv6state_op.cpp:8-21.

@@ -12,7 +12,8 @@ from .heads import (add_layernorm, create_mask_and_rev_idx, eos_gather, eos_inde
 from .cmix import cmix_shift_lerp2, cmix_x060_forward, relu_sq, sigmoid_mul  # noqa: F401
 from .encoders import (GraphedForward, bi_encoder_encode, bi_encoder_hidden, bi_tmix_forward, blocks_forward, causal_hidden, classification_logits,  # noqa: F401
                        cross_encoder_rows, encode_corpus, length_buckets, sequence_embedding)
-from .infctx import BlockState, BlockStateList, ChannelMixState, TimeMixState  # noqa: F401
+from .infctx import (BlockState, BlockStateList, ChannelMixState, TimeMixState, infctx_forward,  # noqa: F401
+                     infctx_train_step)
 from .tmix import Tmix_x060, tmix_x060_finish, tmix_x060_forward, tmix_x060_project  # noqa: F401
 
 __version__ = "0.1.0"

@@ -287,8 +287,8 @@ int wkv6_train_forward(int B, int T, int C, int H, const void *r, const void *k,
 // the training pair's backward, with (gT) or without (gT = NULL) a gradient arriving at the final state
 static int train_backward(int B, int T, int C, int H, const void *r, const void *k, const void *v, const void *w,
                           const void *u, const void *s0, int s0_batched, const void *gy, void *gr, void *gk, void *gv,
-                          void *gw, void *gu, void *gu_total, void *gs, const void *gT, int gT_f32, const void *saved,
-                          void *workspace, size_t workspace_bytes, void *stream) {
+                          void *gw, void *gu, void *gu_total, void *gs, int gs_f32, const void *gT, int gT_f32,
+                          const void *saved, void *workspace, size_t workspace_bytes, void *stream) {
     if (int rc = check_shape(B, T, C, H)) return rc;
     if ((size_t)B * T == 0) return WKV6_OK;
     REQUIRE_PTRS(r, k, v, w, u, gy, gr, gk, gv, gw, gu);
@@ -297,7 +297,7 @@ static int train_backward(int B, int T, int C, int H, const void *r, const void 
     a.B = B; a.T = T; a.H = H; a.r = r; a.k = k; a.v = v; a.w = w; a.w_kind = W_RAW_BF16; a.u = u;
     a.s0 = s0; a.s0_bstride = s0_batched ? (long long)H * N * N : 0; a.gy = gy; a.gr = gr; a.gk = gk;
     a.gv = gv; a.gw = gw; a.gu = gu; a.gs = gs; a.workspace = workspace; a.workspace_bytes = workspace_bytes;
-    a.gT = gT; a.gT_f32 = gT_f32;
+    a.gT = gT; a.gT_f32 = gT_f32; a.gs_f32 = gs_f32;
     a.saved = const_cast<void *>(saved);
     a.stream = (cudaStream_t)stream;
     a.gu_total = gu_total;
@@ -309,7 +309,7 @@ int wkv6_train_backward(int B, int T, int C, int H, const void *r, const void *k
                         const void *w, const void *u, const void *s0, int s0_batched, const void *gy,
                         void *gr, void *gk, void *gv, void *gw, void *gu, void *gu_total, void *gs,
                         const void *saved, void *workspace, size_t workspace_bytes, void *stream) {
-    return train_backward(B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gu_total, gs, nullptr, 0,
+    return train_backward(B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gu_total, gs, 0, nullptr, 0,
                           saved, workspace, workspace_bytes, stream);
 }
 int wkv6_train_backward_state_grad(int B, int T, int C, int H, const void *r, const void *k, const void *v,
@@ -321,7 +321,20 @@ int wkv6_train_backward_state_grad(int B, int T, int C, int H, const void *r, co
     if (!gT) { set_error("%s: gT is NULL (wkv6_train_backward is the call without a final-state gradient)", __func__); return WKV6_EINVAL; }
     if (gT_f32 != 0 && gT_f32 != 1) { set_error("%s: gT_f32 = %d (0: bf16 gT, 1: fp32 gT)", __func__, gT_f32); return WKV6_EINVAL; }
     if (!check_aligned16(__func__, {{"gT", gT}})) return WKV6_EINVAL;
-    return train_backward(B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gu_total, gs, gT, gT_f32,
+    return train_backward(B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gu_total, gs, 0, gT, gT_f32,
+                          saved, workspace, workspace_bytes, stream);
+}
+int wkv6_train_backward_state_grad_ex(int B, int T, int C, int H, const void *r, const void *k, const void *v,
+                                      const void *w, const void *u, const void *s0, int s0_batched, const void *gy,
+                                      void *gr, void *gk, void *gv, void *gw, void *gu, void *gu_total,
+                                      const void *gT, int gT_f32, void *gs, int gs_f32, const void *saved,
+                                      void *workspace, size_t workspace_bytes, void *stream) {
+    if (int rc = check_shape(B, T, C, H)) return rc;
+    if (gT_f32 != 0 && gT_f32 != 1) { set_error("%s: gT_f32 = %d (0: bf16 gT, 1: fp32 gT)", __func__, gT_f32); return WKV6_EINVAL; }
+    if (gs_f32 != 0 && gs_f32 != 1) { set_error("%s: gs_f32 = %d (0: bf16 gs, 1: fp32 gs)", __func__, gs_f32); return WKV6_EINVAL; }
+    if (!gs) { set_error("%s: gs is NULL", __func__); return WKV6_EINVAL; }
+    if (!check_aligned16(__func__, {{"gT", gT}, {"gs", gs}})) return WKV6_EINVAL;
+    return train_backward(B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gu_total, gs, gs_f32, gT, gT_f32,
                           saved, workspace, workspace_bytes, stream);
 }
 

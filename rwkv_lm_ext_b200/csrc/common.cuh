@@ -54,6 +54,7 @@ struct Args {
     // training pair only: nullptr (the final state feeds nothing) | dL/dS_T, bf16/fp32 [B,H,64(value),64(key)]
     const void *gT = nullptr;
     int gT_f32 = 0;
+    int gs_f32 = 0;                   // training pair only: gs is fp32 (else bf16)
     mutable bool gu_total_done = false;   // set by the route whose kernel added the rows itself
     void *workspace = nullptr;
     size_t workspace_bytes = 0;

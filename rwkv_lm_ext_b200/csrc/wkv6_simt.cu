@@ -388,7 +388,7 @@ __global__ void __launch_bounds__(NT, 2) bwd_r_kernel(Args a, int mode, const fl
             // gs[b,h,j,i] = dL/dS_0[i][j]; thread (x = j, g) holds i in slice
 #pragma unroll
             for (int q = 0; q < SL; q++)
-                ((IO *)a.gs)[((size_t)b * a.H + h) * N * N + (size_t)x * N + g * SL + q] = from_f32<IO>(G2[q]);
+                store_state(a.gs, a.gs_f32, ((size_t)b * a.H + h) * N * N + (size_t)x * N + g * SL + q, G2[q]);
         }
     }
 }

@@ -100,6 +100,7 @@ struct Params {
     const int *row_order;     // BI modes: batch rows sorted by length, longest first, device int [B]
     long long *dbg;           // nullptr, or [gridDim][NC][8 (32 in the profiling build)] clock64 stamps of warp 0 at the stage boundaries (profiling aid)
     int g_init_f32;           // (last: the fields above keep their offsets, and SEG = false reads none of the new ones)
+    int gs_f32;               // SEG only: gs is fp32 (reinterpreted), else bf16
 };
 
 // true when `x` holds in any of the 256 compute threads (named barrier B_SCAN, which they all reach)
@@ -864,9 +865,12 @@ wkv6_tc3_bwd_kernel(const __grid_constant__ CUtensorMap map_r, const __grid_cons
 #pragma unroll
                     for (int g = 0; g < 4; g++)
 #pragma unroll
-                        for (int e = 0; e < 2; e++)   // gs[b,h,j,i] = dL/dS_0[i][j]
-                            p.gs[(((size_t)row * p.H + h) * 64 + F.col(g, e)) * 64 + F.row(hh)] =
-                                __float2bfloat16_rn(__uint_as_float(v[4 * g + 2 * hh + e]) * es);
+                        for (int e = 0; e < 2; e++) {   // gs[b,h,j,i] = dL/dS_0[i][j]
+                            const size_t gi = (((size_t)row * p.H + h) * 64 + F.col(g, e)) * 64 + F.row(hh);
+                            const float gsv = __uint_as_float(v[4 * g + 2 * hh + e]) * es;
+                            if (SEG && p.gs_f32) reinterpret_cast<float *>(p.gs)[gi] = gsv;
+                            else p.gs[gi] = __float2bfloat16_rn(gsv);
+                        }
                 }
             }
             tmem_wait_st();
@@ -1037,8 +1041,11 @@ static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu
     p.lmin = tc_lmin_log2(a);
     p.gu = (bf16 *)a.gu; p.gs = (bf16 *)a.gs;
     p.hz_flags = flags;
+    p.gs_f32 = a.gs_f32;
+    // an fp32 gs, like a g_init or segments, takes the SEG instantiation
+    const bool seg_inst = nseg > 1 || g_init || a.gs_f32;
     // in-kernel sum of gu over the rows: ordinary call only
-    const bool sum_gu = a.gu_total && gu_count && nseg == 1 && !g_init && bi == BI_NONE && a.H <= 512;
+    const bool sum_gu = a.gu_total && gu_count && !seg_inst && bi == BI_NONE && a.H <= 512;
     p.gu_total = sum_gu ? (bf16 *)a.gu_total : nullptr;
     p.gu_count = gu_count;
     if (sum_gu) a.gu_total_done = true;
@@ -1053,7 +1060,7 @@ static int launch_bwd(const Args &a, const bf16 *ckpt, const int *flags, int *gu
     int rc;
     if (bi == BI_CAUSAL) rc = launch_bwd_kernel<false, BI_CAUSAL>(grid, a.stream, maps, p);
     else if (bi == BI_REV) rc = launch_bwd_kernel<false, BI_REV>(grid, a.stream, maps, p);
-    else if (nseg > 1 || g_init) rc = launch_bwd_kernel<true, BI_NONE>(grid, a.stream, maps, p);
+    else if (seg_inst) rc = launch_bwd_kernel<true, BI_NONE>(grid, a.stream, maps, p);
     else rc = launch_bwd_kernel<false, BI_NONE>(grid, a.stream, maps, p);
     if (rc != WKV6_OK) return rc;
     if (clamp) {                       // opt-in decay clamp: a clamped decay no longer depends on w (kept out of the hot kernel)
@@ -1093,12 +1100,15 @@ static int tc3_backward_segmented(const Args &a, int nseg, int seg_chunks) {
     // the chain starts from the caller's final-state gradient (or 0), which the last segment then reads like the others
     if (rc == WKV6_OK) rc = seg_scan(a.B, nseg, a.H, lam, g_loc, a.gT, a.gT_f32, (long long)a.H * 4096, g_end, nullptr, 0, 1, nullptr, a.stream);
     Args v = a;
-    v.gu = gu_tmp; v.gs = a.gs ? gs_tmp : nullptr;
+    // an fp32 gs is staged in g_loc, which nothing reads once the scan has produced g_end
+    void *gs_stage = a.gs_f32 ? (void *)g_loc : (void *)gs_tmp;
+    const size_t gs_el = a.gs_f32 ? 4 : 2;
+    v.gu = gu_tmp; v.gs = a.gs ? gs_stage : nullptr;
     if (rc == WKV6_OK) rc = launch_bwd(v, ckpt, nullptr, nullptr, g_end, 1, nseg, seg_chunks, a.s0 != nullptr);
     if (rc == WKV6_OK) rc = seg_sum_gu(a.B, nseg, C, gu_tmp, a.gu, a.stream);
     if (rc == WKV6_OK && a.gs)                    // dL/dS_0 is what segment 0 of every sequence produced
-        rc = cudaMemcpy2DAsync(a.gs, (size_t)a.H * 4096 * 2, gs_tmp, (size_t)nseg * a.H * 4096 * 2, (size_t)a.H * 4096 * 2, a.B,
-                               cudaMemcpyDeviceToDevice, a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
+        rc = cudaMemcpy2DAsync(a.gs, (size_t)a.H * 4096 * gs_el, gs_stage, (size_t)nseg * a.H * 4096 * gs_el, (size_t)a.H * 4096 * gs_el,
+                               a.B, cudaMemcpyDeviceToDevice, a.stream) == cudaSuccess ? WKV6_OK : WKV6_ECUDA;
     return rc;
 }
 

@@ -75,9 +75,10 @@ class exact_route_report:
         return 0, self._streams
 
 
-def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs, gT=None):
+def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs, gT=None, gs_f32=False):
     """Returns gu summed over the batch rows (src/model.py:232 `torch.sum(gu, 0)`), computed by the library.
-    gT: None, or the gradient of the final state (bf16/fp32 [B,H,64,64], contiguous, 16-byte aligned)."""
+    gT: None, or the gradient of the final state (bf16/fp32 [B,H,64,64], contiguous, 16-byte aligned).
+    gs_f32: gs is an fp32 tensor that the kernels write in fp32 (wkv6_train_backward_state_grad_ex)."""
     saved = ctx.saved_state
     n = lib.wkv6_train_backward_workspace_bytes(B, T, C, H, int(saved is not None))
     ws = torch.empty(max(n, 1), dtype=torch.uint8, device=gy.device)
@@ -85,7 +86,12 @@ def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr,
     head = (B, T, C, H, ptr(r), ptr(k), ptr(v), ptr(w), ptr(u), ptr(s0), int(s0_batched),
             ptr(gy), ptr(gr), ptr(gk), ptr(gv), ptr(gw), ptr(gu), ptr(gu_total), ptr(gs))
     tail = (ptr(saved), ptr(ws), n, stream_of(gy))
-    if gT is None:
+    if gs_f32:
+        head = head[:-1]
+        gT_f32 = int(gT is not None and gT.dtype == torch.float32)
+        check(lib.wkv6_train_backward_state_grad_ex(*head, ptr(gT), gT_f32, ptr(gs), 1, *tail),
+              "wkv6_train_backward_state_grad_ex")
+    elif gT is None:
         check(lib.wkv6_train_backward(*head, *tail), "wkv6_train_backward")
     else:
         check(lib.wkv6_train_backward_state_grad(*head, ptr(gT), int(gT.dtype == torch.float32), *tail),
@@ -217,10 +223,12 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
     ``s_final`` is a new tensor with the dtype of ``s``, bf16 or the fp32 carry), and the gradient of ``s_final``
     flows back into r, k, v, w, u and ``s``.  Chunked long-context training then computes the gradients of one
     pass over the whole sequence.  A ``s_final`` that feeds nothing (gradient None) runs the backward of
-    WKV_6STATE_INFCTX."""
+    WKV_6STATE_INFCTX.
+    fp32_state_grad (fp32 ``s`` only): the kernels write the gradient of ``s`` in fp32 instead of rounding it to bf16,
+    so a reverse sweep over many chunks carries the state gradient at the precision the forward carries the state."""
 
     @staticmethod
-    def forward(ctx, B, T, C, H, r, k, v, w, u, s):
+    def forward(ctx, B, T, C, H, r, k, v, w, u, s, fp32_state_grad=False):
         with torch.no_grad():
             _assert_bf16_contig(r, k, v, w, u)
             assert s.dtype in (torch.bfloat16, torch.float32)
@@ -235,6 +243,7 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
             lib = _lib.load()
             _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, s_final, y)
             ctx.s_dtype = s.dtype
+            ctx.gs_f32 = bool(fp32_state_grad) and s.dtype == torch.float32
             return y, s_final
 
     @staticmethod
@@ -248,7 +257,7 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
             gy = gy.contiguous()
             gr, gk, gv, gw = (torch.empty((B, T, C), device=gy.device, dtype=torch.bfloat16) for _ in range(4))
             gu = torch.empty((B, C), device=gy.device, dtype=torch.bfloat16)
-            gs = torch.empty((B, H, C // H, C // H), device=gy.device, dtype=torch.bfloat16)
+            gs = torch.empty((B, H, C // H, C // H), device=gy.device, dtype=torch.float32 if ctx.gs_f32 else torch.bfloat16)
             gT = None
             if gs_final is not None:
                 gT = gs_final.contiguous()
@@ -256,14 +265,15 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
                 if gT.data_ptr() % 16:                             # the library reads it with 16-byte accesses
                     gT = gT.clone()
             lib = _lib.load()
-            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs, gT)
+            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs, gT, ctx.gs_f32)
             gu = gu.view(H, C // H)
-            return (None, None, None, None, gr, gk, gv, gw, gu, gs.to(ctx.s_dtype))
+            return (None, None, None, None, gr, gk, gv, gw, gu, gs.to(ctx.s_dtype), None)
 
 
-def RUN_CUDA_RWKV6_STATE_BPTT(B, T, C, H, r, k, v, w, u, s):
-    """(y, s_final) of the infctx operator, differentiable through s_final (WKV_6STATE_BPTT); ``s`` is not modified."""
-    return WKV_6STATE_BPTT.apply(B, T, C, H, r, k, v, w, u, s)
+def RUN_CUDA_RWKV6_STATE_BPTT(B, T, C, H, r, k, v, w, u, s, fp32_state_grad=False):
+    """(y, s_final) of the infctx operator, differentiable through s_final (WKV_6STATE_BPTT); ``s`` is not modified.
+    fp32_state_grad: with an fp32 ``s``, its gradient comes from the kernels in fp32 (default: bf16, then cast)."""
+    return WKV_6STATE_BPTT.apply(B, T, C, H, r, k, v, w, u, s, fp32_state_grad)
 
 
 def RUN_CUDA_RWKV6_STATE(B, T, C, H, r, k, v, w, u, s):

@@ -73,9 +73,11 @@ def tmix_x060_finish(layer, y, g):
     return layer.output(heads.groupnorm_gate(y, g, layer.ln_x.weight, layer.ln_x.bias, H, layer.ln_x.eps, gate_act="silu"))
 
 
-def tmix_x060_forward(layer, x, last_state=None, *, exact_state_grad=False):
+def tmix_x060_forward(layer, x, last_state=None, *, exact_state_grad=False, fp32_state_grad=False):
     """Drop-in for RWKV_Tmix_x060.forward (plain, state-tuning and infctx flavours).
-    exact_state_grad (infctx only): let the gradient of the returned wkv_state flow back into this chunk."""
+    exact_state_grad (infctx only): let the gradient of the returned wkv_state flow back into this chunk.
+    fp32_state_grad (with exact_state_grad and an fp32 wkv_state): the gradient of the incoming wkv_state is computed
+    in fp32 by the kernels instead of being rounded to bf16 (ops.WKV_6STATE_BPTT)."""
     B, T, C = x.shape
     H = layer.time_faaaa.shape[0]
     if last_state is not None:                                  # infctx: (shift_state [B,C], wkv_state [B,H,64,64])
@@ -83,7 +85,7 @@ def tmix_x060_forward(layer, x, last_state=None, *, exact_state_grad=False):
         r, k, v, g, w = tmix_x060_project(layer, x, shift_state)
         u = heads._bf16_param(layer.time_faaaa)
         if exact_state_grad:
-            y, new_state = ops.WKV_6STATE_BPTT.apply(B, T, C, H, r, k, v, w, u, wkv_state.contiguous())
+            y, new_state = ops.WKV_6STATE_BPTT.apply(B, T, C, H, r, k, v, w, u, wkv_state.contiguous(), fp32_state_grad)
         else:
             y, new_state = ops.WKV_6STATE_INFCTX.apply(B, T, C, H, r, k, v, w, u, wkv_state.clone().contiguous())
         out = tmix_x060_finish(layer, y, g)
