@@ -311,6 +311,23 @@ WKV6_API int scatter_rows_bf16(int B, int T, int D, const void *gout, const int6
  * gx[b,rev_idx[b,t],:] = gout[b,t,:]. */
 WKV6_API int scatter_tokens_bf16(int B, int T, int D, const void *gout, const int64_t *rev_idx, void *gx,
                         void *stream);
+/* gradient of groupnorm_gate_pair_bf16.  With G = the bf16 gradient of the averaged GroupNorm input (what
+ * groupnorm_gate_backward_bf16 writes for it):  gy[b,t] = G[b,t] / 2,  gy_rev[b, rev_idx[b,t]] = G[b,t] / 2,  gg and
+ * gln_w / gln_b (fp32 [C], or both NULL when frozen) as groupnorm_gate_backward_bf16 -- one pass, the average recomputed
+ * as the forward computes it.  gy and gy_rev may be the two halves of one [2B,T,C] buffer (the gradient of one WKV6 call
+ * over both directions).  rev_idx is a per-row permutation (what create_mask_rev_idx builds), else rows of gy_rev no
+ * entry points at are left unwritten; an entry outside [0, T) writes nothing.  B*T <= INT_MAX.
+ * ws: elementwise_backward_workspace_bytes(B, T, C, 2) bytes. */
+WKV6_API int groupnorm_gate_pair_backward_bf16(int B, int T, int C, int H, float eps, int gate_act, const void *y,
+                                      const void *y_rev, const int64_t *rev_idx, const void *g, const void *ln_w,
+                                      const void *ln_b, const void *gout, void *gy, void *gy_rev, void *gg,
+                                      float *gln_w, float *gln_b, void *ws, size_t ws_bytes, void *stream);
+/* gradient of stack_reversed_bf16:  gx[b,t,:] = gxx[b,t,:] + gxx[B+b, rev_idx[b,t],:]  (one bf16 rounding), gxx [2B,T,D].
+ * Precondition: rev_idx is a per-row involution (rev[b, rev[b,t]] == t), as create_mask_rev_idx builds it; the
+ * scatter of the reversed half is then this gather.  An entry outside [0, T) reads gxx[B+b, t].  D % 8 == 0,
+ * 2*B*T <= INT_MAX. */
+WKV6_API int stack_reversed_backward_bf16(int B, int T, int D, const void *gxx, const int64_t *rev_idx, void *gx,
+                                 void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * Channel mix (RWKV_CMix_x060.forward, src/model.py:635-644; infctx :804-812): the elementwise pieces

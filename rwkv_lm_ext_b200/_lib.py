@@ -71,6 +71,8 @@ SIGNATURES = {
     "sigmoid_mul_bf16": (c_i, [c_sz, c_p, c_p, c_p, c_p]),
     "sigmoid_mul_backward_bf16": (c_i, [c_sz, c_p, c_p, c_p, c_p, c_p, c_p]),
     "scatter_tokens_bf16": (c_i, [c_i, c_i, c_i, c_p, c_p, c_p, c_p]),
+    "groupnorm_gate_pair_backward_bf16": (c_i, [c_i, c_i, c_i, c_i, c_f, c_i] + [c_p] * 13 + [c_sz, c_p]),
+    "stack_reversed_backward_bf16": (c_i, [c_i, c_i, c_i, c_p, c_p, c_p, c_p]),
     "cross_entropy_l2wrap_bf16": (c_i, [ctypes.c_longlong, c_i, c_p, c_p, ctypes.c_longlong, c_p, c_p, c_p, c_p]),
     "cross_entropy_l2wrap_backward_bf16": (c_i, [ctypes.c_longlong, c_i, c_p, c_p, ctypes.c_longlong, c_p, c_p, c_p, c_p, c_f, c_p, c_p]),
 }

@@ -38,13 +38,25 @@ __global__ void sum_partials_kernel(int S, int n, size_t stride, const float *__
 //   gg = gout * z ;  gz = gout * g ;  glw = sum_rows gz * n ;  glb = sum_rows gz
 //   gn = gz * w ;  gy = rstd * (gn - mean(gn) - n * mean(gn * n))
 // 8 consecutive lanes = one group.
+// PAIR: the input was (y + y2[b, rev[b,t]]) / 2 (groupnorm_gate_pair_bf16), recomputed here as the forward computes it;
+// G = bf16(gy) of that average, and G/2 goes to gy[b,t] and to gy2[b, rev[b,t]].  An entry of rev outside [0, T) reads
+// y2[b,t] and writes no gy2 row, so it never leaves its row.
 // ------------------------------------------------------------------------------------------------
-template <bool SILU>
+// row b*T+t of the reversed operand: b*T + rev[b*T+t], and whether rev[b*T+t] is inside [0, T)
+__device__ __forceinline__ long long pair_src(long long row, int T, const int64_t *__restrict__ rev, bool &in_row) {
+    const long long t = rev[row], rb0 = row - row % T;
+    in_row = (unsigned long long)t < (unsigned long long)T;
+    return in_row ? rb0 + t : row;
+}
+
+template <bool SILU, bool PAIR>
 __global__ void __launch_bounds__(256) gn_gate_bwd_kernel(long long BT, int C, float eps, Split sp,
                                                           const bf16 *__restrict__ y, const bf16 *__restrict__ g,
                                                           const bf16 *__restrict__ lw, const bf16 *__restrict__ lb,
                                                           const bf16 *__restrict__ gout, bf16 *__restrict__ gy,
-                                                          bf16 *__restrict__ gg, float *__restrict__ partial) {
+                                                          bf16 *__restrict__ gg, float *__restrict__ partial,
+                                                          const bf16 *__restrict__ y2, const int64_t *__restrict__ rev, int T,
+                                                          bf16 *__restrict__ gy2) {
     const int lane = threadIdx.x & 31, tl = threadIdx.x >> 5;
     const int c_raw = (blockIdx.x * 32 + lane) * 8;
     const bool live = c_raw < C;
@@ -62,20 +74,32 @@ __global__ void __launch_bounds__(256) gn_gate_bwd_kernel(long long BT, int C, f
     unpack8(ld8(lb + c), bfv);
 
     // one row ahead: the three 16-byte loads of row + 1 are in flight while row is reduced (a row is 12 shuffles deep)
-    bf16x8 ny, ng, ngo;
+    bf16x8 ny, ng, ngo, ny2;
+    long long nsrc = 0;
+    bool nin = true;
     if (r0 < r1) {
         const size_t off0 = (size_t)r0 * C + c;
         ny = ld8(y + off0); ng = ld8(g + off0); ngo = ld8(gout + off0);
+        if (PAIR) { nsrc = pair_src(r0, T, rev, nin); ny2 = ld8(y2 + (size_t)nsrc * C + c); }
     }
     for (long long row = r0; row < r1; row++) {          // warp-uniform bounds: shuffles are safe
         const size_t off = (size_t)row * C + c;
+        const long long src = nsrc;
+        const bool in_row = nin;
         float f[8], gf[8], go[8];
         unpack8(ny, f);
         unpack8(ng, gf);
         unpack8(ngo, go);
+        if (PAIR) {                                        // exactly the forward's average (elementwise.cu, gn_gate_kernel)
+            float f2[8];
+            unpack8(ny2, f2);
+#pragma unroll
+            for (int e = 0; e < 8; e++) f[e] = rb(f[e] + f2[e]) * 0.5f;
+        }
         if (row + 1 < r1) {
             const size_t offn = off + C;
             ny = ld8(y + offn); ng = ld8(g + offn); ngo = ld8(gout + offn);
+            if (PAIR) { nsrc = pair_src(row + 1, T, rev, nin); ny2 = ld8(y2 + (size_t)nsrc * C + c); }
         }
         float s = 0.f;
 #pragma unroll
@@ -122,7 +146,15 @@ __global__ void __launch_bounds__(256) gn_gate_bwd_kernel(long long BT, int C, f
 #pragma unroll
         for (int e = 0; e < 8; e++) o[e] = rstd * (gn[e] - m1 - f[e] * m2);
         if (live) {
-            st8(gy + off, pack8(o));
+            if (PAIR) {                                    // bf16(G) / 2: the composition's divide backward, exact
+#pragma unroll
+                for (int e = 0; e < 8; e++) o[e] = rb(o[e]) * 0.5f;
+                const bf16x8 h = pack8(o);
+                st8(gy + off, h);
+                if (in_row) st8(gy2 + (size_t)src * C + c, h);
+            } else {
+                st8(gy + off, pack8(o));
+            }
             st8(gg + off, pack8(ggv));
         }
     }
@@ -201,6 +233,30 @@ __global__ void scatter_tokens_kernel(int BT, int T, int D, const bf16 *__restri
     }
 }
 
+// gx[b,t,:] = gxx[b,t,:] + gxx[B+b, rev[b,t],:]  (gradient of stack_reversed_bf16 when rev is a per-row involution:
+// the scatter of the reversed half then equals this gather).  One warp per token row; an entry of rev outside [0, T)
+// reads the row's own token.
+__global__ void stack_reversed_bwd_kernel(int BT, int T, int D, const bf16 *__restrict__ gxx, const int64_t *__restrict__ rev,
+                                          bf16 *__restrict__ gx) {
+    const int warps = (gridDim.x * blockDim.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    for (int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < BT; row += warps) {
+        const int b = row / T;
+        const int64_t t = rev[row];
+        const size_t rrow = (unsigned long long)t < (unsigned long long)T ? (size_t)b * T + (size_t)t : (size_t)row;
+        const bf16 *src = gxx + (size_t)row * D, *srcr = gxx + ((size_t)BT + rrow) * D;
+        bf16 *dst = gx + (size_t)row * D;
+        for (int d = lane * 8; d < D; d += 256) {
+            float a[8], r[8];
+            unpack8(ld8(src + d), a);
+            unpack8(ld8(srcr + d), r);
+#pragma unroll
+            for (int e = 0; e < 8; e++) a[e] += r[e];
+            st8(dst + d, pack8(a));
+        }
+    }
+}
+
 // number of row splits: enough blocks to fill 148 SMs a few times over, at least 8 rows per lane
 int splits_for(long long BT, int C) {
     const int colblocks = (C + 255) / 256;
@@ -230,6 +286,26 @@ int shift_lerp_backward(int nout, int B, int T, int C, const void *x, const void
                                                                                       (const float *)ws, gmaa);
         count_launch();
     }
+    WKV6_CUDA_CHECK(cudaGetLastError());
+    return WKV6_OK;
+}
+
+// the GroupNorm*gate backward (PAIR when y2 is given) and the fixed-order sums of its partials.  The caller has checked
+// the arguments and the workspace (S row splits).
+int gn_gate_backward(int BT, int C, float eps, int gate_act, const void *y, const void *g, const void *ln_w, const void *ln_b,
+                     const void *gout, void *gy, void *gg, float *gln_w, float *gln_b, void *ws, int S, const void *y2,
+                     const int64_t *rev, int T, void *gy2, void *stream) {
+    const dim3 grid((C + 255) / 256, S);
+    const Split sp = split_of(BT, S);
+    float *partial = (float *)ws;
+    auto kernel = y2 ? (gate_act ? gn_gate_bwd_kernel<true, true> : gn_gate_bwd_kernel<false, true>)
+                     : (gate_act ? gn_gate_bwd_kernel<true, false> : gn_gate_bwd_kernel<false, false>);
+    kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(BT, C, eps, sp, (const bf16 *)y, (const bf16 *)g, (const bf16 *)ln_w,
+                                                   (const bf16 *)ln_b, (const bf16 *)gout, (bf16 *)gy, (bf16 *)gg, partial,
+                                                   (const bf16 *)y2, rev, T, (bf16 *)gy2);
+    if (gln_w) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, C, (size_t)2 * C, partial, gln_w);
+    if (gln_b) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, C, (size_t)2 * C, partial + C, gln_b);
+    count_launch(gln_w ? 3 : 1);
     WKV6_CUDA_CHECK(cudaGetLastError());
     return WKV6_OK;
 }
@@ -298,19 +374,44 @@ int groupnorm_gate_backward_bf16(int BT, int C, int H, float eps, int gate_act, 
         set_error("groupnorm_gate_backward_bf16: workspace too small");
         return WKV6_EINVAL;
     }
-    dim3 grid((C + 255) / 256, S);
-    float *partial = (float *)ws;
-    if (gate_act)
-        gn_gate_bwd_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(
-            BT, C, eps, split_of(BT, S), (const bf16 *)y, (const bf16 *)g, (const bf16 *)ln_w, (const bf16 *)ln_b,
-            (const bf16 *)gout, (bf16 *)gy, (bf16 *)gg, partial);
-    else
-        gn_gate_bwd_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(
-            BT, C, eps, split_of(BT, S), (const bf16 *)y, (const bf16 *)g, (const bf16 *)ln_w, (const bf16 *)ln_b,
-            (const bf16 *)gout, (bf16 *)gy, (bf16 *)gg, partial);
-    if (gln_w) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, C, (size_t)2 * C, partial, gln_w);
-    if (gln_b) sum_partials_kernel<<<(C + 255) / 256, 256, 0, (cudaStream_t)stream>>>(S, C, (size_t)2 * C, partial + C, gln_b);
-    count_launch(gln_w ? 3 : 1);
+    return gn_gate_backward(BT, C, eps, gate_act, y, g, ln_w, ln_b, gout, gy, gg, gln_w, gln_b, ws, S, nullptr, nullptr, 1,
+                            nullptr, stream);
+}
+
+int groupnorm_gate_pair_backward_bf16(int B, int T, int C, int H, float eps, int gate_act, const void *y, const void *y_rev,
+                                      const int64_t *rev_idx, const void *g, const void *ln_w, const void *ln_b,
+                                      const void *gout, void *gy, void *gy_rev, void *gg, float *gln_w, float *gln_b,
+                                      void *ws, size_t ws_bytes, void *stream) {
+    if (B < 0 || T < 0 || H <= 0 || C != H * 64) { set_error("groupnorm_gate_pair_backward_bf16: need C == H*64"); return WKV6_EINVAL; }
+    if ((long long)B * T > INT_MAX) { set_error("groupnorm_gate_pair_backward_bf16: need B*T <= INT_MAX"); return WKV6_EINVAL; }
+    const int BT = B * T;
+    if (BT == 0) return WKV6_OK;
+    if (!y || !y_rev || !rev_idx || !g || !ln_w || !ln_b || !gout || !gy || !gy_rev || !gg || (!gln_w != !gln_b) || !ws) {
+        set_error("groupnorm_gate_pair_backward_bf16: null pointer");
+        return WKV6_EINVAL;
+    }
+    if (!check_aligned16("groupnorm_gate_pair_backward_bf16", {{"y", y}, {"y_rev", y_rev}, {"g", g}, {"ln_w", ln_w}, {"ln_b", ln_b},
+                                                                {"gout", gout}, {"gy", gy}, {"gy_rev", gy_rev}, {"gg", gg}}))
+        return WKV6_EINVAL;
+    const int S = splits_for(BT, C);
+    if (ws_bytes < (size_t)S * 2 * C * sizeof(float)) {
+        set_error("groupnorm_gate_pair_backward_bf16: workspace too small");
+        return WKV6_EINVAL;
+    }
+    return gn_gate_backward(BT, C, eps, gate_act, y, g, ln_w, ln_b, gout, gy, gg, gln_w, gln_b, ws, S, y_rev, rev_idx, T, gy_rev,
+                            stream);
+}
+
+int stack_reversed_backward_bf16(int B, int T, int D, const void *gxx, const int64_t *rev_idx, void *gx, void *stream) {
+    if (B < 0 || T < 0 || D <= 0 || (D & 7)) { set_error("stack_reversed_backward_bf16: need D %% 8 == 0"); return WKV6_EINVAL; }
+    if ((long long)B * T > INT_MAX / 2) { set_error("stack_reversed_backward_bf16: need 2*B*T <= INT_MAX"); return WKV6_EINVAL; }
+    if ((size_t)B * T == 0) return WKV6_OK;
+    if (!gxx || !rev_idx || !gx) { set_error("stack_reversed_backward_bf16: null pointer"); return WKV6_EINVAL; }
+    if (!check_aligned16("stack_reversed_backward_bf16", {{"gxx", gxx}, {"gx", gx}})) return WKV6_EINVAL;
+    const int BT = B * T;
+    stack_reversed_bwd_kernel<<<grid_for((size_t)BT * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+        BT, T, D, (const bf16 *)gxx, rev_idx, (bf16 *)gx);
+    count_launch();
     WKV6_CUDA_CHECK(cudaGetLastError());
     return WKV6_OK;
 }

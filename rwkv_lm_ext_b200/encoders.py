@@ -17,6 +17,7 @@ Per layer ("semantics 2": a causal pass over the tokens and one over each row's 
     channel mix             cmix_x060_forward: 3 fused elementwise kernels around the two GEMMs
 """
 import torch
+import torch.utils.checkpoint
 
 from . import cmix, heads, ops, tmix
 
@@ -38,8 +39,8 @@ def bi_tmix_forward(att, x, rev_idx):
     xx = heads.stack_reversed(x, rev_idx)
     r, k, v, g, w = tmix.tmix_x060_project(att, xx, gate_rows=B)
     y2 = ops.RUN_CUDA_RWKV6(2 * B, T, C, H, r, k, v, w, att.time_faaaa)
-    y, ry = y2[:B], y2[B:]                                                       # ry: still in reversed token order
-    z = heads.groupnorm_gate_pair(y, ry, rev_idx, g, att.ln_x.weight, att.ln_x.bias, H, att.ln_x.eps, gate_act="silu")
+    # y2[:B] plain, y2[B:] still in reversed token order; passed whole, so that its gradient is one [2B,T,C] tensor
+    z = heads.groupnorm_gate_pair(y2, None, rev_idx, g, att.ln_x.weight, att.ln_x.bias, H, att.ln_x.eps, gate_act="silu")
     return att.output(z)
 
 
@@ -49,13 +50,20 @@ def _ffn(ffn, h):
     return ffn(h)
 
 
-def blocks_forward(blocks, x, ln_out, att):
+def blocks_forward(blocks, x, ln_out, att, checkpoint=False):
     """ln_out(block_L(... block_1(x))) for `Block.forward` of src/model.py:904-933 (x = ln0(x) in block 0;
     x = x + att(ln1(x)); x = x + ffn(ln2(x))), with every residual add fused with the LayerNorm that follows it
     (heads.add_layernorm: one pass over the residual stream instead of an add pass and a LayerNorm pass).
-    `att(blk, h)` computes the time-mix output of a block from its normalised input."""
+    `att(blk, h)` computes the time-mix output of a block from its normalised input.
+    checkpoint=True: every block body (x, h) -> (x', h') runs under non-reentrant torch.utils.checkpoint, like the
+    reference's trainers (deepspeed.checkpointing.checkpoint(block)); a training step then keeps only the two
+    block-boundary tensors of each layer and recomputes the block in the backward."""
     def ln(mod, x_, delta=None):
         return heads.add_layernorm(x_, delta, mod.weight, mod.bias, mod.eps)
+
+    def body(blk, nxt, x_, h_):
+        x_, h_ = ln(blk.ln2, x_, att(blk, h_))                        # x += att(ln1(x));  h = ln2(x)
+        return ln(nxt, x_, _ffn(blk.ffn, h_))                         # x += ffn(ln2(x));  h = next ln1(x) / ln_out(x)
     h = None
     n = len(blocks)
     for i, blk in enumerate(blocks):
@@ -63,24 +71,28 @@ def blocks_forward(blocks, x, ln_out, att):
             x = ln(blk.ln0, x)[1]
         if h is None:
             h = ln(blk.ln1, x)[1]
-        x, h = ln(blk.ln2, x, att(blk, h))                            # x += att(ln1(x));  h = ln2(x)
         nxt = blocks[i + 1].ln1 if i + 1 < n else ln_out
-        x, h = ln(nxt, x, _ffn(blk.ffn, h))                           # x += ffn(ln2(x));  h = next ln1(x) / ln_out(x)
+        if checkpoint and torch.is_grad_enabled():
+            x, h = torch.utils.checkpoint.checkpoint(body, blk, nxt, x, h, use_reentrant=False)
+        else:
+            x, h = body(blk, nxt, x, h)
     return h
 
 
-def bi_encoder_hidden(model, idx):
-    """ln_out(blocks(emb(idx)))  [B,T,D] in the model's dtype (bf16 weights expected)."""
+def bi_encoder_hidden(model, idx, checkpoint=False):
+    """ln_out(blocks(emb(idx)))  [B,T,D] in the model's dtype (bf16 weights expected).  Differentiable on the same
+    fused kernels as the inference forward; checkpoint=True recomputes every block in the backward (blocks_forward)."""
     emb_id, pad_id = _ids(model)
     idx = idx.contiguous()
     _, rev_idx = heads.create_mask_and_rev_idx(idx, emb_id, pad_id)
-    return blocks_forward(model.blocks, model.emb(idx), model.ln_out, lambda blk, h: bi_tmix_forward(blk.att, h, rev_idx))
+    return blocks_forward(model.blocks, model.emb(idx), model.ln_out, lambda blk, h: bi_tmix_forward(blk.att, h, rev_idx),
+                          checkpoint)
 
 
-def bi_encoder_encode(model, idx):
+def bi_encoder_encode(model, idx, checkpoint=False):
     """encode_sentence: the hidden state at each row's first `emb_id` token.  [B,D]."""
     emb_id, _ = _ids(model)
-    hidden = bi_encoder_hidden(model, idx)
+    hidden = bi_encoder_hidden(model, idx, checkpoint)
     return heads.eos_gather(hidden.contiguous(), idx, emb_id)[0]
 
 
@@ -91,24 +103,24 @@ def _base(wrapper):
     return getattr(wrapper, "rwkvModel", wrapper)
 
 
-def causal_hidden(model, idx):
+def causal_hidden(model, idx, checkpoint=False):
     """ln_out(blocks(emb(idx)))  [B,T,D] of the plain (causal) RWKV-6 model -- the body shared by
     `RwkvForSequenceEmbedding.forward` (src/model_ext.py:1739-1762) and `RwkvForClassification.forward`
     (src/model_ext.py:183-205) -- with every block on the fused kernels.  Right padding never reaches a position
     before it, so a padded batch gives each row what the reference's one-sentence-at-a-time inference classes
-    (src/model_run.py:815-848) compute for it."""
+    (src/model_run.py:815-848) compute for it.  checkpoint: recompute every block in the backward (blocks_forward)."""
     base = _base(model)
     return blocks_forward(base.blocks, base.emb(idx.contiguous()), base.ln_out,
-                          lambda blk, h: tmix.tmix_x060_forward(blk.att, h))
+                          lambda blk, h: tmix.tmix_x060_forward(blk.att, h), checkpoint)
 
 
-def sequence_embedding(wrapper, idx, variant="train"):
+def sequence_embedding(wrapper, idx, variant="train", checkpoint=False):
     """`RwkvForSequenceEmbedding.forward`: hidden states -> position of the first `embedding_id` token (bit-exact
     index kernel) -> pooling (`weightedmean` / `lasttoken` / `avg`; variant "train" = src/model_ext.py:1708-1738,
     "infer" = src/model_run.py:777-797) -> optional dense + tanh head.  `wrapper` carries the reference's
     attribute names: rwkvModel, embedding_id, pooling_type, add_mlp, dense, activation."""
     emb_id = int(getattr(wrapper, "embedding_id", 1))
-    hidden = causal_hidden(wrapper, idx).contiguous()
+    hidden = causal_hidden(wrapper, idx, checkpoint).contiguous()
     pos = heads.eos_index(idx, emb_id)
     x = heads.pooling(hidden, pos, getattr(wrapper, "pooling_type", "weightedmean"), variant)
     if getattr(wrapper, "add_mlp", False):
@@ -116,12 +128,12 @@ def sequence_embedding(wrapper, idx, variant="train"):
     return x
 
 
-def classification_logits(wrapper, idx):
+def classification_logits(wrapper, idx, checkpoint=False):
     """`RwkvForClassification.forward` (src/model_ext.py:183-211): score(hidden)[b, first class_id token].  The row is
     gathered BEFORE the score Linear (same numbers, T times fewer FLOPs than scoring every token).  This is also the
     reference's cross-encoder: rows are "query [sep] document [cls]" (see `cross_encoder_rows`)."""
     cls_id = int(getattr(wrapper, "class_id", 1))
-    hidden = causal_hidden(wrapper, idx).contiguous()
+    hidden = causal_hidden(wrapper, idx, checkpoint).contiguous()
     row, _ = heads.eos_gather(hidden, idx, cls_id)
     return wrapper.score(row.to(wrapper.score.weight.dtype))
 

@@ -174,18 +174,44 @@ class _ReverseX(torch.autograd.Function):
         return gx, None
 
 
-def stack_reversed(x: torch.Tensor, rev_idx: torch.Tensor) -> torch.Tensor:
-    """cat([x, reverse_x(x, rev_idx)], 0)  [2B,T,D]: both directions of a bidirectional encoder layer as one batch.
-    One kernel (x read once) when no gradient is needed; the differentiable pieces otherwise."""
-    _cuda(x)
-    if _needs_grad(x) or x.shape[-1] % 8 != 0:
-        return torch.cat([x, reverse_x(x, rev_idx)], 0)
-    assert x.dtype == torch.bfloat16 and x.dim() == 3 and rev_idx.dtype == torch.int64 and rev_idx.shape == x.shape[:2]
-    x, rev_idx = _dense(x), rev_idx.contiguous()
+def _stack_reversed_fwd(x, rev_idx):
     B, T, D = x.shape
     out = torch.empty((2 * B, T, D), device=x.device, dtype=x.dtype)
     check(_lib.load().stack_reversed_bf16(B, T, D, ptr(x), ptr(rev_idx), ptr(out), stream_of(x)), "stack_reversed_bf16")
     return out
+
+
+class _StackReversed(torch.autograd.Function):
+    """x -> [x; reverse_x(x)].  Backward: gx = gxx[:B] + reverse_x(gxx[B:]) in one pass (rev_idx is an involution)."""
+
+    @staticmethod
+    def forward(ctx, x, rev_idx):
+        ctx.save_for_backward(rev_idx)
+        return _stack_reversed_fwd(x, rev_idx)
+
+    @staticmethod
+    def backward(ctx, gxx):
+        (rev_idx,) = ctx.saved_tensors
+        gxx = _dense(gxx)
+        B, T, D = gxx.shape[0] // 2, gxx.shape[1], gxx.shape[2]
+        gx = torch.empty((B, T, D), device=gxx.device, dtype=gxx.dtype)
+        check(_lib.load().stack_reversed_backward_bf16(B, T, D, ptr(gxx), ptr(rev_idx), ptr(gx), stream_of(gxx)),
+              "stack_reversed_backward_bf16")
+        return gx, None
+
+
+def stack_reversed(x: torch.Tensor, rev_idx: torch.Tensor) -> torch.Tensor:
+    """cat([x, reverse_x(x, rev_idx)], 0)  [2B,T,D]: both directions of a bidirectional encoder layer as one batch,
+    one kernel (x read once).  Differentiable w.r.t. x when rev_idx is a per-row involution (what reverse_x_idx builds):
+    the backward is one kernel too.  D % 8 != 0 takes the differentiable pieces."""
+    _cuda(x)
+    if x.shape[-1] % 8 != 0:
+        return torch.cat([x, reverse_x(x, rev_idx)], 0)
+    assert x.dtype == torch.bfloat16 and x.dim() == 3 and rev_idx.dtype == torch.int64 and rev_idx.shape == x.shape[:2]
+    x, rev_idx = _dense(x), rev_idx.contiguous()
+    if _needs_grad(x):
+        return _StackReversed.apply(x, rev_idx)
+    return _stack_reversed_fwd(x, rev_idx)
 
 
 def reverse_x(x: torch.Tensor, rev_idx: torch.Tensor) -> torch.Tensor:
@@ -398,21 +424,68 @@ def groupnorm_gate(y, g, ln_w, ln_b, H, eps, gate_act=None):
     return _gn_fwd(y, g, ln_w, ln_b, H, eps, act)
 
 
+def _gn_pair_fwd(y, y_rev, rev_idx, g, ln_w, ln_b, H, eps, act):
+    B, T, C = y.shape
+    out = torch.empty_like(y)
+    check(_lib.load().groupnorm_gate_pair_bf16(B, T, C, H, float(eps), act, ptr(y), ptr(y_rev), ptr(rev_idx), ptr(g),
+                                               ptr(ln_w), ptr(ln_b), ptr(out), stream_of(y)), "groupnorm_gate_pair_bf16")
+    return out
+
+
+class _GroupNormGatePair(torch.autograd.Function):
+    """(y2 = [y; y_rev] [2B,T,C], g) -> ln_x((y + reverse_x(y_rev)) / 2) * g.  Saves y2 and recomputes the average in
+    the backward kernel, which writes the gradient of y2 as ONE [2B,T,C] tensor: the WKV6 call over both directions
+    takes it as is."""
+
+    @staticmethod
+    def forward(ctx, y2, rev_idx, g, ln_w, ln_b, H, eps, act):
+        B = y2.shape[0] // 2
+        ctx.save_for_backward(y2, rev_idx, g, ln_w, ln_b)
+        ctx.meta = (H, eps, act)
+        return _gn_pair_fwd(y2[:B], y2[B:], rev_idx, g, ln_w, ln_b, H, eps, act)
+
+    @staticmethod
+    def backward(ctx, gout):
+        y2, rev_idx, g, ln_w, ln_b = ctx.saved_tensors
+        H, eps, act = ctx.meta
+        lib = _lib.load()
+        B, T, C = g.shape
+        gout = _dense(gout)
+        gy2, gg = torch.empty_like(y2), torch.empty_like(g)
+        need_p = ctx.needs_input_grad[3] or ctx.needs_input_grad[4]                       # frozen affine: no reduction
+        gw = torch.empty(C, dtype=torch.float32, device=g.device) if need_p else None
+        gb = torch.empty(C, dtype=torch.float32, device=g.device) if need_p else None
+        ws = _ws(lib, B, T, C, 2, g.device)
+        check(lib.groupnorm_gate_pair_backward_bf16(B, T, C, H, float(eps), act, ptr(y2[:B]), ptr(y2[B:]), ptr(rev_idx), ptr(g),
+                                                    ptr(ln_w), ptr(ln_b), ptr(gout), ptr(gy2[:B]), ptr(gy2[B:]), ptr(gg), ptr(gw),
+                                                    ptr(gb), ptr(ws), ws.numel(), stream_of(g)),
+              "groupnorm_gate_pair_backward_bf16")
+        return (gy2, None, gg, (gw.to(ln_w.dtype) if need_p else None), (gb.to(ln_b.dtype) if need_p else None),
+                None, None, None)
+
+
 def groupnorm_gate_pair(y, y_rev, rev_idx, g, ln_w, ln_b, H, eps, gate_act=None):
     """ln_x((y + reverse_x(y_rev, rev_idx)) / 2) * g  -- the tail of bi_att_forward_batch
     (src/model_encoder_run.py:72-74) with the reverse gather and the average inside the kernel.
-    Under autograd the pieces run separately (each is differentiable)."""
+    y_rev=None: y is the [2B,T,C] stack of both directions (plain rows first), e.g. the output of one WKV6 call over
+    `stack_reversed`; its gradient is then one [2B,T,C] tensor, with no slicing in the graph.
+    Differentiable w.r.t. y, y_rev, g and the GroupNorm affine parameters when rev_idx is a per-row permutation; given
+    separately under autograd, y and y_rev are stacked first (one copy)."""
     _cuda(y)
+    assert y.dtype == torch.bfloat16 and g.dtype == torch.bfloat16 and rev_idx.dtype == torch.int64
+    assert y_rev is None or y_rev.dtype == torch.bfloat16
+    B = g.shape[0]
+    g, rev_idx = _dense(g), rev_idx.contiguous()
+    ln_w, ln_b, act = _bf16_param(ln_w), _bf16_param(ln_b), _GATE_ACT[gate_act]
     if _needs_grad(y, y_rev, g, ln_w, ln_b):
-        return groupnorm_gate((y + reverse_x(y_rev, rev_idx)) / 2, g, ln_w, ln_b, H, eps, gate_act)
-    assert y.dtype == torch.bfloat16 and y_rev.dtype == torch.bfloat16 and g.dtype == torch.bfloat16 and rev_idx.dtype == torch.int64
-    y, y_rev, g, rev_idx = _dense(y), _dense(y_rev), _dense(g), rev_idx.contiguous()
-    B, T, C = y.shape
-    out = torch.empty_like(y)
-    check(_lib.load().groupnorm_gate_pair_bf16(B, T, C, H, float(eps), _GATE_ACT[gate_act], ptr(y), ptr(y_rev), ptr(rev_idx), ptr(g),
-                                               ptr(_bf16_param(ln_w)), ptr(_bf16_param(ln_b)), ptr(out), stream_of(y)),
-          "groupnorm_gate_pair_bf16")
-    return out
+        y2 = _dense(y if y_rev is None else torch.cat([y, y_rev], 0))
+        assert y2.shape[0] == 2 * B and y2.shape[1:] == g.shape[1:] and y2.shape[-1] == H * 64
+        return _GroupNormGatePair.apply(y2, rev_idx, g, ln_w, ln_b, H, eps, act)
+    if y_rev is None:
+        y, y_rev = y[:B], y[B:]
+    y, y_rev = _dense(y), _dense(y_rev)
+    assert y.shape == g.shape and y_rev.shape == g.shape and y.shape[-1] == H * 64
+    return _gn_pair_fwd(y, y_rev, rev_idx, g, ln_w, ln_b, H, eps, act)
 
 
 def _add_ln_fwd(x, delta, w, b, eps, want_stats):

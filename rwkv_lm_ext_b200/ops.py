@@ -36,9 +36,10 @@ def _workspace(lib, B, T, C, H, device):
 
 def _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, sT, y):
     """Forward of the training pair (include/wkv6_b200.h): when a gradient will be asked for, the
-    kernel also leaves the bf16 chunk-start states in ``ctx.saved_state`` -- kept next to
-    save_for_backward's r,k,v,w,u like the reference keeps its inputs (src/model.py:203) -- so that
-    backward does not re-run the recurrence."""
+    kernel also leaves the bf16 chunk-start states in a buffer that is returned (else None) -- the caller
+    saves it with save_for_backward next to r,k,v,w,u, like the reference keeps its inputs (src/model.py:203),
+    so that backward does not re-run the recurrence, and so that torch.utils.checkpoint drops and recomputes
+    it with the rest of a checkpointed block."""
     saved = None
     if any(ctx.needs_input_grad):
         saved = torch.empty(lib.wkv6_saved_bytes(B, T, C, H), dtype=torch.uint8, device=r.device)
@@ -48,9 +49,10 @@ def _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, sT, y):
     check(lib.wkv6_train_forward(B, T, C, H, ptr(r), ptr(k), ptr(v), ptr(w), ptr(u), ptr(s0), int(s0_batched),
                                  s0_f32, ptr(sT), sT_f32, ptr(y), ptr(saved), ctypes.byref(valid), stream_of(r)),
           "wkv6_train_forward")
-    ctx.saved_state = saved if valid.value else None
-    if _diag["collect"] and ctx.saved_state is not None:
+    saved = saved if valid.value else None
+    if _diag["collect"] and saved is not None:
         _diag["streams"] += B * H
+    return saved
 
 
 # Diagnostics: how many (b,h) streams of the training forwards left the tensor-core kernels for the exact SIMT route.
@@ -75,11 +77,11 @@ class exact_route_report:
         return 0, self._streams
 
 
-def _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs, gT=None, gs_f32=False):
+def _train_backward(saved, lib, B, T, C, H, r, k, v, w, u, s0, s0_batched, gy, gr, gk, gv, gw, gu, gs, gT=None, gs_f32=False):
     """Returns gu summed over the batch rows (src/model.py:232 `torch.sum(gu, 0)`), computed by the library.
+    saved: what _train_forward returned (None: the backward re-runs the recurrence).
     gT: None, or the gradient of the final state (bf16/fp32 [B,H,64,64], contiguous, 16-byte aligned).
     gs_f32: gs is an fp32 tensor that the kernels write in fp32 (wkv6_train_backward_state_grad_ex)."""
-    saved = ctx.saved_state
     n = lib.wkv6_train_backward_workspace_bytes(B, T, C, H, int(saved is not None))
     ws = torch.empty(max(n, 1), dtype=torch.uint8, device=gy.device)
     gu_total = torch.empty((C,), device=gy.device, dtype=torch.bfloat16)
@@ -113,10 +115,10 @@ class WKV_6(torch.autograd.Function):
             assert HEAD_SIZE == C // H
             _require_cuda(r)
             ctx.B, ctx.T, ctx.C, ctx.H = B, T, C, H
-            ctx.save_for_backward(r, k, v, w, u)
             y = torch.empty((B, T, C), device=r.device, dtype=torch.bfloat16, memory_format=torch.contiguous_format)
             lib = _lib.load()
-            _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, None, False, None, y)
+            saved = _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, None, False, None, y)
+            ctx.save_for_backward(r, k, v, w, u, saved)
             return y
 
     @staticmethod
@@ -125,11 +127,11 @@ class WKV_6(torch.autograd.Function):
             assert gy.dtype == torch.bfloat16
             B, T, C, H = ctx.B, ctx.T, ctx.C, ctx.H
             gy = gy.contiguous()
-            r, k, v, w, u = ctx.saved_tensors
+            r, k, v, w, u, saved = ctx.saved_tensors
             gr, gk, gv, gw = (torch.empty((B, T, C), device=gy.device, dtype=torch.bfloat16) for _ in range(4))
             gu = torch.empty((B, C), device=gy.device, dtype=torch.bfloat16)
             lib = _lib.load()
-            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, None, False, gy, gr, gk, gv, gw, gu, None)
+            gu = _train_backward(saved, lib, B, T, C, H, r, k, v, w, u, None, False, gy, gr, gk, gv, gw, gu, None)
             gu = gu.view(H, C // H)                        # src/model.py:232 (the sum over B happens in the library)
             return (None, None, None, None, gr, gk, gv, gw, gu)
 
@@ -151,10 +153,10 @@ class WKV_6STATE(torch.autograd.Function):
             _require_cuda(r)
             assert tuple(s.shape) == (H, HEAD_SIZE, HEAD_SIZE)
             ctx.B, ctx.T, ctx.C, ctx.H = B, T, C, H
-            ctx.save_for_backward(r, k, v, w, u, s)
             y = torch.empty((B, T, C), device=r.device, dtype=torch.bfloat16, memory_format=torch.contiguous_format)
             lib = _lib.load()
-            _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, False, None, y)
+            saved = _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, False, None, y)
+            ctx.save_for_backward(r, k, v, w, u, s, saved)
             return y
 
     @staticmethod
@@ -163,12 +165,12 @@ class WKV_6STATE(torch.autograd.Function):
             assert gy.dtype == torch.bfloat16
             B, T, C, H = ctx.B, ctx.T, ctx.C, ctx.H
             gy = gy.contiguous()
-            r, k, v, w, u, s = ctx.saved_tensors
+            r, k, v, w, u, s, saved = ctx.saved_tensors
             gr, gk, gv, gw = (torch.empty((B, T, C), device=gy.device, dtype=torch.bfloat16) for _ in range(4))
             gu = torch.empty((B, C), device=gy.device, dtype=torch.bfloat16)
             gs = torch.empty((B, H, C // H, C // H), device=gy.device, dtype=torch.bfloat16)
             lib = _lib.load()
-            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s, False, gy, gr, gk, gv, gw, gu, gs)
+            gu = _train_backward(saved, lib, B, T, C, H, r, k, v, w, u, s, False, gy, gr, gk, gv, gw, gu, gs)
             gu = gu.view(H, C // H)                                # src/model.py:181 (summed over B in the library)
             gs = torch.sum(gs, 0).view(H, C // H, C // H)          # src/model.py:182
             return (None, None, None, None, gr, gk, gv, gw, gu, gs)
@@ -191,10 +193,10 @@ class WKV_6STATE_INFCTX(torch.autograd.Function):
             # the reference saves `s` and then overwrites it (src/model.py:104-106), so its backward
             # sees the FINAL state; keep the initial one instead (SURVEY.md 2.3)
             s_init = s.to(torch.bfloat16, copy=True)
-            ctx.save_for_backward(r, k, v, w, u, s_init)
             y = torch.empty((B, T, C), device=r.device, dtype=torch.bfloat16, memory_format=torch.contiguous_format)
             lib = _lib.load()
-            _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, s, y)
+            saved = _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, s, y)
+            ctx.save_for_backward(r, k, v, w, u, s_init, saved)
             ctx.mark_dirty(s)
             ctx.s_dtype = s.dtype
             return y, s
@@ -205,12 +207,12 @@ class WKV_6STATE_INFCTX(torch.autograd.Function):
             assert gy.dtype == torch.bfloat16
             B, T, C, H = ctx.B, ctx.T, ctx.C, ctx.H
             gy = gy.contiguous()
-            r, k, v, w, u, s = ctx.saved_tensors
+            r, k, v, w, u, s, saved = ctx.saved_tensors
             gr, gk, gv, gw = (torch.empty((B, T, C), device=gy.device, dtype=torch.bfloat16) for _ in range(4))
             gu = torch.empty((B, C), device=gy.device, dtype=torch.bfloat16)
             gs = torch.empty((B, H, C // H, C // H), device=gy.device, dtype=torch.bfloat16)
             lib = _lib.load()
-            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs)
+            gu = _train_backward(saved, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs)
             gu = gu.view(H, C // H)
             # per-sample state: its gradient is per sample too.  (The reference sums gs over the
             # batch into [H,64,64] even here, src/model.py:128 -- a shape that cannot flow back
@@ -237,11 +239,12 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
             _require_cuda(r)
             assert tuple(s.shape) == (B, H, HEAD_SIZE, HEAD_SIZE)
             ctx.B, ctx.T, ctx.C, ctx.H = B, T, C, H
-            ctx.save_for_backward(r, k, v, w, u, s.to(torch.bfloat16))
+            s_init = s.to(torch.bfloat16)
             y = torch.empty((B, T, C), device=r.device, dtype=torch.bfloat16, memory_format=torch.contiguous_format)
             s_final = torch.empty_like(s, memory_format=torch.contiguous_format)
             lib = _lib.load()
-            _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, s_final, y)
+            saved = _train_forward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, s_final, y)
+            ctx.save_for_backward(r, k, v, w, u, s_init, saved)
             ctx.s_dtype = s.dtype
             ctx.gs_f32 = bool(fp32_state_grad) and s.dtype == torch.float32
             return y, s_final
@@ -250,7 +253,7 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
     def backward(ctx, gy, gs_final):
         with torch.no_grad():
             B, T, C, H = ctx.B, ctx.T, ctx.C, ctx.H
-            r, k, v, w, u, s = ctx.saved_tensors
+            r, k, v, w, u, s, saved = ctx.saved_tensors
             if gy is None:                                         # only the final state feeds the loss
                 gy = torch.zeros((B, T, C), device=r.device, dtype=torch.bfloat16)
             assert gy.dtype == torch.bfloat16
@@ -265,7 +268,7 @@ class WKV_6STATE_BPTT(torch.autograd.Function):
                 if gT.data_ptr() % 16:                             # the library reads it with 16-byte accesses
                     gT = gT.clone()
             lib = _lib.load()
-            gu = _train_backward(ctx, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs, gT, ctx.gs_f32)
+            gu = _train_backward(saved, lib, B, T, C, H, r, k, v, w, u, s, True, gy, gr, gk, gv, gw, gu, gs, gT, ctx.gs_f32)
             gu = gu.view(H, C // H)
             return (None, None, None, None, gr, gk, gv, gw, gu, gs.to(ctx.s_dtype), None)
 
