@@ -182,7 +182,6 @@ ddlerp_lora_kernel(const __grid_constant__ CUtensorMap map_h, const __grid_const
                     outp[q * 4 + e] = *reinterpret_cast<const uint32_t *>(&o2);
                 }
             }
-            if (n == NOUT - 1) mbar_arrive(&bar.x_free[gi & 1]);
             // staging buffer free?  (thread 0 issued the previous store)
             if (threadIdx.x == 0) tma_store_wait_read<0>();
             named_bar_sync<1, EPI_THREADS>();
@@ -190,6 +189,10 @@ ddlerp_lora_kernel(const __grid_constant__ CUtensorMap map_h, const __grid_const
             for (int q = 0; q < 4; q++)
                 *reinterpret_cast<uint4 *>(sm + OFF_STG + sw128(row, (half * 4 + q) * 16)) =
                     make_uint4(outp[q * 4], outp[q * 4 + 1], outp[q * 4 + 2], outp[q * 4 + 3]);
+            // The x buffer is released only after stores that consume every value read from it: the arrive does not wait
+            // for loads still in flight, and an arrive ahead of them lets the refill of group gi+2 land under the reads
+            // of this item.
+            if (n == NOUT - 1) mbar_arrive(&bar.x_free[gi & 1]);
             fence_proxy_async();
             named_bar_sync<2, EPI_THREADS>();
             if (threadIdx.x == 0) {

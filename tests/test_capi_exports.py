@@ -123,6 +123,24 @@ def test_ddlerp_backward_rejects_more_than_int_max_m_rows():
     assert rc == -1 and lib.wkv6b200_last_error().decode() == "tmix_ddlerp_mix_backward_bf16: need 5*B <= INT_MAX"
 
 
+@pytest.mark.skipif(torch.cuda.is_available(),
+                    reason="a library without the check would launch its kernels on the fake addresses")
+@pytest.mark.parametrize("R,C", [(64, 64), (16, 64), (32, 96)])
+def test_ddlerp_lora_rejects_other_ranks_before_any_launch(R, C):
+    """The fused kernel is rank 32 over 64-channel groups only: any other R, or C not a multiple of 64, is
+    WKV6_EUNSUPPORTED with a message naming the bmm route, checked before anything is launched on the aligned fake
+    pointers."""
+    from rwkv_lm_ext_b200 import _lib
+    lib = _lib.load()
+    names = _ALIGNED_ENTRIES["tmix_ddlerp_lora_bf16"][0]
+    fake = {name: 0x7f0000000000 + 0x100000 * i for i, name in enumerate(names)}
+    shape = dict(_SHAPE_ARGS, R=R, C=C, stream=None)
+    rc = lib.tmix_ddlerp_lora_bf16(*[shape[n] if n in shape else fake[n] for n in names])
+    assert rc == -4
+    assert (lib.wkv6b200_last_error().decode()
+            == "tmix_ddlerp_lora_bf16: needs R == 32 and C % 64 == 0 (use bmm + tmix_ddlerp_mix_bf16)")
+
+
 def test_product_never_imports_oracle():
     pkg = os.path.join(ROOT, "rwkv_lm_ext_b200")
     for dirpath, _, files in os.walk(pkg):
